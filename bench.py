@@ -32,6 +32,8 @@ data path.  A "step" is one pass of the whole path over the rank's batch.
            the reference's fastest CPU mode; its parallel mode cannot run 64 utterances on this host).
   --global-batch G : strong scaling (BASELINE configs[2]): G utterances split over the ranks.
   --quantized      : BASELINE configs[4] semantics (quantize.py FakeQuantize model), same timing.
+  --dump-outputs D : after the timed steps, what the last one returned (see dump_outputs) as D/<name>.npy, so that
+           two builds can be compared output for output; the inputs are seeded, so equal arguments mean equal inputs.
 """
 import argparse
 import json
@@ -40,6 +42,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True     # the tree may be read-only: the benchmark writes nothing into it
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (os.path.join(ROOT, "velocity-asr_b200"), os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
@@ -149,6 +153,26 @@ def emit(line):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, tokens, lens):
+    """What a caller of the timed path receives for its batch: tokens.npy (B, L) the greedy-CTC ids, -1 past each
+    utterance's count, and lengths.npy (B,) the counts, both float32 (ids and counts are exact in it).  Should that
+    exceed 64 MB, a fixed seeded sample of utterances; rows.npy names the rows written."""
+    import numpy as np
+    tokens, lens = np.asarray(tokens), np.asarray(lens)
+    tokens = np.where(np.arange(tokens.shape[1]) < lens[:, None], tokens, -1)
+    rows = np.arange(len(lens))
+    per_row = 4 * (tokens.shape[1] + 2)
+    if per_row * len(rows) > DUMP_LIMIT_BYTES - 4096:            # 4 KB: the three .npy headers
+        keep = (DUMP_LIMIT_BYTES - 4096) // per_row
+        rows = np.sort(np.random.RandomState(0).choice(len(rows), keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("tokens", tokens[rows]), ("lengths", lens[rows]), ("rows", rows)):
+        np.save(os.path.join(out_dir, name + ".npy"), arr.astype(np.float32))
+
+
 # ----------------------------------------------------------------------------- reference ---
 def load_reference_impl():
     """(kind, module): the unmodified reference if it travelled with the repo, else None."""
@@ -248,8 +272,14 @@ def run_reference_arm(args):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        out = step()
     total = time.perf_counter() - t0
+    if args.dump_outputs:
+        import numpy as np
+        tok = np.full((n_utt, (1 + SR * UTT_SECONDS // 160 + 1) // 2), -1, np.int32)
+        for b, t in enumerate(out):
+            tok[b, :len(t)] = t
+        dump_outputs(args.dump_outputs, tok, [len(t) for t in out])
     value = args.steps * n_utt * UTT_SECONDS / total
     sample = (f"each step = {n_utt} of the workload's {BATCH_PER_GPU} utterances (x {UTT_SECONDS} s), "
               f"scan_mode={SCAN_MODE}, {'torch CPU (unmodified reference)' if ref is not None else 'numpy oracle port'}, "
@@ -415,6 +445,8 @@ def run_own_arm(args):
     dev_ms = e0.elapsed_time(e1)
     launches = lib.vasr_kernel_launches(eng.handle) - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tokens.cpu().numpy(), lens.cpu().numpy())
 
     # ---- parity material: what the timed path produces for the first utterances of input set 0
     step_dev(0)
@@ -619,6 +651,8 @@ def main():
                     help="strong scaling: this many utterances in total, split over the ranks (configs[2]: 512)")
     ap.add_argument("--quantized", action="store_true", help="time the FakeQuantize model (configs[4] semantics)")
     ap.add_argument("--bind-cores", action="store_true", help="N > 1: pin each rank to its share of the GPU's cores")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's shard when N > 1)")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3

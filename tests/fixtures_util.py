@@ -55,3 +55,10 @@ def state_dict_digest(sd: dict) -> np.ndarray:
     """(n_tensors, 2) float64: sum and abs-sum per tensor in key order — proves two boxes
     drew the same random init without shipping 25 MB of weights."""
     return np.array([[float(v.double().sum()), float(v.double().abs().sum())] for _, v in sd.items()])
+
+
+def state_dict_fingerprint(sd: dict) -> list:
+    """'<key> <shape> <sha256 of the bytes>' per tensor in key order: equal lists mean equal trees, bit for bit."""
+    import hashlib
+    return [f"{k} {tuple(v.shape)} {hashlib.sha256(v.contiguous().numpy().tobytes()).hexdigest()}"
+            for k, v in sd.items()]

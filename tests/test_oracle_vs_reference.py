@@ -1,107 +1,91 @@
-"""Live comparison of the oracle with the unmodified reference, when it is importable
-(/root/reference in the build container, or baseline/_ref).  CPU only."""
+"""The oracle and the product's parameter tree on fresh seeds, against what the unmodified reference computed for
+the same inputs, recorded in tests/golden/oracle_vs_reference.npz (tests/golden/make_golden_oracle_vs_reference.py
+says which values are equal to the reference's and which are within its tolerance).  CPU only."""
+import ast
+
 import numpy as np
 import pytest
 import torch
 
 import fixtures_util as FU
 import velocity_oracle as O
-from refload import load_reference
 
-R = load_reference()
-pytestmark = pytest.mark.skipif(R is None, reason="reference tree not present on this box")
+# Recorded values that stand within 1e-4 (mel) / 5e-5 (logits) of the reference's are matched far tighter, so
+# the oracle stays as close to the reference as it was: the oracle is float64 throughout and a re-run differs
+# only in summation order; the recorded mel is float32.
+MEL_PIN = 1e-6
+LOGIT_PIN = 1e-9
 
 
 def rel(a, b):
     return float(np.abs(np.asarray(a, dtype=np.float64) - b).max() / (np.abs(b).max() + 1e-30))
 
 
-def test_mel_and_forward_fresh_seed():
+@pytest.fixture(scope="module")
+def g(golden):
+    return golden("oracle_vs_reference")
+
+
+def recorded(g, name):
+    return ast.literal_eval(str(g[name]))
+
+
+def test_mel_and_forward_fresh_seed(g):
+    import velocity_asr
     audio = FU.synth_audio(2, 24000, seed=321)
-    with torch.no_grad():
-        mel = R.compute_mel_spectrogram(audio)
-    assert np.abs(O.log_mel(audio.numpy()) - mel.numpy()).max() < 1e-4
+    mel = g["mel"]
+    assert np.abs(O.log_mel(audio.numpy()) - mel).max() < MEL_PIN
     for mode in ("sequential", "parallel"):
         torch.manual_seed(5)
-        m = R.VELOCITYASR(R.VelocityASRConfig(scan_mode=mode)).eval()
-        m.load_state_dict(FU.amplify_state_dict(m.state_dict(), seed=9))
-        sd = {k: v.numpy() for k, v in m.state_dict().items()}
-        with torch.no_grad():
-            ref = m(mel)
-        got = O.forward(mel.numpy(), sd, dict(scan_mode=mode))
-        assert rel(got, ref.numpy()) < 5e-5
-        assert O.ctc_greedy_decode(got) == R.ctc_greedy_decode(ref)
+        m = velocity_asr.VELOCITYASR(velocity_asr.VelocityASRConfig(scan_mode=mode))
+        sd = {k: v.numpy() for k, v in FU.amplify_state_dict(m.state_dict(), seed=9).items()}
+        got = O.forward(mel, sd, dict(scan_mode=mode))
+        assert rel(got[:, ::8], g[mode + "_logits_sub"]) < LOGIT_PIN
+        assert O.ctc_greedy_decode(got) == recorded(g, mode + "_tokens")
 
 
-def test_product_parameter_tree_draws_reference_weights():
+def test_product_parameter_tree_draws_reference_weights(g):
     import velocity_asr
-    torch.manual_seed(11)
-    a = R.VELOCITYASR(R.VelocityASRConfig()).state_dict()
     torch.manual_seed(11)
     b = velocity_asr.VELOCITYASR(velocity_asr.VelocityASRConfig()).state_dict()
-    assert list(a) == list(b)
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
+    assert FU.state_dict_fingerprint(b) == g["tree_seed11"].tolist()
 
 
-def test_yaml_mapping_matches_reference_defaults():
-    import os
-    import velocity_asr
-    path = "/root/reference/configs/model.yaml"
-    if not os.path.exists(path):
-        pytest.skip("configs/model.yaml only exists in the source tree")
-    c = velocity_asr.config_from_yaml(path)
-    r = R.VelocityASRConfig()
-    for f in ("mel_bins", "d_model", "ssm_layers", "ssm_state_dim", "ssm_expand_ratio", "ssm_kernel_size",
-              "global_ssm_layers", "global_ssm_state_dim", "attention_heads", "attention_dim", "vocab_size",
-              "scan_mode", "dropout"):
-        assert getattr(c, f) == getattr(r, f), f
-
-
-def test_timestamp_decode_matches_reference():
+def test_timestamp_decode_matches_reference(g):
     """decode.py:74-125 against the oracle's restatement, on run-heavy random predictions."""
     rs = np.random.RandomState(3)
-    for (B, L, V) in [(5, 97, 6), (3, 1, 4), (2, 300, 3), (1, 33, 2)]:
+    for i, (B, L, V) in enumerate([(5, 97, 6), (3, 1, 4), (2, 300, 3), (1, 33, 2)]):
         lg = rs.standard_normal((B, L, V)).astype(np.float32)
         lg[..., 0] += 0.8
         lg = np.repeat(lg, 2, axis=1)[:, :L]
-        ref = R.decode.ctc_greedy_decode_with_timestamps(torch.from_numpy(lg))
-        assert [(list(t), [tuple(x) for x in s]) for t, s in ref] == O.ctc_greedy_decode_with_timestamps(lg)
+        assert recorded(g, f"timestamps_{i}") == O.ctc_greedy_decode_with_timestamps(lg)
 
 
-def test_beam_search_matches_reference():
-    """decode.py:128-217 run live against the restatement fed with the reference's log-prob table."""
+def test_beam_search_matches_reference(g):
+    """decode.py:128-217 against the restatement fed with the reference's log-prob table."""
     rs = np.random.RandomState(5)
-    for (B, L, V, W, blank) in [(2, 18, 9, 4, 0), (1, 10, 4, 6, 1), (2, 9, 7, 1, 0), (1, 14, 5, 3, 4)]:
+    for i, (B, L, V, W, blank) in enumerate([(2, 18, 9, 4, 0), (1, 10, 4, 6, 1), (2, 9, 7, 1, 0), (1, 14, 5, 3, 4)]):
         lg = (np.round(rs.standard_normal((B, L, V)) * 3.0) / 3.0).astype(np.float32)
-        ref = R.decode.ctc_beam_search(torch.from_numpy(lg), beam_width=W, blank_token=blank)
         lp = torch.log_softmax(torch.from_numpy(lg), dim=-1).numpy()
         got = O.ctc_beam_search(lg, W, blank, log_probs=lp)
-        assert [[(d.tokens, d.score) for d in utt] for utt in ref] == got
+        assert recorded(g, f"beam_{i}") == got
 
 
-def test_non_default_local_stack_shapes():
+def test_non_default_local_stack_shapes(g):
     """A config whose LOCAL stack differs from the global one (ssm_kernel_size 3, expand_ratio 1, 3 layers, state 32):
     GlobalSSM keeps expand_ratio 2 / kernel_size 4 whatever the config says (ssm.py:529-538).  The product's parameter
     tree must draw the same tensors as the reference and the oracle (shape-driven) must follow it."""
     import velocity_asr
     kw = dict(ssm_layers=3, ssm_state_dim=32, ssm_expand_ratio=1, ssm_kernel_size=3, scan_mode="sequential")
     torch.manual_seed(21)
-    ref = R.VELOCITYASR(R.VelocityASRConfig(**kw)).eval()
-    torch.manual_seed(21)
-    ours = velocity_asr.VELOCITYASR(velocity_asr.VelocityASRConfig(**kw))
-    a, b = ref.state_dict(), ours.state_dict()
-    assert list(a) == list(b)
-    for k in a:
-        assert a[k].shape == b[k].shape and torch.equal(a[k], b[k]), k
+    a = velocity_asr.VELOCITYASR(velocity_asr.VelocityASRConfig(**kw)).state_dict()
+    assert FU.state_dict_fingerprint(a) == g["tree_nondefault"].tolist()
     assert a["local_ssm.layers.0.conv.weight"].shape[-1] == 3
     assert a["global_context.global_ssm.layers.0.conv.weight"].shape[-1] == 4
     assert a["global_context.global_ssm.layers.0.ssm.in_proj.weight"].shape[0] == 2 * 2 * 192
     sd = FU.amplify_state_dict(a, seed=4)
-    ref.load_state_dict(sd)
     audio = FU.synth_audio(2, 12000, seed=8)
-    with torch.no_grad():
-        mel = R.compute_mel_spectrogram(audio)
-        want = ref(mel).numpy()
-    got = O.forward(mel.numpy(), {k: v.numpy() for k, v in sd.items()}, dict(kw))
-    assert rel(got, want) < 5e-5
+    mel = g["nondefault_mel"]
+    assert np.abs(O.log_mel(audio.numpy()) - mel).max() < MEL_PIN
+    got = O.forward(mel, {k: v.numpy() for k, v in sd.items()}, dict(kw))
+    assert rel(got[:, ::8], g["nondefault_logits_sub"]) < LOGIT_PIN
