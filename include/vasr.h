@@ -147,6 +147,34 @@ int vasr_forward_ragged(vasr_handle* h, const float* mel_dev, const int32_t* fra
 int vasr_ctc_beam_search(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
                          int32_t* tokens_dev, int32_t* lens_dev, double* scores_dev, void* stream);
 
+/* ---- n-gram language model over token ids (ARPA), fused into the prefix beam search
+ * lm(prefix, tok), natural log: the history is ("<s>",) + prefix cut to its last order-1 items; P(w | h) = p(h w)
+ * when listed, else bow(h) + P(w | h[1:]) (bow of an unlisted context = 0); a token without a unigram takes the
+ * <unk> unigram.  Every ARPA value (log10) is parsed as fp64, times ln 10 in fp64, rounded once to fp32; the
+ * back-off sum is fp64 (the listed entry found, then the back-off weights from the shortest context outward),
+ * rounded to fp32.  An ARPA word maps to the vocabulary entry with the same string, <space> to " "; n-grams with a
+ * word outside the vocabulary are dropped, <s> is kept as a context, </s> is unused, the blank is never scored. */
+typedef struct vasr_lm vasr_lm;
+/* Parses the ARPA file at `path` for a vocabulary of V NUL-terminated UTF-8 strings and uploads its tables to
+ * `device` (< 0: the calling thread's current device).  Malformed files (bad header, section counts that differ
+ * from \data\, an unparsable number, no \end\), an order above 8, and a non-blank token with no unigram in a file
+ * without <unk> fail with VASR_ERR_INVALID and a message naming the line, before any device call. */
+int vasr_lm_create_arpa(const char* path, const char* const* vocab, int64_t V, int blank, int device, vasr_lm** out);
+void vasr_lm_destroy(vasr_lm* lm);
+int vasr_lm_order(const vasr_lm* lm);
+/* out[i] = lm(prefix_i, tokens[i]) fp32, n rows.  prefixes (n, max(order-1, 1)) int32 holds the last
+ * min(len_i, order-1) tokens of prefix i right-aligned (newest last); prefix_lens (n) its true length, so a prefix
+ * shorter than order-1 starts at <s>.  All device pointers on the LM's device; a token outside [0, V) gives NaN. */
+int vasr_lm_log_prob(const vasr_lm* lm, const int32_t* prefixes_dev, const int32_t* prefix_lens_dev, int64_t n,
+                     const int32_t* tokens_dev, float* out_dev, void* stream);
+/* vasr_ctc_beam_search with shallow fusion: an offer that extends a prefix by tok scores
+ * (score + log_prob[tok]) + lm_weight * lm(prefix, tok) in fp64; blank and repeat offers are unchanged.  Outputs as
+ * vasr_ctc_beam_search, scores are the fused ones.  The LM must be built for this V and blank, and logits_dev must be
+ * device memory on the LM's device (else VASR_ERR_INVALID); lm_weight finite.  1 <= beam_width <= 32. */
+int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
+                            const vasr_lm* lm, double lm_weight, int32_t* tokens_dev, int32_t* lens_dev,
+                            double* scores_dev, void* stream);
+
 /* ---- transcribe: load -> mel -> model -> greedy (scripts/transcribe.py:69-82), batched.
  * tokens (B, L) int32, lens (B); L = vasr_num_tokens(vasr_num_frames(S)). */
 int vasr_transcribe(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S,

@@ -12,10 +12,31 @@
 // beam_search_kernel then runs the frames in order, one warp per utterance, one beam per lane, scores in
 // fp64 (the reference adds Python floats), ties broken by the reference's insertion order
 // (beam rank, then blank, then token id).
+//
+// With an n-gram LM (beam_search_lm_kernel), an offer that extends a prefix scores
+//   (score + lp[tok]) + lm_weight * lm(prefix, tok)          fp64, in this order;
+// blank and repeat offers are unchanged.  One CTA per utterance, one warp per beam:
+//  * each beam keeps a dense fp32 row lm(prefix, .) over V in a slot of global memory.  A row is built only when
+//    a new prefix is created (at most W per frame) from the LM's suffix chain and continuation lists; blank and
+//    repeat survivors keep their prefix, their slot and their row;
+//  * each beam's warp lists its own W+1 best extension tokens by the fused offer (ties -> lower token id).  W+1
+//    still suffices: every entry ranked above a token x in that list is the beam's last token, or a token whose
+//    child prefix is already a beam — and that child's key scores at least the parent's offer (max-merge) and
+//    was inserted no later, so it outranks x too — or another extension that outranks x.  So if x makes the
+//    global top-W, at most W-1 entries above it are extensions or child keys, plus possibly `last`, whose repeat
+//    offer carries no LM term and need not dominate x: x is among the first W+1;
+//  * the parent's offer to a child beam needs lm(parent prefix, token), a property of the child's prefix: it is
+//    stored in the trie node when the node is created;
+//  * the rank / merge / selection loop is beam_search_kernel's, run by warp 0 (one lane per beam), with one change:
+//    trie nodes are canonical.  An extension that recreates a prefix seen before (it dropped out of the beams and
+//    comes back) reuses that prefix's node, found in its parent's child list, so "beam j's parent node is beam i's
+//    node" means "beam j's prefix extends beam i's" even then.  With an LM prefixes drop out and return often, and
+//    a fresh node would hide a surviving child from its recreated parent (two offers to one prefix, unmerged).
 #include <float.h>
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "lm.cuh"
 
 namespace vasr {
 
@@ -253,6 +274,346 @@ __global__ void __launch_bounds__(32) beam_search_kernel(
   }
 }
 
+// ---- the search with an n-gram LM ----------------------------------------------------------------------------
+constexpr int kLaneTop = 4;   // entries each lane buffers while a warp lists a beam's candidates
+
+// row[tok] = lm(prefix of `node`, tok) for every tok: the unigram row backed off through the whole history, then
+// the continuation lists of the listed suffixes, shortest first, so a longer listed context overwrites
+__device__ __forceinline__ void lm_build_row(const LmView& lm, const int32_t* parent, const int32_t* token,
+                                             const int32_t* depth, int node, float* row, int lane) {
+  const int d = depth[node];
+  const int k = min(lm.order - 1, d + 1);
+  int nd = node;
+  int ctx[kLmMaxOrder];
+  float bw[kLmMaxOrder];
+  const int m = lm_walk(lm, k, [&](int q) {
+    if (q > d) return lm.V;   // <s>
+    const int s = token[nd];
+    nd = parent[nd];
+    return s;
+  }, ctx, bw);
+  for (int tok = lane; tok < lm.V; tok += 32) row[tok] = lm_backoff(lm.uni[tok], 0, k, bw);
+  __syncwarp();
+#pragma unroll
+  for (int j = 1; j < kLmMaxOrder; ++j) {
+    if (j <= m) {
+      const int64_t e1 = lm.off[ctx[j] + 1];
+      for (int64_t e = lm.off[ctx[j]] + lane; e < e1; e += 32) row[lm.cont_tok[e]] = lm_backoff(lm.cont_lp[e], j, k, bw);
+    }
+    __syncwarp();
+  }
+}
+
+// One beam's K best extension tokens by fused offer (ties -> lower token id) -> c_tok / c_sc / c_lm[0 .. K), -1
+// padded.  Each lane buffers the kLaneTop best of its own tokens and refills after its last taken entry when the
+// buffer runs dry; the warp takes the best buffered head K times.
+__device__ __forceinline__ void lm_candidates(const float* x, float2 st, const float* row, double score, double lmw,
+                                              int V, int K, int blank, int lane, int* c_tok, double* c_sc,
+                                              float* c_lm) {
+  auto offer = [&](int tok) {
+    const double lp = (double)((x[tok] - st.x) - st.y);
+    return __dadd_rn(__dadd_rn(score, lp), __dmul_rn(lmw, (double)row[tok]));
+  };
+  double hv[kLaneTop];
+  int hi[kLaneTop];
+  double pv = INFINITY;
+  int pi = -1;
+  bool more = false;
+  auto refill = [&]() {
+#pragma unroll
+    for (int q = 0; q < kLaneTop; ++q) {
+      hv[q] = -INFINITY;
+      hi[q] = -1;
+    }
+    int cnt = 0;
+    for (int tok = lane; tok < V; tok += 32) {
+      if (tok == blank) continue;
+      const double v = offer(tok);
+      if (pi >= 0 && !(v < pv || (v == pv && tok > pi))) continue;   // taken already
+      ++cnt;
+      if (hi[kLaneTop - 1] >= 0 && !(v > hv[kLaneTop - 1])) continue;   // tokens ascend: a tie goes after
+      hv[kLaneTop - 1] = v;
+      hi[kLaneTop - 1] = tok;
+#pragma unroll
+      for (int q = kLaneTop - 1; q > 0; --q) {
+        if (hi[q - 1] < 0 || hv[q] > hv[q - 1]) {
+          const double tv = hv[q];
+          hv[q] = hv[q - 1];
+          hv[q - 1] = tv;
+          const int ti = hi[q];
+          hi[q] = hi[q - 1];
+          hi[q - 1] = ti;
+        }
+      }
+    }
+    more = cnt > kLaneTop;
+  };
+  refill();
+  for (int k = 0; k < K; ++k) {
+    double bv = hv[0];
+    int bi = hi[0];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+      if (oi >= 0 && (bi < 0 || ov > bv || (ov == bv && oi < bi))) {
+        bv = ov;
+        bi = oi;
+      }
+    }
+    if (bi < 0) {
+      for (int kk = k + lane; kk < K; kk += 32) c_tok[kk] = -1;
+      break;
+    }
+    if (hi[0] == bi) {   // the lane that owns the token
+      c_tok[k] = bi;
+      c_sc[k] = bv;
+      c_lm[k] = row[bi];
+      pv = bv;
+      pi = bi;
+#pragma unroll
+      for (int q = 0; q < kLaneTop - 1; ++q) {
+        hv[q] = hv[q + 1];
+        hi[q] = hi[q + 1];
+      }
+      hv[kLaneTop - 1] = -INFINITY;
+      hi[kLaneTop - 1] = -1;
+      if (hi[0] < 0 && more) refill();
+    }
+  }
+}
+
+__global__ void __launch_bounds__(512) beam_search_lm_kernel(
+    const float* __restrict__ logits, const float2* __restrict__ stats, const LmView lm, double lmw, int K,
+    int64_t L, int V, int W, int blank, int32_t* trie_parent, int32_t* trie_token, int32_t* trie_depth,
+    int32_t* trie_child, int32_t* trie_sibling, float* trie_lm, int64_t trie_cap, float* rows, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
+    double* __restrict__ out_scores) {
+  const int64_t b = blockIdx.x;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  int32_t* parent = trie_parent + b * trie_cap;
+  int32_t* token = trie_token + b * trie_cap;
+  int32_t* depth = trie_depth + b * trie_cap;
+  int32_t* first_child = trie_child + b * trie_cap;
+  int32_t* next_sibling = trie_sibling + b * trie_cap;
+  float* node_lm = trie_lm + b * trie_cap;   // lm(parent prefix, token) of each node
+  float* urows = rows + b * (int64_t)W * V;
+
+  // warp 0's selection state, as in beam_search_kernel
+  __shared__ int s_node[32], s_last[32], s_pl[32], s_tk[32], n_node[32], n_last[32], n_slot[32];
+  __shared__ double s_score[32], n_score[32];
+  // each beam's candidate list
+  __shared__ int c_tok[32][33];
+  __shared__ double c_sc[32][33];
+  __shared__ float c_lm[32][33];
+  // the beams as every warp sees them
+  __shared__ int b_node[32], b_slot[32], b_new[32], b_nb;
+  __shared__ double b_score[32];
+
+  if (threadIdx.x == 0) {
+    parent[0] = -1;
+    token[0] = -1;
+    depth[0] = 0;
+    first_child[0] = -1;
+    node_lm[0] = 0.f;
+    b_node[0] = 0;
+    b_slot[0] = 0;
+    b_new[0] = 1;
+    b_score[0] = 0.0;
+    b_nb = 1;
+  }
+  int nb = 1, n_nodes = 1;
+  int node = 0, last = -1, slot = 0;
+  double score = 0.0;
+  const long long Vp = (long long)V + 1;
+  __syncthreads();
+
+  for (int64_t t = 0; t < L; ++t) {
+    const int64_t rw = b * L + t;
+    const float* x = logits + rw * V;
+    const float2 st = stats[rw];
+    for (int w = warp; w < b_nb; w += nwarps) {
+      float* row = urows + (int64_t)b_slot[w] * V;
+      if (b_new[w]) lm_build_row(lm, parent, token, depth, b_node[w], row, lane);
+      lm_candidates(x, st, row, b_score[w], lmw, V, K, blank, lane, c_tok[w], c_sc[w], c_lm[w]);
+    }
+    __syncthreads();
+
+    if (warp == 0) {
+      auto lp = [&](int tok) -> double { return (double)((x[tok] - st.x) - st.y); };
+      const bool valid = lane < nb;
+
+      s_node[lane] = valid ? node : -2;
+      const int par = valid ? parent[node] : -3;
+      const int tk = valid ? token[node] : -1;
+      __syncwarp();
+      int pl = -1;
+      if (valid && par >= 0)
+        for (int j = 0; j < nb; ++j)
+          if (s_node[j] == par) pl = j;
+      s_pl[lane] = pl;
+      s_tk[lane] = tk;
+      s_last[lane] = last;
+      s_score[lane] = score;
+      __syncwarp();
+
+      double e_score = -INFINITY;
+      int e_last = blank;
+      long long e_order = kNoOrder;
+      bool e_avail = valid;
+      if (valid) {
+        double cs[3];
+        int cl[3];
+        long long co[3];
+        bool ch[3];
+        const bool h1 = pl >= 0 && s_last[pl] != tk;
+        const double sc1 = h1 ? __dadd_rn(__dadd_rn(s_score[pl], lp(tk)), __dmul_rn(lmw, (double)node_lm[node])) : 0.0;
+        const long long o1 = (long long)pl * Vp + 1 + tk;
+        const bool h3 = last >= 0 && last != blank;
+        const double sc3 = h3 ? score + lp(last) : 0.0;
+        const int first = (h1 && pl < lane) ? 0 : 2;
+        const int i2 = first == 0 ? 1 : 0, i3 = i2 + 1;
+        cs[first] = sc1, cl[first] = tk, co[first] = o1, ch[first] = h1;
+        cs[i2] = score + lp(blank), cl[i2] = blank, co[i2] = (long long)lane * Vp, ch[i2] = true;
+        cs[i3] = sc3, cl[i3] = last, co[i3] = (long long)lane * Vp + 1 + last, ch[i3] = h3;
+        bool none = true;
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          if (!ch[i]) continue;
+          if (none || cs[i] > e_score) {
+            e_score = cs[i];
+            e_last = cl[i];
+          }
+          if (none) e_order = co[i];
+          none = false;
+        }
+      }
+
+      int p = valid ? 0 : K;
+      int x_tok = -1;
+      double x_score = -INFINITY;
+      auto advance = [&]() {
+        while (p < K) {
+          const int tok = c_tok[lane][p];
+          if (tok < 0) {
+            p = K;
+            break;
+          }
+          bool skip = tok == last;
+          for (int j = 0; j < nb && !skip; ++j) skip = s_pl[j] == lane && s_tk[j] == tok;
+          if (!skip) {
+            x_tok = tok;
+            x_score = c_sc[lane][p];
+            return;
+          }
+          ++p;
+        }
+      };
+      advance();
+
+      int count = 0;
+      for (int r = 0; r < W; ++r) {
+        const bool hx = p < K;
+        const long long x_order = (long long)lane * Vp + 1 + x_tok;
+        bool take_e = e_avail;
+        if (e_avail && hx) take_e = e_score > x_score || (e_score == x_score && e_order < x_order);
+        double ps = take_e ? e_score : (hx ? x_score : -INFINITY);
+        long long po = take_e ? e_order : (hx ? x_order : kNoOrder);
+        double bs = ps;
+        long long bo = po;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          const double os = __shfl_xor_sync(0xffffffffu, bs, o);
+          const long long oo = __shfl_xor_sync(0xffffffffu, bo, o);
+          if (oo != kNoOrder && (bo == kNoOrder || os > bs || (os == bs && oo < bo))) {
+            bs = os;
+            bo = oo;
+          }
+        }
+        if (bo == kNoOrder) break;
+        const bool mine = po == bo;
+        bool created = false;
+        if (mine) {
+          if (take_e) {
+            n_node[r] = node;
+            n_score[r] = e_score;
+            n_last[r] = e_last;
+            n_slot[r] = slot;
+            e_avail = false;
+          } else {
+            int c = first_child[node];
+            while (c >= 0 && token[c] != x_tok) c = next_sibling[c];
+            if (c < 0) {
+              c = n_nodes;
+              parent[c] = node;
+              token[c] = x_tok;
+              depth[c] = depth[node] + 1;
+              node_lm[c] = c_lm[lane][p];
+              first_child[c] = -1;
+              next_sibling[c] = first_child[node];
+              first_child[node] = c;
+              created = true;
+            }
+            n_node[r] = c;
+            n_score[r] = x_score;
+            n_last[r] = x_tok;
+            n_slot[r] = -1;
+            ++p;
+            advance();
+          }
+        }
+        n_nodes += __ballot_sync(0xffffffffu, created) != 0;
+        ++count;
+      }
+      __syncwarp();
+      nb = count;
+      int ns = -1;
+      if (lane < nb) {
+        node = n_node[lane];
+        score = n_score[lane];
+        last = n_last[lane];
+        ns = n_slot[lane];
+      }
+      // survivors keep their row slot; new prefixes take the free ones, in beam order
+      const bool fresh = lane < nb && ns < 0;
+      const unsigned used = __reduce_or_sync(0xffffffffu, (lane < nb && ns >= 0) ? 1u << ns : 0u);
+      const unsigned freshm = __ballot_sync(0xffffffffu, fresh);
+      if (fresh) {
+        unsigned fr = ~used;
+        for (int q = __popc(freshm & ((1u << lane) - 1u)); q > 0; --q) fr &= fr - 1u;
+        ns = __ffs(fr) - 1;
+      }
+      slot = ns;
+      if (lane < nb) {
+        b_node[lane] = node;
+        b_slot[lane] = slot;
+        b_new[lane] = fresh;
+        b_score[lane] = score;
+      }
+      if (lane == 0) b_nb = nb;
+    }
+    __syncthreads();
+  }
+
+  if (warp == 0 && lane < W) {
+    int32_t* out = out_tokens + (b * W + lane) * L;
+    if (lane < nb) {
+      const int len = depth[node];
+      out_scores[b * W + lane] = score;
+      out_lens[b * W + lane] = len;
+      int nd = node;
+      for (int i = len - 1; i >= 0; --i) {
+        out[i] = token[nd];
+        nd = parent[nd];
+      }
+      for (int64_t i = len; i < L; ++i) out[i] = -1;
+    } else {
+      out_scores[b * W + lane] = -INFINITY;
+      out_lens[b * W + lane] = -1;
+      for (int64_t i = 0; i < L; ++i) out[i] = -1;
+    }
+  }
+}
+
 }  // namespace
 
 cudaError_t launch_beam_rows(const float* logits, float2* stats, int32_t* top_tok, int64_t M, int V, int K,
@@ -272,6 +633,20 @@ cudaError_t launch_beam_search(const float* logits, const float2* stats, const i
                                                 trie + B * trie_cap, trie + 2 * B * trie_cap, trie_cap, out_tokens,
                                                 out_lens, out_scores);
   if (launches) ++*launches;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_beam_search_lm(const float* logits, const float2* stats, const LmView& lm, double lm_weight,
+                                  int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_lm,
+                                  int64_t trie_cap, float* rows, int32_t* out_tokens, int32_t* out_lens,
+                                  double* out_scores, cudaStream_t s) {
+  if (B <= 0) return cudaSuccess;
+  const int K = V - 1 < W + 1 ? (V - 1 > 0 ? V - 1 : 1) : W + 1;
+  const int warps = W < 16 ? W : 16;
+  beam_search_lm_kernel<<<(unsigned)B, 32 * warps, 0, s>>>(logits, stats, lm, lm_weight, K, L, V, W, blank, trie,
+                                                           trie + B * trie_cap, trie + 2 * B * trie_cap,
+                                                           trie + 3 * B * trie_cap, trie + 4 * B * trie_cap, trie_lm,
+                                                           trie_cap, rows, out_tokens, out_lens, out_scores);
   return cudaGetLastError();
 }
 

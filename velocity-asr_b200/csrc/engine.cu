@@ -13,6 +13,7 @@
 #include "../../include/vasr.h"
 #include "common.cuh"
 #include "kernels.cuh"
+#include "lm.cuh"
 
 using namespace vasr;
 
@@ -1262,6 +1263,104 @@ int vasr_ctc_beam_search(const float* logits_dev, int64_t B, int64_t L, int64_t 
   CK(cudaFreeAsync(stats, s));
   CK(cudaFreeAsync(top, s));
   CK(cudaFreeAsync(trie, s));
+  return VASR_OK;
+}
+
+struct vasr_lm {
+  int device = 0, blank = 0;
+  void* block = nullptr;   // every device table (lm.cu)
+  LmView view;
+};
+
+int vasr_lm_create_arpa(const char* path, const char* const* vocab, int64_t V, int blank, int device, vasr_lm** out) {
+  if (!path || !vocab || !out) return fail(VASR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (V < 1 || V >= 0x7fffffff) return fail(VASR_ERR_INVALID, "vocabulary size must be in [1, 2^31 - 1)");
+  if (blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  LmHostTables t;
+  std::string err;
+  if (!lm_parse_arpa(path, vocab, (int)V, blank, &t, &err)) return fail(VASR_ERR_INVALID, err);
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(VASR_ERR_CUDA, "no CUDA device: libvasr has no CPU path");
+  if (device < 0) CK(cudaGetDevice(&device));
+  if (device >= ndev) return fail(VASR_ERR_INVALID, "bad device index");
+  DeviceGuard dev_guard(device);
+  vasr_lm* lm = new vasr_lm;
+  lm->device = device;
+  lm->blank = blank;
+  const cudaError_t e = lm_upload(t, &lm->block, &lm->view);
+  if (e != cudaSuccess) {
+    delete lm;
+    return fail(VASR_ERR_CUDA, std::string("LM upload: ") + cudaGetErrorString(e));
+  }
+  *out = lm;
+  return VASR_OK;
+}
+
+void vasr_lm_destroy(vasr_lm* lm) {
+  if (!lm) return;
+  DeviceGuard dev_guard(lm->device);
+  cudaFree(lm->block);
+  delete lm;
+}
+
+int vasr_lm_order(const vasr_lm* lm) { return lm ? lm->view.order : 0; }
+
+int vasr_lm_log_prob(const vasr_lm* lm, const int32_t* prefixes_dev, const int32_t* prefix_lens_dev, int64_t n,
+                     const int32_t* tokens_dev, float* out_dev, void* stream) {
+  if (!lm || n < 0) return fail(VASR_ERR_INVALID, "null argument");
+  if (n == 0) return VASR_OK;
+  if (!prefixes_dev || !prefix_lens_dev || !tokens_dev || !out_dev) return fail(VASR_ERR_INVALID, "null argument");
+  DeviceGuard dev_guard(lm->device);
+  KL(launch_lm_log_prob(lm->view, prefixes_dev, prefix_lens_dev, n, tokens_dev, out_dev,
+                        static_cast<cudaStream_t>(stream)));
+  return VASR_OK;
+}
+
+int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
+                            const vasr_lm* lm, double lm_weight, int32_t* tokens_dev, int32_t* lens_dev,
+                            double* scores_dev, void* stream) {
+  if (!lm) return fail(VASR_ERR_INVALID, "null LM");
+  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
+  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
+  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  if (V != lm->view.V)
+    return fail(VASR_ERR_INVALID, "the LM is built for a vocabulary of " + std::to_string(lm->view.V) +
+                                      " tokens, the logits have " + std::to_string(V));
+  if (blank != lm->blank)
+    return fail(VASR_ERR_INVALID, "the LM is built with blank token " + std::to_string(lm->blank) +
+                                      ", the search uses " + std::to_string(blank));
+  if (!std::isfinite(lm_weight)) return fail(VASR_ERR_INVALID, "lm_weight must be finite");
+  if (B <= 0) return VASR_OK;
+  if (B * L > 0) {
+    cudaPointerAttributes at = {};
+    if (cudaPointerGetAttributes(&at, logits_dev) != cudaSuccess || at.type == cudaMemoryTypeUnregistered ||
+        at.type == cudaMemoryTypeHost || at.device != lm->device) {
+      cudaGetLastError();
+      return fail(VASR_ERR_INVALID, "the logits are not device memory on the LM's device (" +
+                                        std::to_string(lm->device) + ")");
+    }
+  }
+  DeviceGuard dev_guard(lm->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int W = beam_width;
+  const int64_t M = B * L, cap = 1 + L * W;
+  float2* stats = nullptr;
+  int32_t* trie = nullptr;
+  float *trie_lm = nullptr, *rows = nullptr;
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)5 * B * cap * sizeof(int32_t), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie_lm), (size_t)B * cap * sizeof(float), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&rows), (size_t)B * W * V * sizeof(float), s));
+  KL(launch_beam_rows(logits_dev, stats, nullptr, M, (int)V, 0, blank, s, nullptr));   // log-softmax stats only
+  KL(launch_beam_search_lm(logits_dev, stats, lm->view, lm_weight, B, L, (int)V, W, blank, trie, trie_lm, cap, rows,
+                           tokens_dev, lens_dev, scores_dev, s));
+  CK(cudaFreeAsync(stats, s));
+  CK(cudaFreeAsync(trie, s));
+  CK(cudaFreeAsync(trie_lm, s));
+  CK(cudaFreeAsync(rows, s));
   return VASR_OK;
 }
 

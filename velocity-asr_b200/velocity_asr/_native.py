@@ -2,7 +2,7 @@
 missing, or there is no CUDA device, every compute entry point raises."""
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_float, c_int, c_int32, c_int64, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VASR_LIB") or os.path.join(_HERE, "libvasr.so")   # VASR_LIB: A/B runs of two builds
@@ -40,6 +40,12 @@ _SIGNATURES = {
                                            c_void_p, c_void_p]),
     "vasr_ctc_beam_search": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                      c_void_p]),
+    "vasr_lm_create_arpa": (c_int, [c_char_p, c_void_p, c_int64, c_int, c_int, POINTER(c_void_p)]),
+    "vasr_lm_destroy": (None, [c_void_p]),
+    "vasr_lm_order": (c_int, [c_void_p]),
+    "vasr_lm_log_prob": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "vasr_ctc_beam_search_lm": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_double,
+                                        c_void_p, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "vasr_transcribe_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),

@@ -7,6 +7,7 @@ from typing import Any, List, Optional, Tuple
 import torch
 
 from . import _native
+from .lm import NGramLM
 
 BLANK_TOKEN = 0  # decode.py:14
 
@@ -111,14 +112,31 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
                     lm_weight: float = 0.0, lm_scorer: Optional[Any] = None) -> List[List[DecodingResult]]:
     """decode.py:128-217 on the GPU: per utterance the `beam_width` best prefixes, best first, with the
     reference's rule (log_softmax; blank / repeated token keep the prefix, any other token extends it; equal
-    prefixes keep the better score; fp64 score sums; ties in insertion order).  A Python `lm_scorer` cannot
-    run inside the device loop and is refused rather than silently ignored."""
-    if lm_scorer is not None and lm_weight > 0:
+    prefixes keep the better score; fp64 score sums; ties in insertion order).
+
+    Shallow fusion: with an NGramLM as `lm_scorer` and lm_weight > 0, an offer that extends a prefix by `tok`
+    scores (score + log_prob[tok]) + lm_weight * lm(prefix, tok); blank and repeat offers are unchanged and the
+    returned scores are the fused ones.  The LM must be built for this vocabulary size and blank token and live on
+    the logits' device (host logits are staged to it).  A Python `lm_scorer` callback cannot run inside the device
+    loop and is refused rather than silently ignored."""
+    use_lm = isinstance(lm_scorer, NGramLM) and lm_weight > 0
+    if lm_scorer is not None and lm_weight > 0 and not use_lm:
         raise NotImplementedError("velocity_asr (B200 build): ctc_beam_search runs on the device and takes no "
-                                  "Python lm_scorer")
+                                  "Python lm_scorer (use velocity_asr.NGramLM)")
     if logits.dim() != 3:
         raise RuntimeError(f"expected (batch, seq_len, vocab) logits, got {tuple(logits.shape)}")
-    if logits.device.type != "cuda":       # host logits: staged to the current CUDA device (no CPU decoder exists)
+    if use_lm:
+        lm_scorer._live()
+        if logits.shape[-1] != lm_scorer.vocab_size:
+            raise ValueError(f"the LM is built for a vocabulary of {lm_scorer.vocab_size} tokens, the logits have "
+                             f"{logits.shape[-1]}")
+        if int(blank_token) != lm_scorer.blank_token:
+            raise ValueError(f"the LM is built with blank token {lm_scorer.blank_token}, the search uses {blank_token}")
+        if logits.device.type != "cuda":   # host logits: staged to the LM's device
+            logits = logits.to(lm_scorer.device)
+        elif logits.device != lm_scorer.device:
+            raise ValueError(f"the LM is on {lm_scorer.device}, the logits on {logits.device}")
+    elif logits.device.type != "cuda":     # host logits: staged to the current CUDA device (no CPU decoder exists)
         logits = logits.to(_native.default_cuda_device())
     B, L, V = logits.shape
     W = int(beam_width)
@@ -130,9 +148,15 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     scores = torch.empty(B, W, dtype=torch.float64, device=lg.device)
     lib = _native.lib()
     with torch.cuda.device(lg.device):
-        _native.check(lib.vasr_ctc_beam_search(
-            _native.ptr(lg), B, L, V, W, int(blank_token), _native.ptr(tokens), _native.ptr(lens),
-            _native.ptr(scores), ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)))
+        stream = ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)
+        if use_lm:
+            _native.check(lib.vasr_ctc_beam_search_lm(
+                _native.ptr(lg), B, L, V, W, int(blank_token), lm_scorer._handle, float(lm_weight),
+                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), stream))
+        else:
+            _native.check(lib.vasr_ctc_beam_search(
+                _native.ptr(lg), B, L, V, W, int(blank_token), _native.ptr(tokens), _native.ptr(lens),
+                _native.ptr(scores), stream))
     tokens, lens, scores = tokens.cpu().numpy(), lens.cpu().tolist(), scores.cpu().tolist()
     return [[DecodingResult(text="", tokens=tokens[b, r, :n].tolist(), score=scores[b][r])
              for r, n in enumerate(lens[b]) if n >= 0] for b in range(B)]
@@ -151,9 +175,12 @@ class CTCDecoder:
         seqs = ctc_greedy_decode(logits, blank_token=self.blank_token, collapse_repeated=collapse_repeated)
         return [self._tokens_to_text(s) for s in seqs]
 
-    def decode_beam_search(self, logits: torch.Tensor, beam_width: int = 10, return_all_beams: bool = False):
-        """decode.py:265-300: best-beam texts, or every beam with its text filled in."""
-        beams = ctc_beam_search(logits, beam_width=beam_width, blank_token=self.blank_token)
+    def decode_beam_search(self, logits: torch.Tensor, beam_width: int = 10, return_all_beams: bool = False,
+                           lm_scorer: Optional[Any] = None, lm_weight: float = 0.0):
+        """decode.py:265-300: best-beam texts, or every beam with its text filled in.  `lm_scorer` / `lm_weight`
+        go to ctc_beam_search (shallow fusion with an NGramLM)."""
+        beams = ctc_beam_search(logits, beam_width=beam_width, blank_token=self.blank_token, lm_weight=lm_weight,
+                                lm_scorer=lm_scorer)
         if return_all_beams:
             for utt in beams:
                 for r in utt:
