@@ -175,6 +175,45 @@ int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64
                             const vasr_lm* lm, double lm_weight, int32_t* tokens_dev, int32_t* lens_dev,
                             double* scores_dev, void* stream);
 
+/* ---- word-level n-gram LM over a character vocabulary, fused into the prefix beam search
+ * The LM above over the file's own words: word id = index in the unigram section (first occurrence, <s> excluded),
+ * <s> is the context symbol, </s> and <unk> are ordinary words; lm(h, w) is the rule above over word ids.
+ * d = the vocabulary entry `delimiter` (the first one).  Spelling: a word's characters (UTF-8 code points), one
+ * token each, the first vocabulary entry with that one-character string, which must be neither the blank nor d;
+ * a word that cannot be spelled stays in the LM but not in the lexicon = the spellable unigram words other than
+ * <s>, </s>, <unk>.
+ * A prefix P (collapsed token ids) splits at each d into runs: the non-empty runs before the last d are its words
+ * w_1 .. w_k, the tokens after the last d its pending run u (possibly empty); word(run) = the lexicon word spelled
+ * by the run, else <unk>;
+ * h(P) = (<s>, word(w_1), ..., word(w_k)) cut to its last order-1 items.
+ * Offers from hypothesis (P, s, last) at a frame with fp32 log-softmax lp, summed in fp64 in exactly this order:
+ *   blank, repeat of last: P kept, s + lp[tok], no LM term (as vasr_ctc_beam_search);
+ *   d (d != last): u empty -> P+d, s + lp[d]; else ((s + lp[d]) + lm_weight * lm(h(P), word(u))) + word_score;
+ *     constrained: not offered when u is non-empty and not a lexicon word;
+ *   any other t: P+t, s + lp[t]; constrained: offered only when u+t is a prefix of a lexicon word's spelling.
+ *   Max-merge, first offer wins a tie, the stable top beam_width: as vasr_ctc_beam_search.
+ * End of utterance, per surviving hypothesis, in order: (1) u non-empty: constrained and u not a lexicon word ->
+ * dropped (len -1, as a missing beam); else s = (s + lm_weight * lm(h, word(u))) + word_score and word(u) joins the
+ * history; (2) s += lm_weight * lm(h', </s>) (</s> absent from the file: <unk>); (3) a stable sort by s, descending.
+ * L = 0 gives the empty beam with lm_weight * lm((<s>), </s>). */
+/* Parses a word ARPA file and builds the lexicon for a vocabulary of V strings; constrained != 0 limits hypotheses
+ * to lexicon words.  VASR_ERR_INVALID, before any device call, for: a delimiter missing from the vocabulary or equal
+ * to the blank, the malformed files of vasr_lm_create_arpa (naming the line), lexicon-free mode without <unk>, a
+ * file with neither </s> nor <unk>, constrained mode with an empty lexicon.  vasr_lm_order, vasr_lm_destroy and
+ * vasr_lm_log_prob (over word ids) take the result. */
+int vasr_lm_create_word_arpa(const char* path, const char* const* vocab, int64_t V, int blank, const char* delimiter,
+                             int constrained, int device, vasr_lm** out);
+/* ids_host[i] = the word id of words[i]; a string that is not a word of the LM maps to <unk> (fails without one). */
+int vasr_lm_word_ids(const vasr_lm* lm, const char* const* words, int64_t n, int32_t* ids_host);
+/* The lexicon size of a word LM, -1 for a token LM. */
+int64_t vasr_lm_lexicon_size(const vasr_lm* lm);
+/* The search with a word LM, outputs as vasr_ctc_beam_search_lm; returned scores are the final ones (after the end
+ * of utterance).  lm_weight finite and >= 0, word_score finite.  A token LM here, or a word LM given to
+ * vasr_ctc_beam_search_lm, fails with VASR_ERR_INVALID. */
+int vasr_ctc_beam_search_word_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
+                                 const vasr_lm* lm, double lm_weight, double word_score, int32_t* tokens_dev,
+                                 int32_t* lens_dev, double* scores_dev, void* stream);
+
 /* ---- transcribe: load -> mel -> model -> greedy (scripts/transcribe.py:69-82), batched.
  * tokens (B, L) int32, lens (B); L = vasr_num_tokens(vasr_num_frames(S)). */
 int vasr_transcribe(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S,

@@ -614,6 +614,377 @@ __global__ void __launch_bounds__(512) beam_search_lm_kernel(
   }
 }
 
+// ---- the search with a word LM ---------------------------------------------------------------------------------
+// Words are spelled in the character vocabulary and closed by the delimiter d (include/vasr.h states the rule).
+// Only the offer by d that closes a non-empty pending run u carries a term, ((score + lp[d]) + lm_weight *
+// lm(h, word(u))) + word_score; every other extension scores score + lp[tok].  In constrained mode a beam may only
+// offer tokens that keep u on a lexicon word's spelling, and d only when u is empty or a lexicon word.
+// One CTA per utterance, one warp per beam, beam_search_lm_kernel's canonical trie and warp 0's rank / merge /
+// selection loop, but no V-wide LM rows.  Each trie node holds, set when it is created: its spelling-trie node
+// (0: u is empty, -1: u is off the lexicon), the latest node at or above it whose token closed a word, the word
+// that token closed, and how many words its prefix has closed — so the word history is a walk up closing nodes.
+// lm(h, word(u)) is cached per node the first time a beam sits on it.
+// W+1 suffices again: among a beam's offers the non-d ones rank by lp alone (the same score is added), and d is
+// a single extra entry.  In lexicon-free mode every non-blank token is allowed, so a non-d token outside the
+// frame's W+2 best non-blank tokens (beam_rows_kernel, ties -> lower id) has at least W+1 non-d offers above it
+// in the beam's list; in constrained mode the allowed non-d tokens are the spelling node's children.  So the
+// beam's W+1 best fused offers are among those tokens plus d, and the argument of beam_search_lm_kernel (every
+// entry above a token x is `last`, a child key that outranks x, or an extension that outranks x) shows that a
+// token making the global top W is among the beam's first W+1.  The parent's offer to a child beam is the same
+// function of the parent's state.  After the last frame: close each beam's pending run (constrained: drop the
+// beam when it is not a lexicon word), add lm_weight * lm(h, </s>), and sort the beams stably by that score.
+struct WordTrie {
+  int32_t *parent, *token, *depth, *first_child, *next_sibling;
+  int32_t *lex, *closer, *word, *nwords;   // spelling node, latest closing node (-1: none), word closed, words so far
+  float* close_lm;                         // lm(h, word(u)) of the node's prefix, NaN until computed
+};
+
+// lm(h(node) [+ extra], w): the node's word history, with `extra` (>= 0) appended as the newest word
+__device__ __forceinline__ float word_lm(const LmView& lm, const WordTrie& tr, int node, int extra, int w) {
+  int hn = tr.closer[node];
+  bool first = extra >= 0;
+  const int k = min(lm.order - 1, tr.nwords[node] + (first ? 1 : 0) + 1);
+  return lm_score(lm, k, [&](int) {
+    if (first) {
+      first = false;
+      return extra;
+    }
+    if (hn < 0) return lm.V;   // <s>
+    const int s = tr.word[hn];
+    hn = tr.closer[tr.parent[hn]];
+    return s;
+  }, w);
+}
+
+__device__ __forceinline__ int word_of(const LexView& lx, int ln) {
+  const int w = ln >= 0 ? lx.word[ln] : -1;
+  return w >= 0 ? w : lx.unk;
+}
+
+// the offer by d from a beam: ((score + lp) + lmw * lm) + ws when it closes a word, else score + lp
+__device__ __forceinline__ double word_offer(double score, double lp, bool closes, float lm, double lmw, double ws) {
+  const double s = __dadd_rn(score, lp);
+  return closes ? __dadd_rn(__dadd_rn(s, __dmul_rn(lmw, (double)lm)), ws) : s;
+}
+
+__global__ void __launch_bounds__(512, 1) beam_search_word_lm_kernel(
+    const float* __restrict__ logits, const float2* __restrict__ stats, const int32_t* __restrict__ top_tok, int K,
+    const LmView lm, const LexView lx, double lmw, double ws, int64_t L, int V, int W, int blank, int32_t* trie,
+    float* trie_f, int64_t trie_cap, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
+    double* __restrict__ out_scores) {
+  const int64_t b = blockIdx.x;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  const int64_t pb = (int64_t)gridDim.x * trie_cap;   // one plane of the trie
+  int32_t* base = trie + b * trie_cap;
+  const WordTrie tr{base,          base + pb,     base + 2 * pb, base + 3 * pb, base + 4 * pb,
+                    base + 5 * pb, base + 6 * pb, base + 7 * pb, base + 8 * pb, trie_f + b * trie_cap};
+  const int d = lx.delim;
+  const int KC = W + 1;   // entries of each beam's candidate list
+
+  __shared__ int s_node[32], s_last[32], s_pl[32], s_tk[32], n_node[32], n_last[32];
+  __shared__ double s_score[32], n_score[32];
+  __shared__ int c_tok[32][33], c_lex[32][33];
+  __shared__ double c_sc[32][33];
+  __shared__ int b_node[32], b_lex[32], b_nb;
+  __shared__ float b_dlm[32];
+  __shared__ double b_score[32];
+
+  if (threadIdx.x == 0) {
+    tr.parent[0] = -1;
+    tr.token[0] = -1;
+    tr.depth[0] = 0;
+    tr.first_child[0] = -1;
+    tr.lex[0] = 0;
+    tr.closer[0] = -1;
+    tr.nwords[0] = 0;
+    tr.close_lm[0] = __int_as_float(0x7fffffff);
+    b_node[0] = 0;
+    b_score[0] = 0.0;
+    b_nb = 1;
+  }
+  int nb = 1, n_nodes = 1;
+  int node = 0, last = -1;
+  double score = 0.0;
+  const long long Vp = (long long)V + 1;
+  __syncthreads();
+
+  for (int64_t t = 0; t < L; ++t) {
+    const int64_t rw = b * L + t;
+    const float* x = logits + rw * V;
+    const float2 st = stats[rw];
+    auto lp = [&](int tok) -> double { return (double)((x[tok] - st.x) - st.y); };
+
+    // each beam's W+1 best offers, selection passes over its allowed tokens plus d (ties -> lower token id)
+    for (int w = warp; w < b_nb; w += nwarps) {
+      const int bn = b_node[w];
+      const double s = b_score[w];
+      const int ln = tr.lex[bn];
+      const bool d_ok = ln == 0 || !lx.constrained || (ln > 0 && lx.word[ln] >= 0);
+      const bool closes = ln != 0;
+      float dlm = 0.f;
+      if (closes && d_ok) {
+        dlm = tr.close_lm[bn];
+        if (isnan(dlm)) {
+          if (lane == 0) {
+            dlm = word_lm(lm, tr, bn, -1, word_of(lx, ln));
+            tr.close_lm[bn] = dlm;
+          }
+          dlm = __shfl_sync(0xffffffffu, dlm, 0);
+        }
+      }
+      const int lo = lx.constrained ? lx.off[ln] : 0;
+      const int n = (lx.constrained ? lx.off[ln + 1] - lo : K) + 1;   // the last entry is d
+      const int32_t* top = top_tok + rw * K;
+      auto cand = [&](int i, int& tok, double& v) {
+        if (i == n - 1) {
+          tok = d;
+          v = word_offer(s, lp(d), closes, dlm, lmw, ws);
+          return d_ok;
+        }
+        tok = lx.constrained ? lx.tok[lo + i] : top[i];
+        v = __dadd_rn(s, tok >= 0 ? lp(tok) : 0.0);
+        return tok >= 0 && tok != d;
+      };
+      double pv = INFINITY;
+      int pi = -1, cnt = 0;
+      for (int k = 0; k < KC; ++k) {
+        double bv = -INFINITY;
+        int bi = 0x7fffffff;
+        for (int i = lane; i < n; i += 32) {
+          int tok;
+          double v;
+          if (!cand(i, tok, v)) continue;
+          const bool after = v < pv || (v == pv && tok > pi);
+          if (after && (bi == 0x7fffffff || v > bv || (v == bv && tok < bi))) {
+            bv = v;
+            bi = tok;
+          }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+          const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+          if (oi != 0x7fffffff && (bi == 0x7fffffff || ov > bv || (ov == bv && oi < bi))) {
+            bv = ov;
+            bi = oi;
+          }
+        }
+        if (bi == 0x7fffffff) break;
+        if (lane == 0) {
+          c_tok[w][k] = bi;
+          c_sc[w][k] = bv;
+        }
+        pv = bv;
+        pi = bi;
+        ++cnt;
+      }
+      __syncwarp();
+      // the spelling node each listed extension leads to
+      for (int k = lane; k < KC; k += 32) {
+        if (k >= cnt) {
+          c_tok[w][k] = -1;
+          continue;
+        }
+        const int tok = c_tok[w][k];
+        c_lex[w][k] = tok == d ? 0 : lex_child(lx, ln, tok);
+      }
+      if (lane == 0) {
+        b_lex[w] = ln;
+        b_dlm[w] = dlm;
+      }
+    }
+    __syncthreads();
+
+    if (warp == 0) {
+      const bool valid = lane < nb;
+      s_node[lane] = valid ? node : -2;
+      const int par = valid ? tr.parent[node] : -3;
+      const int tk = valid ? tr.token[node] : -1;
+      __syncwarp();
+      int pl = -1;
+      if (valid && par >= 0)
+        for (int j = 0; j < nb; ++j)
+          if (s_node[j] == par) pl = j;
+      s_pl[lane] = pl;
+      s_tk[lane] = tk;
+      s_last[lane] = last;
+      s_score[lane] = score;
+      __syncwarp();
+
+      double e_score = -INFINITY;
+      int e_last = blank;
+      long long e_order = kNoOrder;
+      bool e_avail = valid;
+      if (valid) {
+        double cs[3];
+        int cl[3];
+        long long co[3];
+        bool ch[3];
+        const bool h1 = pl >= 0 && s_last[pl] != tk;
+        const double sc1 =
+            h1 ? (tk == d ? word_offer(s_score[pl], lp(tk), b_lex[pl] != 0, b_dlm[pl], lmw, ws) : s_score[pl] + lp(tk))
+               : 0.0;
+        const long long o1 = (long long)pl * Vp + 1 + tk;
+        const bool h3 = last >= 0 && last != blank;
+        const double sc3 = h3 ? score + lp(last) : 0.0;
+        const int first = (h1 && pl < lane) ? 0 : 2;
+        const int i2 = first == 0 ? 1 : 0, i3 = i2 + 1;
+        cs[first] = sc1, cl[first] = tk, co[first] = o1, ch[first] = h1;
+        cs[i2] = score + lp(blank), cl[i2] = blank, co[i2] = (long long)lane * Vp, ch[i2] = true;
+        cs[i3] = sc3, cl[i3] = last, co[i3] = (long long)lane * Vp + 1 + last, ch[i3] = h3;
+        bool none = true;
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          if (!ch[i]) continue;
+          if (none || cs[i] > e_score) {
+            e_score = cs[i];
+            e_last = cl[i];
+          }
+          if (none) e_order = co[i];
+          none = false;
+        }
+      }
+
+      int p = valid ? 0 : KC;
+      int x_tok = -1;
+      double x_score = -INFINITY;
+      auto advance = [&]() {
+        while (p < KC) {
+          const int tok = c_tok[lane][p];
+          if (tok < 0) {
+            p = KC;
+            break;
+          }
+          bool skip = tok == last;
+          for (int j = 0; j < nb && !skip; ++j) skip = s_pl[j] == lane && s_tk[j] == tok;
+          if (!skip) {
+            x_tok = tok;
+            x_score = c_sc[lane][p];
+            return;
+          }
+          ++p;
+        }
+      };
+      advance();
+
+      int count = 0;
+      for (int r = 0; r < W; ++r) {
+        const bool hx = p < KC;
+        const long long x_order = (long long)lane * Vp + 1 + x_tok;
+        bool take_e = e_avail;
+        if (e_avail && hx) take_e = e_score > x_score || (e_score == x_score && e_order < x_order);
+        double ps = take_e ? e_score : (hx ? x_score : -INFINITY);
+        long long po = take_e ? e_order : (hx ? x_order : kNoOrder);
+        double bs = ps;
+        long long bo = po;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          const double os = __shfl_xor_sync(0xffffffffu, bs, o);
+          const long long oo = __shfl_xor_sync(0xffffffffu, bo, o);
+          if (oo != kNoOrder && (bo == kNoOrder || os > bs || (os == bs && oo < bo))) {
+            bs = os;
+            bo = oo;
+          }
+        }
+        if (bo == kNoOrder) break;
+        const bool mine = po == bo;
+        bool created = false;
+        if (mine) {
+          if (take_e) {
+            n_node[r] = node;
+            n_score[r] = e_score;
+            n_last[r] = e_last;
+            e_avail = false;
+          } else {
+            int c = tr.first_child[node];
+            while (c >= 0 && tr.token[c] != x_tok) c = tr.next_sibling[c];
+            if (c < 0) {
+              c = n_nodes;
+              tr.parent[c] = node;
+              tr.token[c] = x_tok;
+              tr.depth[c] = tr.depth[node] + 1;
+              tr.first_child[c] = -1;
+              tr.next_sibling[c] = tr.first_child[node];
+              tr.first_child[node] = c;
+              tr.lex[c] = c_lex[lane][p];
+              const bool closes = x_tok == d && b_lex[lane] != 0;
+              tr.closer[c] = closes ? c : tr.closer[node];
+              tr.word[c] = closes ? word_of(lx, b_lex[lane]) : -1;
+              tr.nwords[c] = tr.nwords[node] + (closes ? 1 : 0);
+              tr.close_lm[c] = __int_as_float(0x7fffffff);
+              created = true;
+            }
+            n_node[r] = c;
+            n_score[r] = x_score;
+            n_last[r] = x_tok;
+            ++p;
+            advance();
+          }
+        }
+        n_nodes += __ballot_sync(0xffffffffu, created) != 0;
+        ++count;
+      }
+      __syncwarp();
+      nb = count;
+      if (lane < nb) {
+        node = n_node[lane];
+        score = n_score[lane];
+        last = n_last[lane];
+        b_node[lane] = node;
+        b_score[lane] = score;
+      }
+      if (lane == 0) b_nb = nb;
+    }
+    __syncthreads();
+  }
+
+  if (warp == 0) {
+    // end of utterance: close the pending run, add </s>, stable sort
+    bool keep = lane < nb;
+    double f = -INFINITY;
+    if (keep) {
+      const int ln = tr.lex[node];
+      int extra = -1;
+      f = score;
+      if (ln != 0) {
+        if (lx.constrained && (ln < 0 || lx.word[ln] < 0)) {
+          keep = false;
+        } else {
+          extra = word_of(lx, ln);
+          f = __dadd_rn(__dadd_rn(f, __dmul_rn(lmw, (double)word_lm(lm, tr, node, -1, extra))), ws);
+        }
+      }
+      if (keep) f = __dadd_rn(f, __dmul_rn(lmw, (double)word_lm(lm, tr, node, extra, lx.eos)));
+    }
+    n_score[lane] = f;
+    n_node[lane] = keep;
+    __syncwarp();
+    const unsigned keepm = __ballot_sync(0xffffffffu, keep);
+    const int cnt = __popc(keepm);
+    int rank = 0;
+    for (int j = 0; j < nb; ++j)
+      if (n_node[j] && (n_score[j] > f || (n_score[j] == f && j < lane))) ++rank;
+    if (keep) {
+      int32_t* out = out_tokens + (b * W + rank) * L;
+      const int len = tr.depth[node];
+      out_scores[b * W + rank] = f;
+      out_lens[b * W + rank] = len;
+      int nd = node;
+      for (int i = len - 1; i >= 0; --i) {
+        out[i] = tr.token[nd];
+        nd = tr.parent[nd];
+      }
+      for (int64_t i = len; i < L; ++i) out[i] = -1;
+    }
+    if (lane >= cnt && lane < W) {
+      int32_t* out = out_tokens + (b * W + lane) * L;
+      out_scores[b * W + lane] = -INFINITY;
+      out_lens[b * W + lane] = -1;
+      for (int64_t i = 0; i < L; ++i) out[i] = -1;
+    }
+  }
+}
+
 }  // namespace
 
 cudaError_t launch_beam_rows(const float* logits, float2* stats, int32_t* top_tok, int64_t M, int V, int K,
@@ -647,6 +1018,19 @@ cudaError_t launch_beam_search_lm(const float* logits, const float2* stats, cons
                                                            trie + B * trie_cap, trie + 2 * B * trie_cap,
                                                            trie + 3 * B * trie_cap, trie + 4 * B * trie_cap, trie_lm,
                                                            trie_cap, rows, out_tokens, out_lens, out_scores);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_beam_search_word_lm(const float* logits, const float2* stats, const int32_t* top_tok, int K,
+                                       const LmView& lm, const LexView& lx, double lm_weight, double word_score,
+                                       int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_f,
+                                       int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens, double* out_scores,
+                                       cudaStream_t s) {
+  if (B <= 0) return cudaSuccess;
+  const int warps = W < 16 ? W : 16;
+  beam_search_word_lm_kernel<<<(unsigned)B, 32 * warps, 0, s>>>(logits, stats, top_tok, K, lm, lx, lm_weight,
+                                                                word_score, L, V, W, blank, trie, trie_f, trie_cap,
+                                                                out_tokens, out_lens, out_scores);
   return cudaGetLastError();
 }
 

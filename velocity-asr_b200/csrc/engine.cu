@@ -1270,6 +1270,12 @@ struct vasr_lm {
   int device = 0, blank = 0;
   void* block = nullptr;   // every device table (lm.cu)
   LmView view;
+  // a word LM: view is over word ids; the search's vocabulary size, the spelling trie and the word strings
+  bool word = false;
+  int64_t vocab = 0, lexicon = 0;
+  void* lex_block = nullptr;
+  LexView lex;
+  std::unordered_map<std::string, int> word_id;
 };
 
 int vasr_lm_create_arpa(const char* path, const char* const* vocab, int64_t V, int blank, int device, vasr_lm** out) {
@@ -1298,11 +1304,61 @@ int vasr_lm_create_arpa(const char* path, const char* const* vocab, int64_t V, i
   return VASR_OK;
 }
 
+int vasr_lm_create_word_arpa(const char* path, const char* const* vocab, int64_t V, int blank, const char* delimiter,
+                             int constrained, int device, vasr_lm** out) {
+  if (!path || !vocab || !delimiter || !out) return fail(VASR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (V < 1 || V >= 0x7fffffff) return fail(VASR_ERR_INVALID, "vocabulary size must be in [1, 2^31 - 1)");
+  if (blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  LmHostTables t;
+  LexHostTables x;
+  std::string err;
+  if (!lm_parse_word_arpa(path, vocab, (int)V, blank, delimiter, constrained != 0, &t, &x, &err))
+    return fail(VASR_ERR_INVALID, err);
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(VASR_ERR_CUDA, "no CUDA device: libvasr has no CPU path");
+  if (device < 0) CK(cudaGetDevice(&device));
+  if (device >= ndev) return fail(VASR_ERR_INVALID, "bad device index");
+  DeviceGuard dev_guard(device);
+  vasr_lm* lm = new vasr_lm;
+  lm->device = device;
+  lm->blank = blank;
+  lm->word = true;
+  lm->vocab = V;
+  lm->lexicon = x.lexicon;
+  for (size_t i = 0; i < x.words.size(); ++i) lm->word_id.emplace(x.words[i], (int)i);
+  cudaError_t e = lm_upload(t, &lm->block, &lm->view);
+  if (e == cudaSuccess) e = lex_upload(x, constrained != 0, &lm->lex_block, &lm->lex);
+  if (e != cudaSuccess) {
+    vasr_lm_destroy(lm);
+    return fail(VASR_ERR_CUDA, std::string("LM upload: ") + cudaGetErrorString(e));
+  }
+  *out = lm;
+  return VASR_OK;
+}
+
 void vasr_lm_destroy(vasr_lm* lm) {
   if (!lm) return;
   DeviceGuard dev_guard(lm->device);
   cudaFree(lm->block);
+  cudaFree(lm->lex_block);
   delete lm;
+}
+
+int64_t vasr_lm_lexicon_size(const vasr_lm* lm) { return lm && lm->word ? lm->lexicon : -1; }
+
+int vasr_lm_word_ids(const vasr_lm* lm, const char* const* words, int64_t n, int32_t* ids_host) {
+  if (!lm || n < 0 || (n > 0 && (!words || !ids_host))) return fail(VASR_ERR_INVALID, "null argument");
+  if (!lm->word) return fail(VASR_ERR_INVALID, "not a word LM");
+  for (int64_t i = 0; i < n; ++i) {
+    if (!words[i]) return fail(VASR_ERR_INVALID, "null word");
+    auto it = lm->word_id.find(words[i]);
+    if (it != lm->word_id.end()) ids_host[i] = it->second;
+    else if (lm->lex.unk >= 0) ids_host[i] = lm->lex.unk;
+    else return fail(VASR_ERR_INVALID, std::string("`") + words[i] + "` is not a word of the LM, which has no <unk>");
+  }
+  return VASR_OK;
 }
 
 int vasr_lm_order(const vasr_lm* lm) { return lm ? lm->view.order : 0; }
@@ -1322,6 +1378,7 @@ int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64
                             const vasr_lm* lm, double lm_weight, int32_t* tokens_dev, int32_t* lens_dev,
                             double* scores_dev, void* stream) {
   if (!lm) return fail(VASR_ERR_INVALID, "null LM");
+  if (lm->word) return fail(VASR_ERR_INVALID, "a word LM runs in vasr_ctc_beam_search_word_lm");
   if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
   if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
   if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
@@ -1361,6 +1418,56 @@ int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64
   CK(cudaFreeAsync(trie, s));
   CK(cudaFreeAsync(trie_lm, s));
   CK(cudaFreeAsync(rows, s));
+  return VASR_OK;
+}
+
+int vasr_ctc_beam_search_word_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
+                                 const vasr_lm* lm, double lm_weight, double word_score, int32_t* tokens_dev,
+                                 int32_t* lens_dev, double* scores_dev, void* stream) {
+  if (!lm) return fail(VASR_ERR_INVALID, "null LM");
+  if (!lm->word) return fail(VASR_ERR_INVALID, "a token LM runs in vasr_ctc_beam_search_lm");
+  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
+  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
+  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  if (V != lm->vocab)
+    return fail(VASR_ERR_INVALID, "the LM is built for a vocabulary of " + std::to_string(lm->vocab) +
+                                      " tokens, the logits have " + std::to_string(V));
+  if (blank != lm->blank)
+    return fail(VASR_ERR_INVALID, "the LM is built with blank token " + std::to_string(lm->blank) +
+                                      ", the search uses " + std::to_string(blank));
+  if (!std::isfinite(lm_weight) || lm_weight < 0) return fail(VASR_ERR_INVALID, "lm_weight must be finite and >= 0");
+  if (!std::isfinite(word_score)) return fail(VASR_ERR_INVALID, "word_score must be finite");
+  if (B <= 0) return VASR_OK;
+  if (B * L > 0) {
+    cudaPointerAttributes at = {};
+    if (cudaPointerGetAttributes(&at, logits_dev) != cudaSuccess || at.type == cudaMemoryTypeUnregistered ||
+        at.type == cudaMemoryTypeHost || at.device != lm->device) {
+      cudaGetLastError();
+      return fail(VASR_ERR_INVALID, "the logits are not device memory on the LM's device (" +
+                                        std::to_string(lm->device) + ")");
+    }
+  }
+  DeviceGuard dev_guard(lm->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int W = beam_width;
+  // lexicon-free: each frame's W+2 best non-blank tokens (beam.cu: why W+2); constrained: log-softmax stats only
+  const int K = lm->lex.constrained ? 0 : (int)(V - 1 < W + 2 ? (V - 1 > 0 ? V - 1 : 1) : W + 2);
+  const int64_t M = B * L, cap = 1 + L * W;
+  float2* stats = nullptr;
+  int32_t *top = nullptr, *trie = nullptr;
+  float* trie_f = nullptr;
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&top), (size_t)(M * K > 0 ? M * K : 1) * sizeof(int32_t), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)9 * B * cap * sizeof(int32_t), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie_f), (size_t)B * cap * sizeof(float), s));
+  KL(launch_beam_rows(logits_dev, stats, top, M, (int)V, K, blank, s, nullptr));
+  KL(launch_beam_search_word_lm(logits_dev, stats, top, K, lm->view, lm->lex, lm_weight, word_score, B, L, (int)V, W,
+                                blank, trie, trie_f, cap, tokens_dev, lens_dev, scores_dev, s));
+  CK(cudaFreeAsync(stats, s));
+  CK(cudaFreeAsync(top, s));
+  CK(cudaFreeAsync(trie, s));
+  CK(cudaFreeAsync(trie_f, s));
   return VASR_OK;
 }
 

@@ -1,15 +1,18 @@
-// lm.cu — ARPA n-gram language model over token ids: the host parser (validation before any device call), the
+// lm.cu — ARPA n-gram language models over token ids or over words: the host parser (validation before any device call), the
 // upload of the device tables (layout: lm.cuh) and the scoring kernel behind vasr_lm_log_prob.
 //
 // Vocabulary mapping: an ARPA word maps to the vocabulary entry with the same string (the first one), the word
 // <space> to the entry " ".  <s> is the context symbol V and only a context: an n-gram with <s> anywhere but first,
 // or with a word outside the vocabulary (</s> included), can never be reached and is dropped.  Duplicate lines:
 // the last one wins.
+// A word LM (lm_parse_word_arpa) is the same parse over the file's own unigram words instead of a vocabulary, plus
+// the spelling trie of its lexicon over the token ids of the character vocabulary.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <string_view>
 #include <unordered_map>
 
@@ -59,6 +62,16 @@ int section_order(std::string_view f) {
   return (int)n;
 }
 
+bool read_file(const char* path, std::string* buf) {
+  FILE* fp = fopen(path, "rb");
+  if (!fp) return false;
+  char chunk[1 << 16];
+  size_t n;
+  while ((n = fread(chunk, 1, sizeof chunk, fp)) > 0) buf->append(chunk, n);
+  fclose(fp);
+  return true;
+}
+
 }  // namespace
 
 bool lm_parse_arpa(const char* path, const char* const* vocab, int V, int blank, LmHostTables* t, std::string* err) {
@@ -67,17 +80,10 @@ bool lm_parse_arpa(const char* path, const char* const* vocab, int V, int blank,
     *err = where + ", line " + std::to_string(line) + ": " + msg;
     return false;
   };
-  FILE* fp = fopen(path, "rb");
-  if (!fp) {
+  std::string buf;
+  if (!read_file(path, &buf)) {
     *err = where + ": cannot open";
     return false;
-  }
-  std::string buf;
-  {
-    char chunk[1 << 16];
-    size_t n;
-    while ((n = fread(chunk, 1, sizeof chunk, fp)) > 0) buf.append(chunk, n);
-    fclose(fp);
   }
 
   std::unordered_map<std::string_view, int> word_id;
@@ -312,6 +318,165 @@ cudaError_t lm_upload(const LmHostTables& t, void** block, LmView* view) {
   return cudaSuccess;
 }
 
+bool lm_parse_word_arpa(const char* path, const char* const* vocab, int V, int blank, const char* delimiter,
+                        bool constrained, LmHostTables* t, LexHostTables* x, std::string* err) {
+  for (int i = 0; i < V; ++i)
+    if (!vocab[i]) {
+      *err = "vocabulary entry " + std::to_string(i) + " is NULL";
+      return false;
+    }
+  x->delim = -1;
+  for (int i = 0; i < V && x->delim < 0; ++i)
+    if (strcmp(vocab[i], delimiter) == 0) x->delim = i;
+  if (x->delim < 0) {
+    *err = std::string("the word delimiter `") + delimiter + "` is not in the vocabulary";
+    return false;
+  }
+  if (x->delim == blank) {
+    *err = std::string("the word delimiter `") + delimiter + "` is the blank token (" + std::to_string(blank) + ")";
+    return false;
+  }
+
+  // the words: the unigram section's, <s> excluded, first occurrence first; lm_parse_arpa then takes them as its
+  // vocabulary, so word id = index and <s> is the context symbol as for a token LM
+  std::string buf;
+  if (!read_file(path, &buf)) {
+    *err = std::string(path) + ": cannot open";
+    return false;
+  }
+  {
+    std::unordered_map<std::string_view, int> seen;
+    bool in_uni = false;
+    int64_t line = 0, uni_line = 0;
+    const char* p = buf.data();
+    const char* const e = p + buf.size();
+    while (p < e) {
+      const char* nl = static_cast<const char*>(memchr(p, '\n', (size_t)(e - p)));
+      const char* le = nl ? nl : e;
+      ++line;
+      std::string_view f[2];
+      int nf = 0;
+      for (const char* q = p; q < le && nf < 2;) {
+        while (q < le && is_ws(*q)) ++q;
+        if (q >= le) break;
+        const char* s = q;
+        while (q < le && !is_ws(*q)) ++q;
+        f[nf++] = std::string_view(s, (size_t)(q - s));
+      }
+      p = nl ? nl + 1 : e;
+      if (nf == 0) continue;
+      if (in_uni && f[0][0] == '\\') break;
+      if (f[0] == "\\1-grams:") {
+        in_uni = true;
+        uni_line = line;
+      } else if (in_uni && nf == 2 && f[1] != "<s>" && seen.emplace(f[1], (int)x->words.size()).second) {
+        x->words.emplace_back(f[1]);
+      }
+    }
+    std::vector<const char*> names(x->words.size());
+    for (size_t i = 0; i < names.size(); ++i) names[i] = x->words[i].c_str();
+    if (!lm_parse_arpa(path, names.data(), (int)names.size(), -1, t, err)) return false;
+    auto id = [&](const char* w) {
+      auto it = seen.find(w);
+      return it == seen.end() ? -1 : it->second;
+    };
+    x->unk = id("<unk>");
+    x->eos = id("</s>") >= 0 ? id("</s>") : x->unk;
+    const std::string at = std::string(path) + ", line " + std::to_string(uni_line) + ": ";
+    if (!constrained && x->unk < 0) {
+      *err = at + "lexicon-free mode needs <unk> (a word outside the lexicon scores as <unk>); the file has none";
+      return false;
+    }
+    if (x->eos < 0) {
+      *err = at + "the file has neither </s> nor <unk> to score the end of an utterance";
+      return false;
+    }
+  }
+
+  // spelling: one token per character (UTF-8 code point), the first vocabulary entry with that string, which must
+  // be neither the blank nor the delimiter
+  std::unordered_map<std::string_view, int> char_tok;
+  for (int i = V - 1; i >= 0; --i) char_tok[std::string_view(vocab[i])] = i;   // the first entry wins
+  std::vector<std::map<int32_t, int32_t>> kids(1);
+  std::vector<int32_t> word_at(1, -1);
+  x->lexicon = 0;
+  std::vector<int32_t> spell;
+  for (size_t w = 0; w < x->words.size(); ++w) {
+    const std::string& s = x->words[w];
+    if (s == "<unk>" || s == "</s>") continue;
+    spell.clear();
+    bool ok = !s.empty();
+    for (size_t i = 0; i < s.size() && ok;) {
+      const unsigned char c = (unsigned char)s[i];
+      const size_t n = c < 0x80 ? 1 : (c & 0xe0) == 0xc0 ? 2 : (c & 0xf0) == 0xe0 ? 3 : (c & 0xf8) == 0xf0 ? 4 : 1;
+      auto it = char_tok.find(std::string_view(s).substr(i, n));
+      ok = it != char_tok.end() && it->second != blank && it->second != x->delim;
+      if (ok) spell.push_back(it->second);
+      i += n;
+    }
+    if (!ok) continue;
+    int32_t node = 0;
+    for (int32_t tk : spell) {
+      auto it = kids[node].find(tk);
+      if (it == kids[node].end()) {
+        it = kids[node].emplace(tk, (int32_t)kids.size()).first;
+        kids.emplace_back();
+        word_at.push_back(-1);
+      }
+      node = it->second;
+    }
+    word_at[node] = (int32_t)w;
+    ++x->lexicon;
+  }
+  if (constrained && x->lexicon == 0) {
+    *err = "lexicon-constrained mode needs a lexicon: none of the file's " + std::to_string(x->words.size()) +
+           " words can be spelled in the vocabulary";
+    return false;
+  }
+  x->off.assign(kids.size() + 1, 0);
+  x->tok.clear();
+  x->child.clear();
+  for (size_t n = 0; n < kids.size(); ++n) {
+    for (const auto& kv : kids[n]) {
+      x->tok.push_back(kv.first);
+      x->child.push_back(kv.second);
+    }
+    x->off[n + 1] = (int32_t)x->tok.size();
+  }
+  x->word = std::move(word_at);
+  return true;
+}
+
+cudaError_t lex_upload(const LexHostTables& x, bool constrained, void** block, LexView* view) {
+  const std::vector<int32_t>* parts[4] = {&x.off, &x.tok, &x.child, &x.word};
+  size_t at[4], total = 0;
+  for (int i = 0; i < 4; ++i) {
+    at[i] = total;
+    total += (parts[i]->size() * 4 + 255) / 256 * 256;
+  }
+  char* base = nullptr;
+  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&base), total > 0 ? total : 256);
+  if (e != cudaSuccess) return e;
+  for (int i = 0; i < 4; ++i) {
+    if (parts[i]->empty()) continue;
+    e = cudaMemcpy(base + at[i], parts[i]->data(), parts[i]->size() * 4, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+      cudaFree(base);
+      return e;
+    }
+  }
+  *block = base;
+  view->delim = x.delim;
+  view->constrained = constrained ? 1 : 0;
+  view->unk = x.unk;
+  view->eos = x.eos;
+  view->off = reinterpret_cast<const int32_t*>(base + at[0]);
+  view->tok = reinterpret_cast<const int32_t*>(base + at[1]);
+  view->child = reinterpret_cast<const int32_t*>(base + at[2]);
+  view->word = reinterpret_cast<const int32_t*>(base + at[3]);
+  return cudaSuccess;
+}
+
 namespace {
 
 // one thread per row: the longest listed context that lists the token, then the back-off weights above it
@@ -329,27 +494,7 @@ __global__ void __launch_bounds__(256) lm_log_prob_kernel(LmView lm, const int32
     return;
   }
   const int k = min(lm.order - 1, len + 1);
-  int ctx[kLmMaxOrder];
-  float bw[kLmMaxOrder];
-  const int m = lm_walk(lm, k, [&](int q) { return q <= len ? pre[H - q] : lm.V; }, ctx, bw);
-  float base = lm.uni[tok];
-  int j = 0;
-#pragma unroll
-  for (int q = kLmMaxOrder - 1; q >= 1; --q) {
-    if (j == 0 && q <= m) {
-      int64_t lo = lm.off[ctx[q]], hi = lm.off[ctx[q] + 1];
-      while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (lm.cont_tok[mid] < tok) lo = mid + 1;
-        else hi = mid;
-      }
-      if (lo < lm.off[ctx[q] + 1] && lm.cont_tok[lo] == tok) {
-        base = lm.cont_lp[lo];
-        j = q;
-      }
-    }
-  }
-  out[i] = lm_backoff(base, j, k, bw);
+  out[i] = lm_score(lm, k, [&](int q) { return q <= len ? pre[H - q] : lm.V; }, tok);
 }
 
 }  // namespace

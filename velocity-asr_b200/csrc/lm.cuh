@@ -87,6 +87,58 @@ __device__ __forceinline__ float lm_backoff(float base, int j, int k, const floa
   return __double2float_rn(s);
 }
 
+// lm(history, tok) for a history of k symbols given as lm_walk takes it: the longest listed context that lists
+// the token, then the back-off weights above it
+template <class Sym>
+__device__ __forceinline__ float lm_score(const LmView& lm, int k, Sym sym, int tok) {
+  int ctx[kLmMaxOrder];
+  float bw[kLmMaxOrder];
+  const int m = lm_walk(lm, k, sym, ctx, bw);
+  float base = lm.uni[tok];
+  int j = 0;
+#pragma unroll
+  for (int q = kLmMaxOrder - 1; q >= 1; --q) {
+    if (j == 0 && q <= m) {
+      int64_t lo = lm.off[ctx[q]], hi = lm.off[ctx[q] + 1];
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (lm.cont_tok[mid] < tok) lo = mid + 1;
+        else hi = mid;
+      }
+      if (lo < lm.off[ctx[q] + 1] && lm.cont_tok[lo] == tok) {
+        base = lm.cont_lp[lo];
+        j = q;
+      }
+    }
+  }
+  return lm_backoff(base, j, k, bw);
+}
+
+// ---- word LM over a character vocabulary ------------------------------------------------------------------
+// The LM above with word ids as its symbols (word id = index in the file's unigram list, <s> = the context symbol
+// V = word count), plus the spelling trie of its lexicon over token ids.  Node 0 is the empty spelling; a node has
+// a CSR list of (token, child) pairs, token ascending, and the word it spells (or -1).
+struct LexView {
+  int delim = -1, constrained = 0;
+  int unk = -1, eos = -1;                      // word ids of <unk> (-1: none) and of </s> (<unk>'s when unlisted)
+  const int32_t* off = nullptr;                // (nodes + 1)
+  const int32_t* tok = nullptr;                // (edges)
+  const int32_t* child = nullptr;              // (edges)
+  const int32_t* word = nullptr;               // (nodes)
+};
+
+// the child of spelling node `node` by token t, or -1 (also when node is -1: off the lexicon)
+__device__ __forceinline__ int lex_child(const LexView& lx, int node, int t) {
+  if (node < 0) return -1;
+  int lo = lx.off[node], hi = lx.off[node + 1];
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (lx.tok[mid] < t) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo < lx.off[node + 1] && lx.tok[lo] == t ? lx.child[lo] : -1;
+}
+
 // ---- host side (lm.cu) ------------------------------------------------------------------------------------
 struct LmHostTables {
   int order = 0, V = 0;
@@ -111,5 +163,25 @@ cudaError_t launch_beam_search_lm(const float* logits, const float2* stats, cons
                                   int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_lm,
                                   int64_t trie_cap, float* rows, int32_t* out_tokens, int32_t* out_lens,
                                   double* out_scores, cudaStream_t s);
+
+struct LexHostTables {
+  std::vector<std::string> words;              // word id -> string (the unigram words, <s> excluded, file order)
+  int64_t lexicon = 0;                         // spellable words other than <s>, </s>, <unk>
+  int delim = -1, unk = -1, eos = -1;
+  std::vector<int32_t> off, tok, child, word;
+};
+// Parses a word-level ARPA file (lm_parse_arpa over the file's own unigram words) and builds the spelling trie of
+// its lexicon over `vocab`; no device call.  Returns false with a message on a bad delimiter, a malformed file
+// (naming the line), a lexicon-free model without <unk> or a constrained one with an empty lexicon.
+bool lm_parse_word_arpa(const char* path, const char* const* vocab, int V, int blank, const char* delimiter,
+                        bool constrained, LmHostTables* t, LexHostTables* x, std::string* err);
+cudaError_t lex_upload(const LexHostTables& x, bool constrained, void** block, LexView* view);
+// The prefix beam search with a word LM fused (beam.cu).  top_tok (B*L, K) from launch_beam_rows (lexicon-free mode
+// only, K = min(W + 2, V - 1)); trie: 9 x (B, trie_cap) int32, trie_f (B, trie_cap) fp32.
+cudaError_t launch_beam_search_word_lm(const float* logits, const float2* stats, const int32_t* top_tok, int K,
+                                       const LmView& lm, const LexView& lx, double lm_weight, double word_score,
+                                       int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_f,
+                                       int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens, double* out_scores,
+                                       cudaStream_t s);
 
 }  // namespace vasr

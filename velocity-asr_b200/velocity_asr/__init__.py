@@ -15,7 +15,7 @@ from .audio import compute_mel_spectrogram, SAMPLE_RATE, N_FFT, HOP_LENGTH, N_ME
 from .decode import (ctc_greedy_decode, ctc_greedy_decode_with_timestamps, ctc_beam_search, DecodingResult, CTCDecoder,
                   create_default_vocabulary, frames_to_seconds, words_with_timestamps,
                   BLANK_TOKEN)
-from .lm import NGramLM
+from .lm import NGramLM, WordNGramLM
 from .ops import selective_scan, selective_scan_fn, linear, split_tf32
 from .quantize import QuantizationConfig, prepare_model_for_qat, calibrate_model
 
@@ -31,7 +31,7 @@ __all__ = [
     "__version__", "VELOCITYASR", "VelocityASRConfig", "config_from_yaml", "from_pretrained",
     "compute_mel_spectrogram", "SAMPLE_RATE", "N_FFT", "HOP_LENGTH", "N_MELS",
     "ctc_greedy_decode", "ctc_greedy_decode_with_timestamps", "ctc_beam_search", "DecodingResult", "CTCDecoder", "create_default_vocabulary", "BLANK_TOKEN",
-    "NGramLM",
+    "NGramLM", "WordNGramLM",
     "frames_to_seconds", "words_with_timestamps",
     "selective_scan", "selective_scan_fn", "linear", "split_tf32", "MAMBA_AVAILABLE", "SCAN_MODES",
     "QuantizationConfig", "prepare_model_for_qat", "calibrate_model",

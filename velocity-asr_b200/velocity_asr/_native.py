@@ -46,6 +46,11 @@ _SIGNATURES = {
     "vasr_lm_log_prob": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "vasr_ctc_beam_search_lm": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_double,
                                         c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_lm_create_word_arpa": (c_int, [c_char_p, c_void_p, c_int64, c_int, c_char_p, c_int, c_int, POINTER(c_void_p)]),
+    "vasr_lm_word_ids": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
+    "vasr_lm_lexicon_size": (c_int64, [c_void_p]),
+    "vasr_ctc_beam_search_word_lm": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_double,
+                                             c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "vasr_transcribe_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),

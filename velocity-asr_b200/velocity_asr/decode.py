@@ -1,13 +1,14 @@
 """CTC decoding: ctc_greedy_decode / CTCDecoder / create_default_vocabulary of
 velocity_asr/decode.py, with the argmax and the blank/repeat collapse done on the GPU."""
 import ctypes
+import math
 from dataclasses import dataclass
 from typing import Any, List, Optional, Tuple
 
 import torch
 
 from . import _native
-from .lm import NGramLM
+from .lm import NGramLM, WordNGramLM
 
 BLANK_TOKEN = 0  # decode.py:14
 
@@ -109,7 +110,8 @@ class DecodingResult:
 
 
 def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int = BLANK_TOKEN,
-                    lm_weight: float = 0.0, lm_scorer: Optional[Any] = None) -> List[List[DecodingResult]]:
+                    lm_weight: float = 0.0, lm_scorer: Optional[Any] = None,
+                    word_score: float = 0.0) -> List[List[DecodingResult]]:
     """decode.py:128-217 on the GPU: per utterance the `beam_width` best prefixes, best first, with the
     reference's rule (log_softmax; blank / repeated token keep the prefix, any other token extends it; equal
     prefixes keep the better score; fp64 score sums; ties in insertion order).
@@ -118,8 +120,24 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     scores (score + log_prob[tok]) + lm_weight * lm(prefix, tok); blank and repeat offers are unchanged and the
     returned scores are the fused ones.  The LM must be built for this vocabulary size and blank token and live on
     the logits' device (host logits are staged to it).  A Python `lm_scorer` callback cannot run inside the device
-    loop and is refused rather than silently ignored."""
-    use_lm = isinstance(lm_scorer, NGramLM) and lm_weight > 0
+    loop and is refused rather than silently ignored.
+
+    With a WordNGramLM, words are spelled in the vocabulary and closed by its delimiter: closing a non-empty word
+    adds lm_weight * lm(history, word) + word_score, and the end of the utterance closes the last word and adds
+    lm_weight * lm(history, </s>) (include/vasr.h states the rule).  lm_weight must be finite and >= 0 and
+    word_score finite.  A lexicon-free word LM with lm_weight == 0 and word_score == 0 takes the plain search; in
+    lexicon-constrained mode beams that cannot end on a lexicon word are dropped, so fewer may come back."""
+    word_lm = isinstance(lm_scorer, WordNGramLM)
+    if word_lm:
+        if not (math.isfinite(lm_weight) and lm_weight >= 0):
+            raise ValueError(f"lm_weight must be finite and >= 0 with a WordNGramLM, got {lm_weight}")
+        if not math.isfinite(word_score):
+            raise ValueError(f"word_score must be finite, got {word_score}")
+        use_lm = lm_weight != 0 or word_score != 0 or lm_scorer.lexicon_constrained
+    else:
+        if word_score != 0:
+            raise ValueError("word_score needs a WordNGramLM as lm_scorer")
+        use_lm = isinstance(lm_scorer, NGramLM) and lm_weight > 0
     if lm_scorer is not None and lm_weight > 0 and not use_lm:
         raise NotImplementedError("velocity_asr (B200 build): ctc_beam_search runs on the device and takes no "
                                   "Python lm_scorer (use velocity_asr.NGramLM)")
@@ -149,7 +167,11 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     lib = _native.lib()
     with torch.cuda.device(lg.device):
         stream = ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)
-        if use_lm:
+        if use_lm and word_lm:
+            _native.check(lib.vasr_ctc_beam_search_word_lm(
+                _native.ptr(lg), B, L, V, W, int(blank_token), lm_scorer._handle, float(lm_weight), float(word_score),
+                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), stream))
+        elif use_lm:
             _native.check(lib.vasr_ctc_beam_search_lm(
                 _native.ptr(lg), B, L, V, W, int(blank_token), lm_scorer._handle, float(lm_weight),
                 _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), stream))
@@ -176,11 +198,11 @@ class CTCDecoder:
         return [self._tokens_to_text(s) for s in seqs]
 
     def decode_beam_search(self, logits: torch.Tensor, beam_width: int = 10, return_all_beams: bool = False,
-                           lm_scorer: Optional[Any] = None, lm_weight: float = 0.0):
-        """decode.py:265-300: best-beam texts, or every beam with its text filled in.  `lm_scorer` / `lm_weight`
-        go to ctc_beam_search (shallow fusion with an NGramLM)."""
+                           lm_scorer: Optional[Any] = None, lm_weight: float = 0.0, word_score: float = 0.0):
+        """decode.py:265-300: best-beam texts, or every beam with its text filled in.  `lm_scorer` / `lm_weight` /
+        `word_score` go to ctc_beam_search (shallow fusion with an NGramLM or a WordNGramLM)."""
         beams = ctc_beam_search(logits, beam_width=beam_width, blank_token=self.blank_token, lm_weight=lm_weight,
-                                lm_scorer=lm_scorer)
+                                lm_scorer=lm_scorer, word_score=word_score)
         if return_all_beams:
             for utt in beams:
                 for r in utt:
