@@ -1751,6 +1751,105 @@ int vasr_debug_gemm_trace(long long* dev_buf) {
   return VASR_OK;
 }
 
+/* debug hook (not in vasr.h): one launch_gemm_tc call with every GemmArgs field exposed, for testing the
+ * tensor-core projection kernel one instantiation at a time (tests/test_projection_variants.py).  Device arrays are
+ * used as given; the module's own parameters (W as nn.Linear stores it, bias, and for the folded LayerNorm its gamma
+ * and beta) are host arrays, prepared the way the engine packs them: fold_ln when ln_gamma is set, gate_perm_row on
+ * the rows of the unpermuted [gate | local | global] weight when gate is set, then the TF32 split.  num_sms = 0 takes
+ * the device's count; 1 selects the single-CTA kernel.  On return `variant` holds the launched instantiation
+ * (TcVariant field order; family 0 = nothing launched), and the call has synchronised the stream. */
+struct vasr_debug_gemm_args {
+  const float* A; int64_t lda, rows_per_batch, batch_stride;
+  int64_t M, N, K;
+  float* C; int64_t ldc;
+  const float* resid; int64_t ldr;
+  const float* q_scale; const float* q_zp;
+  const float* pe_time; const float* pe_freq; int64_t pe_half, pe_rows;
+  float* amax_val; int32_t* amax_idx;
+  const float* W; const float* bias; const float* ln_gamma; const float* ln_beta;  // host
+  float ln_eps; int32_t act, act_from, gate, num_sms;
+  void* stream;
+  int32_t variant[8];
+};
+
+int vasr_debug_gemm(vasr_debug_gemm_args* a) {
+  if (!a || !a->A || !a->W || (!a->C && !a->amax_val) || (a->ln_gamma && !a->ln_beta))
+    return fail(VASR_ERR_INVALID, "null argument");
+  const int64_t M = a->M, N = a->N, K = a->K;
+  if (M < 0 || N <= 0 || K <= 0) return fail(VASR_ERR_INVALID, "bad shape");
+  if (a->act < 0 || a->act > 3) return fail(VASR_ERR_INVALID, "unknown activation");
+  memset(a->variant, 0, sizeof(a->variant));
+  cudaStream_t s = static_cast<cudaStream_t>(a->stream);
+  std::vector<float> W(a->W, a->W + N * K), b, cs;
+  if (a->bias) b.assign(a->bias, a->bias + N);
+  const bool lna = a->ln_gamma != nullptr;
+  if (lna) {
+    std::vector<float> Wf, bf;
+    fold_ln(W, N, K, a->bias, a->ln_gamma, a->ln_beta, &Wf, &bf, &cs);
+    W.swap(Wf);
+    b.swap(bf);
+  }
+  if (a->gate && N % 192 == 0) {    // other widths: launch_gemm_tc declines the gate epilogue
+    std::vector<float> Wp(W.size()), bp(b.size());
+    for (int64_t rp = 0; rp < N; ++rp) {
+      const int r = gate_perm_row((int)rp, (int)(N / 3));
+      memcpy(&Wp[(size_t)rp * K], &W[(size_t)r * K], (size_t)K * sizeof(float));
+      if (!b.empty()) bp[(size_t)rp] = b[(size_t)r];
+    }
+    W.swap(Wp);
+    b.swap(bp);
+  }
+  // one scratch allocation: W | W_split | bias | ln_s | ln_stats, each 16-byte aligned
+  auto al4 = [](int64_t n) { return (n + 3) & ~(int64_t)3; };
+  const int64_t o_ws = al4(N * K), o_b = o_ws + al4(2 * N * K), o_s = o_b + al4(N), o_st = o_s + al4(N);
+  const int64_t total = o_st + al4(2 * (M > 0 ? M : 1));
+  float* buf = nullptr;
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&buf), (size_t)total * sizeof(float), s));
+  auto put = [&](const std::vector<float>& v, int64_t off) {
+    return v.empty() ? cudaSuccess : cudaMemcpyAsync(buf + off, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice, s);
+  };
+  cudaError_t e = put(W, 0);
+  if (e == cudaSuccess) e = put(b, o_b);
+  if (e == cudaSuccess) e = put(cs, o_s);
+  if (e == cudaSuccess) e = launch_split_tf32(buf, buf + o_ws, N * K, s);
+  if (e != cudaSuccess) {
+    cudaFreeAsync(buf, s);
+    return fail(VASR_ERR_CUDA, std::string("vasr_debug_gemm staging: ") + cudaGetErrorString(e));
+  }
+  GemmArgs g;
+  g.A = a->A; g.lda = a->lda; g.rows_per_batch = a->rows_per_batch; g.batch_stride = a->batch_stride;
+  g.W = buf; g.W_split = buf + o_ws; g.bias = b.empty() ? nullptr : buf + o_b;
+  g.q_scale = a->q_scale; g.q_zp = a->q_zp;
+  g.C = a->C; g.ldc = a->ldc;
+  g.M = M; g.N = N; g.K = K;
+  g.act = a->act; g.act_from = a->act_from;
+  g.resid = a->resid; g.ldr = a->ldr;
+  if (lna) { g.ln_s = buf + o_s; g.ln_stats = buf + o_st; g.ln_eps = a->ln_eps; }
+  g.amax_val = a->amax_val; g.amax_idx = a->amax_idx;
+  g.gate = a->gate;
+  g.pe_time = a->pe_time; g.pe_freq = a->pe_freq; g.pe_half = (int)a->pe_half; g.pe_rows = a->pe_rows;
+  int sms = a->num_sms;
+  if (sms <= 0) {
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  }
+  tc_last_variant = nullptr;
+  e = launch_gemm_tc(g, sms, s, nullptr);
+  const TcVariant* v = tc_last_variant;
+  if (e == cudaErrorNotSupported) (void)cudaGetLastError();
+  cudaFreeAsync(buf, s);
+  const cudaError_t se = cudaStreamSynchronize(s);     // a fault of the kernel surfaces here
+  if (e == cudaErrorNotSupported) return fail(VASR_ERR_UNSUPPORTED, "launch_gemm_tc declines this projection");
+  if (e != cudaSuccess) return fail(VASR_ERR_CUDA, std::string("launch_gemm_tc: ") + cudaGetErrorString(e));
+  if (se != cudaSuccess) return fail(VASR_ERR_CUDA, std::string("vasr_debug_gemm: ") + cudaGetErrorString(se));
+  if (v) {
+    const int f[8] = {v->family, v->tn, v->act, v->pe, v->resid, v->quant, v->wres, v->epi};
+    memcpy(a->variant, f, sizeof(f));
+  }
+  return VASR_OK;
+}
+
 /* debug hook (not in vasr.h): prints and clears the per-shape projection timings gathered under VASR_PROF=1 */
 int vasr_debug_dump_profile(vasr_handle* h) {
   if (!h) return fail(VASR_ERR_INVALID, "null handle");

@@ -1359,6 +1359,12 @@ bool make_map(CUtensorMap* map, const float* base, int rank, const uint64_t* dim
 }  // namespace
 
 long long* g_trace = nullptr;   // set by vasr_debug_gemm_trace (tools/gemm_trace.py)
+thread_local const TcVariant* tc_last_variant = nullptr;
+
+namespace {
+template <int FAMILY, int ACT, bool PE, bool RESID, bool QUANT, bool WRES = false, int TN = 128, int EPI = 0>
+constexpr TcVariant kTcVariant = {FAMILY, TN, ACT, PE, RESID, QUANT, WRES, EPI};
+}  // namespace
 
 bool gemm_tc_supported(const GemmArgs& g) {
   if (!encode_fn()) return false;
@@ -1472,40 +1478,48 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   if (pe || rs || g.q_scale || !(g.act == ACT_NONE || g.act == ACT_GELU) || t192) a.wres = 0;
   if (a.wres) a.rotate_n = 0;
   cudaError_t err = cudaSuccess;
-  auto go1 = [&](auto kernel) {
+  // each launch site names its instantiation once: VASR_GO1 / VASR_GO2 / VASR_GO192 (template arguments) launch it
+  // and record it in tc_last_variant
+  auto go1 = [&](auto kernel, const TcVariant* v) {
+    tc_last_variant = v;
     err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (err == cudaSuccess) err = launch_k(kernel, dim3(grid), dim3(TC_THREADS), SMEM_BYTES, s, tmA, tmWh, tmWl, a);
   };
-  auto go2 = [&](auto kernel) {
+  auto go2 = [&](auto kernel, const TcVariant* v) {
+    tc_last_variant = v;
     err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, P_SMEM_BYTES);
     if (err == cudaSuccess) err = launch_k(kernel, dim3(grid), dim3(TC_THREADS), P_SMEM_BYTES, s, tmA, tmWh, tmWl, a);
   };
-  auto go192 = [&](auto kernel) {
+  auto go192 = [&](auto kernel, const TcVariant* v) {
+    tc_last_variant = v;
     err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PairCfg<192>::SMEM_BYTES);
     if (err == cudaSuccess)
       err = launch_k(kernel, dim3(grid), dim3(TC_THREADS), PairCfg<192>::SMEM_BYTES, s, tmA, tmWh, tmWl, a);
   };
+#define VASR_GO1(...) go1(gemm_tc_kernel<__VA_ARGS__>, &kTcVariant<1, __VA_ARGS__>)
+#define VASR_GO2(...) go2(gemm_tc2_kernel<__VA_ARGS__>, &kTcVariant<2, __VA_ARGS__>)
+#define VASR_GO192(...) go192(gemm_tc2_kernel<__VA_ARGS__>, &kTcVariant<2, __VA_ARGS__>)
   if (t192) {
     a.rotate_n = 0;
-    if (gate) go192(gemm_tc2_kernel<ACT_NONE, false, false, false, false, 192, EPI_GATE>);
-    else if (lna) go192(gemm_tc2_kernel<ACT_GELU, false, false, false, false, 192, EPI_LNA>);
-    else if (g.act == ACT_SOFTPLUS) go192(gemm_tc2_kernel<ACT_SOFTPLUS, false, false, false, false, 192>);
-    else if (g.act == ACT_GELU) go192(gemm_tc2_kernel<ACT_GELU, false, false, false, false, 192>);
-    else if (rs) go192(gemm_tc2_kernel<ACT_NONE, false, true, false, false, 192>);
-    else go192(gemm_tc2_kernel<ACT_NONE, false, false, false, false, 192>);
+    if (gate) VASR_GO192(ACT_NONE, false, false, false, false, 192, EPI_GATE);
+    else if (lna) VASR_GO192(ACT_GELU, false, false, false, false, 192, EPI_LNA);
+    else if (g.act == ACT_SOFTPLUS) VASR_GO192(ACT_SOFTPLUS, false, false, false, false, 192);
+    else if (g.act == ACT_GELU) VASR_GO192(ACT_GELU, false, false, false, false, 192);
+    else if (rs) VASR_GO192(ACT_NONE, false, true, false, false, 192);
+    else VASR_GO192(ACT_NONE, false, false, false, false, 192);
     if (err != cudaSuccess) return err;
     if (launches) ++*launches;
     return cudaSuccess;
   }
   if (lna || amax) {      // plain projection with a folded LayerNorm and / or the argmax epilogue (CTC head, q, k | v)
     if (a.wres) {
-      if (lna && amax) go2(gemm_tc2_kernel<ACT_NONE, false, false, false, true, 128, EPI_LNA | EPI_AMAX>);
-      else if (lna) go2(gemm_tc2_kernel<ACT_NONE, false, false, false, true, 128, EPI_LNA>);
-      else go2(gemm_tc2_kernel<ACT_NONE, false, false, false, true, 128, EPI_AMAX>);
+      if (lna && amax) VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_LNA | EPI_AMAX);
+      else if (lna) VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_LNA);
+      else VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_AMAX);
     } else {
-      if (lna && amax) go2(gemm_tc2_kernel<ACT_NONE, false, false, false, false, 128, EPI_LNA | EPI_AMAX>);
-      else if (lna) go2(gemm_tc2_kernel<ACT_NONE, false, false, false, false, 128, EPI_LNA>);
-      else go2(gemm_tc2_kernel<ACT_NONE, false, false, false, false, 128, EPI_AMAX>);
+      if (lna && amax) VASR_GO2(ACT_NONE, false, false, false, false, 128, EPI_LNA | EPI_AMAX);
+      else if (lna) VASR_GO2(ACT_NONE, false, false, false, false, 128, EPI_LNA);
+      else VASR_GO2(ACT_NONE, false, false, false, false, 128, EPI_AMAX);
     }
     if (err != cudaSuccess) return err;
     if (launches) ++*launches;
@@ -1515,27 +1529,27 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   if (quant) {   // config 5: the quantised modules are plain projections, or the temporal-binding conv (GELU + pos-enc)
     if (rs || !((g.act == ACT_NONE && !pe) || (g.act == ACT_GELU && pe))) return cudaErrorNotSupported;
     if (pair) {
-      if (pe) go2(gemm_tc2_kernel<ACT_GELU, true, false, true>);
-      else go2(gemm_tc2_kernel<ACT_NONE, false, false, true>);
+      if (pe) VASR_GO2(ACT_GELU, true, false, true);
+      else VASR_GO2(ACT_NONE, false, false, true);
     } else {
-      if (pe) go1(gemm_tc_kernel<ACT_GELU, true, false, true>);
-      else go1(gemm_tc_kernel<ACT_NONE, false, false, true>);
+      if (pe) VASR_GO1(ACT_GELU, true, false, true);
+      else VASR_GO1(ACT_NONE, false, false, true);
     }
   }
 #define VASR_TC_CASE(ACTV)                                                                   \
   if (!quant && g.act == ACTV) {                                                             \
     if (pair) {                                                                              \
-      if (pe && rs) go2(gemm_tc2_kernel<ACTV, true, true, false>);                           \
-      else if (pe) go2(gemm_tc2_kernel<ACTV, true, false, false>);                           \
-      else if (rs) go2(gemm_tc2_kernel<ACTV, false, true, false>);                           \
-      else if (a.wres && ACTV == ACT_NONE) go2(gemm_tc2_kernel<ACT_NONE, false, false, false, true>);   \
-      else if (a.wres && ACTV == ACT_GELU) go2(gemm_tc2_kernel<ACT_GELU, false, false, false, true>);   \
-      else go2(gemm_tc2_kernel<ACTV, false, false, false>);                                  \
+      if (pe && rs) VASR_GO2(ACTV, true, true, false);                                       \
+      else if (pe) VASR_GO2(ACTV, true, false, false);                                       \
+      else if (rs) VASR_GO2(ACTV, false, true, false);                                       \
+      else if (a.wres && ACTV == ACT_NONE) VASR_GO2(ACT_NONE, false, false, false, true);    \
+      else if (a.wres && ACTV == ACT_GELU) VASR_GO2(ACT_GELU, false, false, false, true);    \
+      else VASR_GO2(ACTV, false, false, false);                                              \
     } else {                                                                                 \
-      if (pe && rs) go1(gemm_tc_kernel<ACTV, true, true, false>);                            \
-      else if (pe) go1(gemm_tc_kernel<ACTV, true, false, false>);                            \
-      else if (rs) go1(gemm_tc_kernel<ACTV, false, true, false>);                            \
-      else go1(gemm_tc_kernel<ACTV, false, false, false>);                                   \
+      if (pe && rs) VASR_GO1(ACTV, true, true, false);                                       \
+      else if (pe) VASR_GO1(ACTV, true, false, false);                                       \
+      else if (rs) VASR_GO1(ACTV, false, true, false);                                       \
+      else VASR_GO1(ACTV, false, false, false);                                              \
     }                                                                                        \
   }
   VASR_TC_CASE(ACT_NONE)
@@ -1543,6 +1557,9 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   VASR_TC_CASE(ACT_SOFTPLUS)
   VASR_TC_CASE(ACT_SIGMOID)
 #undef VASR_TC_CASE
+#undef VASR_GO1
+#undef VASR_GO2
+#undef VASR_GO192
   if (err != cudaSuccess) return err;
   if (launches) ++*launches;
   return cudaSuccess;

@@ -52,6 +52,12 @@ cudaError_t launch_gemm(const GemmArgs& g, cudaStream_t s, int64_t* launches);
 // tcgen05 / TMEM / TMA path with 3xTF32 split accumulation (gemm_tc.cu); needs g.W_split.  Returns
 // cudaErrorNotSupported when a tensor map cannot be encoded for this view.
 cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64_t* launches);
+// The template instantiation a launch_gemm_tc call launched (family 1 = gemm_tc_kernel, 2 = gemm_tc2_kernel; tn, act,
+// pe, resid, quant, wres, epi = its template arguments).  Each launch site sets it; the projection tests read it.
+struct TcVariant {
+  int family, tn, act, pe, resid, quant, wres, epi;
+};
+extern thread_local const TcVariant* tc_last_variant;
 // hl[0..n) = rna_tf32(w), hl[n..2n) = rna_tf32(w - hl[0..n)): the weight operand of launch_gemm_tc.
 cudaError_t launch_split_tf32(const float* w, float* hl, int64_t n, cudaStream_t s);
 extern long long* g_trace;   // debug: device buffer (5 x 128 clock64 slots) CTA 0 of the projection kernel writes
