@@ -214,6 +214,40 @@ int vasr_ctc_beam_search_word_lm(const float* logits_dev, int64_t B, int64_t L, 
                                  const vasr_lm* lm, double lm_weight, double word_score, int32_t* tokens_dev,
                                  int32_t* lens_dev, double* scores_dev, void* stream);
 
+/* ---- the prefix beam search over a ragged batch, with or without an LM
+ * lm == NULL runs the rule of vasr_ctc_beam_search (lm_weight and word_score are not used); a token LM the rule of
+ * vasr_ctc_beam_search_lm (word_score must be 0); a word LM the rule of vasr_ctc_beam_search_word_lm.  Argument
+ * checks, messages and the LM's device and vocabulary requirements are those of the matching entry point.
+ * row_lens_host: B frame counts, a HOST array that may be reused as soon as the call returns, or NULL (every
+ * utterance has L frames).  Each 0 <= row_lens[b] <= L, else VASR_ERR_SHAPE before any device work.  Utterance b is
+ * searched over rows b*L + [0, row_lens[b]) of logits (B, L, V); the rows after them are never read, so whatever
+ * they hold (NaN included) does not matter.  A word LM's end-of-utterance step follows the utterance's last frame.
+ * Outputs keep the shapes of vasr_ctc_beam_search: tokens (B, beam_width, L), -1 past each beam's length.
+ * Contract: utterance b gets bit for bit the tokens, lens and fp64 scores that the matching unragged entry point
+ * gives for logits[b : b+1, : row_lens[b]] alone.  row_lens[b] = 0 gives the L = 0 result: the single empty beam
+ * with score 0, or lm_weight * lm((<s>), </s>) under a word LM. */
+int vasr_ctc_beam_search_ragged(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L,
+                                int64_t V, int beam_width, int blank, const vasr_lm* lm, double lm_weight,
+                                double word_score, int32_t* tokens_dev, int32_t* lens_dev, double* scores_dev,
+                                void* stream);
+
+/* ---- transcribe with the beam search: PCM -> log-mel -> model -> logits -> prefix beam search, one call.
+ * pcm (B, S); sample_lens_host (optional, HOST): a ragged batch as vasr_transcribe_ragged (200 < len <= S, else
+ * VASR_ERR_SHAPE).  L = vasr_num_tokens(vasr_num_frames(S)), blank = 0.  Outputs as vasr_ctc_beam_search_ragged:
+ * tokens (B, beam_width, L), lens (B, beam_width), scores (B, beam_width) fp64.  lm: NULL, a token LM or a word LM,
+ * rules and checks as vasr_ctc_beam_search_ragged; it must live on the handle's device and be built for vocab_size
+ * and blank 0, else VASR_ERR_INVALID before any device work.  The CTC head writes the logits (as vasr_forward) into
+ * the handle's workspace, which grows by B * L * vocab_size floats for these calls only.
+ * Contract: utterance b gets bit for bit what vasr_ctc_beam_search_ragged gives on the logits vasr_forward produces
+ * for that utterance alone (its first sample_lens[b] samples, or all S).  The _host variant takes host PCM, returns
+ * host results and synchronises once at the end. */
+int vasr_transcribe_beam(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B, int64_t S,
+                         int beam_width, const vasr_lm* lm, double lm_weight, double word_score, int32_t* tokens_dev,
+                         int32_t* lens_dev, double* scores_dev, void* stream);
+int vasr_transcribe_beam_host(vasr_handle* h, const float* pcm_host, const int32_t* sample_lens_host, int64_t B,
+                              int64_t S, int beam_width, const vasr_lm* lm, double lm_weight, double word_score,
+                              int32_t* tokens_host, int32_t* lens_host, double* scores_host);
+
 /* ---- transcribe: load -> mel -> model -> greedy (scripts/transcribe.py:69-82), batched.
  * tokens (B, L) int32, lens (B); L = vasr_num_tokens(vasr_num_frames(S)). */
 int vasr_transcribe(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S,

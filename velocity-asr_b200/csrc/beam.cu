@@ -42,14 +42,24 @@ namespace vasr {
 
 namespace {
 
+// Ragged batches: every kernel below takes an optional per-utterance frame count, read as (pointer, stride) so
+// the ragged dims of a fused call (kernels.cuh, RAG_L) serve without a copy.  Utterance b is then searched over
+// its rows b * L + [0, len_b) only; the row stride stays L.  A null pointer means len_b = L for every utterance.
+__device__ __forceinline__ int64_t utt_frames(const int32_t* lens, int stride, int64_t b, int64_t L) {
+  return lens ? (int64_t)lens[b * stride] : L;
+}
+
 // One warp per (utterance, frame) row: max, log-sum-exp, and the K best non-blank tokens by
 // log-prob (ties -> lower token id).  log-prob = (x - max) - log(sum exp(x - max)), torch's order.
+// Rows at or past their utterance's length are neither read nor written.
 __global__ void __launch_bounds__(256) beam_rows_kernel(const float* __restrict__ logits, float2* __restrict__ stats,
                                                         int32_t* __restrict__ top_tok, int64_t M, int V, int K,
-                                                        int blank) {
+                                                        int blank, int64_t L, const int32_t* __restrict__ lens,
+                                                        int lens_stride) {
   const int lane = threadIdx.x & 31;
   const int64_t m = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (m >= M) return;
+  if (lens && m % L >= utt_frames(lens, lens_stride, m / L, L)) return;
   const float* x = logits + m * V;
   float mx = -INFINITY;
   for (int n = lane; n < V; n += 32) mx = fmaxf(mx, x[n]);
@@ -99,11 +109,12 @@ constexpr long long kNoOrder = 0x7fffffffffffffffLL;
 
 __global__ void __launch_bounds__(32) beam_search_kernel(
     const float* __restrict__ logits, const float2* __restrict__ stats, const int32_t* __restrict__ top_tok, int K,
-    int64_t L, int V, int W, int blank, int32_t* trie_parent, int32_t* trie_token, int32_t* trie_depth,
-    int64_t trie_cap, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
-    double* __restrict__ out_scores) {
+    int64_t L, const int32_t* __restrict__ lens, int lens_stride, int V, int W, int blank, int32_t* trie_parent,
+    int32_t* trie_token, int32_t* trie_depth, int64_t trie_cap, int32_t* __restrict__ out_tokens,
+    int32_t* __restrict__ out_lens, double* __restrict__ out_scores) {
   const int64_t b = blockIdx.x;
   const int lane = threadIdx.x;
+  const int64_t Lb = utt_frames(lens, lens_stride, b, L);
   int32_t* parent = trie_parent + b * trie_cap;
   int32_t* token = trie_token + b * trie_cap;
   int32_t* depth = trie_depth + b * trie_cap;
@@ -122,7 +133,7 @@ __global__ void __launch_bounds__(32) beam_search_kernel(
   const long long Vp = (long long)V + 1;
   __syncwarp();
 
-  for (int64_t t = 0; t < L; ++t) {
+  for (int64_t t = 0; t < Lb; ++t) {
     const int64_t row = b * L + t;
     const float* x = logits + row * V;
     const float2 st = stats[row];
@@ -385,11 +396,13 @@ __device__ __forceinline__ void lm_candidates(const float* x, float2 st, const f
 
 __global__ void __launch_bounds__(512) beam_search_lm_kernel(
     const float* __restrict__ logits, const float2* __restrict__ stats, const LmView lm, double lmw, int K,
-    int64_t L, int V, int W, int blank, int32_t* trie_parent, int32_t* trie_token, int32_t* trie_depth,
-    int32_t* trie_child, int32_t* trie_sibling, float* trie_lm, int64_t trie_cap, float* rows, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
+    int64_t L, const int32_t* __restrict__ lens, int lens_stride, int V, int W, int blank, int32_t* trie_parent,
+    int32_t* trie_token, int32_t* trie_depth, int32_t* trie_child, int32_t* trie_sibling, float* trie_lm,
+    int64_t trie_cap, float* rows, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
     double* __restrict__ out_scores) {
   const int64_t b = blockIdx.x;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  const int64_t Lb = utt_frames(lens, lens_stride, b, L);
   int32_t* parent = trie_parent + b * trie_cap;
   int32_t* token = trie_token + b * trie_cap;
   int32_t* depth = trie_depth + b * trie_cap;
@@ -427,7 +440,7 @@ __global__ void __launch_bounds__(512) beam_search_lm_kernel(
   const long long Vp = (long long)V + 1;
   __syncthreads();
 
-  for (int64_t t = 0; t < L; ++t) {
+  for (int64_t t = 0; t < Lb; ++t) {
     const int64_t rw = b * L + t;
     const float* x = logits + rw * V;
     const float2 st = stats[rw];
@@ -669,11 +682,12 @@ __device__ __forceinline__ double word_offer(double score, double lp, bool close
 
 __global__ void __launch_bounds__(512, 1) beam_search_word_lm_kernel(
     const float* __restrict__ logits, const float2* __restrict__ stats, const int32_t* __restrict__ top_tok, int K,
-    const LmView lm, const LexView lx, double lmw, double ws, int64_t L, int V, int W, int blank, int32_t* trie,
-    float* trie_f, int64_t trie_cap, int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens,
-    double* __restrict__ out_scores) {
+    const LmView lm, const LexView lx, double lmw, double ws, int64_t L, const int32_t* __restrict__ lens,
+    int lens_stride, int V, int W, int blank, int32_t* trie, float* trie_f, int64_t trie_cap,
+    int32_t* __restrict__ out_tokens, int32_t* __restrict__ out_lens, double* __restrict__ out_scores) {
   const int64_t b = blockIdx.x;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  const int64_t Lb = utt_frames(lens, lens_stride, b, L);   // the end-of-utterance step follows frame Lb - 1
   const int64_t pb = (int64_t)gridDim.x * trie_cap;   // one plane of the trie
   int32_t* base = trie + b * trie_cap;
   const WordTrie tr{base,          base + pb,     base + 2 * pb, base + 3 * pb, base + 4 * pb,
@@ -708,7 +722,7 @@ __global__ void __launch_bounds__(512, 1) beam_search_word_lm_kernel(
   const long long Vp = (long long)V + 1;
   __syncthreads();
 
-  for (int64_t t = 0; t < L; ++t) {
+  for (int64_t t = 0; t < Lb; ++t) {
     const int64_t rw = b * L + t;
     const float* x = logits + rw * V;
     const float2 st = stats[rw];
@@ -988,19 +1002,21 @@ __global__ void __launch_bounds__(512, 1) beam_search_word_lm_kernel(
 }  // namespace
 
 cudaError_t launch_beam_rows(const float* logits, float2* stats, int32_t* top_tok, int64_t M, int V, int K,
-                             int blank, cudaStream_t s, int64_t* launches) {
+                             int blank, int64_t L, const int32_t* lens, int lens_stride, cudaStream_t s,
+                             int64_t* launches) {
   if (M <= 0) return cudaSuccess;
-  beam_rows_kernel<<<(unsigned)((M + 7) / 8), 256, 0, s>>>(logits, stats, top_tok, M, V, K, blank);
+  beam_rows_kernel<<<(unsigned)((M + 7) / 8), 256, 0, s>>>(logits, stats, top_tok, M, V, K, blank, L, lens,
+                                                           lens_stride);
   if (launches) ++*launches;
   return cudaGetLastError();
 }
 
 cudaError_t launch_beam_search(const float* logits, const float2* stats, const int32_t* top_tok, int K, int64_t B,
-                               int64_t L, int V, int W, int blank, int32_t* trie, int64_t trie_cap,
-                               int32_t* out_tokens, int32_t* out_lens, double* out_scores, cudaStream_t s,
-                               int64_t* launches) {
+                               int64_t L, const int32_t* lens, int lens_stride, int V, int W, int blank,
+                               int32_t* trie, int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens,
+                               double* out_scores, cudaStream_t s, int64_t* launches) {
   if (B <= 0) return cudaSuccess;
-  beam_search_kernel<<<(unsigned)B, 32, 0, s>>>(logits, stats, top_tok, K, L, V, W, blank, trie,
+  beam_search_kernel<<<(unsigned)B, 32, 0, s>>>(logits, stats, top_tok, K, L, lens, lens_stride, V, W, blank, trie,
                                                 trie + B * trie_cap, trie + 2 * B * trie_cap, trie_cap, out_tokens,
                                                 out_lens, out_scores);
   if (launches) ++*launches;
@@ -1008,29 +1024,30 @@ cudaError_t launch_beam_search(const float* logits, const float2* stats, const i
 }
 
 cudaError_t launch_beam_search_lm(const float* logits, const float2* stats, const LmView& lm, double lm_weight,
-                                  int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_lm,
-                                  int64_t trie_cap, float* rows, int32_t* out_tokens, int32_t* out_lens,
-                                  double* out_scores, cudaStream_t s) {
+                                  int64_t B, int64_t L, const int32_t* lens, int lens_stride, int V, int W, int blank,
+                                  int32_t* trie, float* trie_lm, int64_t trie_cap, float* rows, int32_t* out_tokens,
+                                  int32_t* out_lens, double* out_scores, cudaStream_t s) {
   if (B <= 0) return cudaSuccess;
   const int K = V - 1 < W + 1 ? (V - 1 > 0 ? V - 1 : 1) : W + 1;
   const int warps = W < 16 ? W : 16;
-  beam_search_lm_kernel<<<(unsigned)B, 32 * warps, 0, s>>>(logits, stats, lm, lm_weight, K, L, V, W, blank, trie,
-                                                           trie + B * trie_cap, trie + 2 * B * trie_cap,
-                                                           trie + 3 * B * trie_cap, trie + 4 * B * trie_cap, trie_lm,
-                                                           trie_cap, rows, out_tokens, out_lens, out_scores);
+  beam_search_lm_kernel<<<(unsigned)B, 32 * warps, 0, s>>>(logits, stats, lm, lm_weight, K, L, lens, lens_stride, V,
+                                                           W, blank, trie, trie + B * trie_cap,
+                                                           trie + 2 * B * trie_cap, trie + 3 * B * trie_cap,
+                                                           trie + 4 * B * trie_cap, trie_lm, trie_cap, rows,
+                                                           out_tokens, out_lens, out_scores);
   return cudaGetLastError();
 }
 
 cudaError_t launch_beam_search_word_lm(const float* logits, const float2* stats, const int32_t* top_tok, int K,
                                        const LmView& lm, const LexView& lx, double lm_weight, double word_score,
-                                       int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_f,
-                                       int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens, double* out_scores,
-                                       cudaStream_t s) {
+                                       int64_t B, int64_t L, const int32_t* lens, int lens_stride, int V, int W,
+                                       int blank, int32_t* trie, float* trie_f, int64_t trie_cap, int32_t* out_tokens,
+                                       int32_t* out_lens, double* out_scores, cudaStream_t s) {
   if (B <= 0) return cudaSuccess;
   const int warps = W < 16 ? W : 16;
   beam_search_word_lm_kernel<<<(unsigned)B, 32 * warps, 0, s>>>(logits, stats, top_tok, K, lm, lx, lm_weight,
-                                                                word_score, L, V, W, blank, trie, trie_f, trie_cap,
-                                                                out_tokens, out_lens, out_scores);
+                                                                word_score, L, lens, lens_stride, V, W, blank, trie,
+                                                                trie_f, trie_cap, out_tokens, out_lens, out_scores);
   return cudaGetLastError();
 }
 

@@ -1241,31 +1241,6 @@ int vasr_ctc_greedy_timestamps(const float* logits_dev, int64_t B, int64_t L, in
   return VASR_OK;
 }
 
-int vasr_ctc_beam_search(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
-                         int32_t* tokens_dev, int32_t* lens_dev, double* scores_dev, void* stream) {
-  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
-  if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
-  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
-  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
-  if (B <= 0) return VASR_OK;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int W = beam_width;
-  const int K = (int)(V - 1 < W + 1 ? V - 1 : W + 1) > 0 ? (int)(V - 1 < W + 1 ? V - 1 : W + 1) : 1;
-  const int64_t M = B * L, cap = 1 + L * W;
-  float2* stats = nullptr;
-  int32_t *top = nullptr, *trie = nullptr;
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&top), (size_t)(M > 0 ? M : 1) * K * sizeof(int32_t), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)3 * B * cap * sizeof(int32_t), s));
-  KL(launch_beam_rows(logits_dev, stats, top, M, (int)V, K, blank, s, nullptr));
-  KL(launch_beam_search(logits_dev, stats, top, K, B, L, (int)V, W, blank, trie, cap, tokens_dev, lens_dev,
-                        scores_dev, s, nullptr));
-  CK(cudaFreeAsync(stats, s));
-  CK(cudaFreeAsync(top, s));
-  CK(cudaFreeAsync(trie, s));
-  return VASR_OK;
-}
-
 struct vasr_lm {
   int device = 0, blank = 0;
   void* block = nullptr;   // every device table (lm.cu)
@@ -1374,51 +1349,131 @@ int vasr_lm_log_prob(const vasr_lm* lm, const int32_t* prefixes_dev, const int32
   return VASR_OK;
 }
 
+namespace {
+
+// Argument checks shared by every search entry point (no device call): lm NULL runs the LM-free rule (lm_weight and
+// word_score unused), a token LM the rule of beam_search_lm_kernel (word_score must be 0), a word LM that of
+// beam_search_word_lm_kernel.  row_lens_host (optional): B frame counts, each in [0, L].
+int beam_check(const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int beam_width,
+               int blank, const vasr_lm* lm, double lm_weight, double word_score, const int32_t* tokens_dev,
+               const int32_t* lens_dev, const double* scores_dev) {
+  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  if (!lens_dev || !scores_dev) return fail(VASR_ERR_INVALID, "null argument");
+  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
+  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  if (lm) {
+    const int64_t lv = lm->word ? lm->vocab : lm->view.V;
+    if (V != lv)
+      return fail(VASR_ERR_INVALID, "the LM is built for a vocabulary of " + std::to_string(lv) +
+                                        " tokens, the logits have " + std::to_string(V));
+    if (blank != lm->blank)
+      return fail(VASR_ERR_INVALID, "the LM is built with blank token " + std::to_string(lm->blank) +
+                                        ", the search uses " + std::to_string(blank));
+    if (lm->word) {
+      if (!std::isfinite(lm_weight) || lm_weight < 0)
+        return fail(VASR_ERR_INVALID, "lm_weight must be finite and >= 0");
+      if (!std::isfinite(word_score)) return fail(VASR_ERR_INVALID, "word_score must be finite");
+    } else {
+      if (!std::isfinite(lm_weight)) return fail(VASR_ERR_INVALID, "lm_weight must be finite");
+      if (word_score != 0) return fail(VASR_ERR_INVALID, "word_score needs a word LM");
+    }
+  }
+  if (row_lens_host)
+    for (int64_t b = 0; b < B; ++b)
+      if (row_lens_host[b] < 0 || row_lens_host[b] > L)
+        return fail(VASR_ERR_SHAPE, "ragged search: every utterance needs between 0 and L frames (utterance " +
+                                        std::to_string(b) + " has " + std::to_string(row_lens_host[b]) + ")");
+  return VASR_OK;
+}
+
+// The body of every search entry point: checks, the device check, scratch sizing and the launches.  Frame counts
+// come from the host (row_lens_host, uploaded here) or are already on the device (lens_dev at stride lens_stride:
+// the RAG_L column of a fused call's ragged dims); neither: every utterance has L frames.
+int beam_search(const float* logits_dev, const int32_t* row_lens_host, const int32_t* lens_dev, int lens_stride,
+                int64_t B, int64_t L, int64_t V, int beam_width, int blank, const vasr_lm* lm, double lm_weight,
+                double word_score, int32_t* tokens_dev, int32_t* out_lens_dev, double* scores_dev, cudaStream_t s) {
+  if (!logits_dev && B * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  RET(beam_check(row_lens_host, B, L, V, beam_width, blank, lm, lm_weight, word_score, tokens_dev, out_lens_dev,
+                 scores_dev));
+  if (B <= 0) return VASR_OK;
+  int dev = 0;
+  if (lm) {
+    dev = lm->device;
+    if (B * L > 0) {
+      cudaPointerAttributes at = {};
+      if (cudaPointerGetAttributes(&at, logits_dev) != cudaSuccess || at.type == cudaMemoryTypeUnregistered ||
+          at.type == cudaMemoryTypeHost || at.device != lm->device) {
+        cudaGetLastError();
+        return fail(VASR_ERR_INVALID, "the logits are not device memory on the LM's device (" +
+                                          std::to_string(lm->device) + ")");
+      }
+    }
+  } else {
+    CK(cudaGetDevice(&dev));
+  }
+  DeviceGuard dev_guard(dev);
+  const int W = beam_width;
+  // candidate tokens per frame (beam.cu says why these counts): LM-free W+1; word LM lexicon-free W+2; a token LM
+  // and a constrained word LM list their own, so beam_rows gives them the log-softmax stats only
+  int K = 0;
+  if (!lm) K = (int)(V - 1 < W + 1 ? V - 1 : W + 1) > 0 ? (int)(V - 1 < W + 1 ? V - 1 : W + 1) : 1;
+  else if (lm->word && !lm->lex.constrained) K = (int)(V - 1 < W + 2 ? (V - 1 > 0 ? V - 1 : 1) : W + 2);
+  const int planes = !lm ? 3 : lm->word ? 9 : 5;
+  const int64_t M = B * L, cap = 1 + L * W;
+  float2* stats = nullptr;
+  int32_t *top = nullptr, *trie = nullptr, *ulens = nullptr;
+  float *trie_f = nullptr, *rows = nullptr;
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
+  if (K > 0) CK(cudaMallocAsync(reinterpret_cast<void**>(&top), (size_t)(M > 0 ? M : 1) * K * sizeof(int32_t), s));
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)planes * B * cap * sizeof(int32_t), s));
+  if (lm) CK(cudaMallocAsync(reinterpret_cast<void**>(&trie_f), (size_t)B * cap * sizeof(float), s));
+  if (lm && !lm->word) CK(cudaMallocAsync(reinterpret_cast<void**>(&rows), (size_t)B * W * V * sizeof(float), s));
+  // The caller may reuse its array as soon as the call returns, and it may be pinned (then the copy would read it
+  // whenever the stream gets there): copy it to pageable memory of our own first.  cudaMemcpyAsync stages a
+  // pageable source before it returns, so this copy may go when the function does.
+  std::vector<int32_t> row_lens;
+  if (row_lens_host) {
+    row_lens.assign(row_lens_host, row_lens_host + B);
+    CK(cudaMallocAsync(reinterpret_cast<void**>(&ulens), (size_t)B * sizeof(int32_t), s));
+    CK(cudaMemcpyAsync(ulens, row_lens.data(), (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    lens_dev = ulens;
+    lens_stride = 1;
+  }
+  KL(launch_beam_rows(logits_dev, stats, top, M, (int)V, K, blank, L, lens_dev, lens_stride, s, nullptr));
+  if (!lm)
+    KL(launch_beam_search(logits_dev, stats, top, K, B, L, lens_dev, lens_stride, (int)V, W, blank, trie, cap,
+                          tokens_dev, out_lens_dev, scores_dev, s, nullptr));
+  else if (!lm->word)
+    KL(launch_beam_search_lm(logits_dev, stats, lm->view, lm_weight, B, L, lens_dev, lens_stride, (int)V, W, blank,
+                             trie, trie_f, cap, rows, tokens_dev, out_lens_dev, scores_dev, s));
+  else
+    KL(launch_beam_search_word_lm(logits_dev, stats, top, K, lm->view, lm->lex, lm_weight, word_score, B, L,
+                                  lens_dev, lens_stride, (int)V, W, blank, trie, trie_f, cap, tokens_dev,
+                                  out_lens_dev, scores_dev, s));
+  CK(cudaFreeAsync(stats, s));
+  if (top) CK(cudaFreeAsync(top, s));
+  CK(cudaFreeAsync(trie, s));
+  if (trie_f) CK(cudaFreeAsync(trie_f, s));
+  if (rows) CK(cudaFreeAsync(rows, s));
+  if (ulens) CK(cudaFreeAsync(ulens, s));
+  return VASR_OK;
+}
+
+}  // namespace
+
+int vasr_ctc_beam_search(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
+                         int32_t* tokens_dev, int32_t* lens_dev, double* scores_dev, void* stream) {
+  return beam_search(logits_dev, nullptr, nullptr, 0, B, L, V, beam_width, blank, nullptr, 0.0, 0.0, tokens_dev,
+                     lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
+}
+
 int vasr_ctc_beam_search_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
                             const vasr_lm* lm, double lm_weight, int32_t* tokens_dev, int32_t* lens_dev,
                             double* scores_dev, void* stream) {
   if (!lm) return fail(VASR_ERR_INVALID, "null LM");
   if (lm->word) return fail(VASR_ERR_INVALID, "a word LM runs in vasr_ctc_beam_search_word_lm");
-  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
-  if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
-  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
-  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
-  if (V != lm->view.V)
-    return fail(VASR_ERR_INVALID, "the LM is built for a vocabulary of " + std::to_string(lm->view.V) +
-                                      " tokens, the logits have " + std::to_string(V));
-  if (blank != lm->blank)
-    return fail(VASR_ERR_INVALID, "the LM is built with blank token " + std::to_string(lm->blank) +
-                                      ", the search uses " + std::to_string(blank));
-  if (!std::isfinite(lm_weight)) return fail(VASR_ERR_INVALID, "lm_weight must be finite");
-  if (B <= 0) return VASR_OK;
-  if (B * L > 0) {
-    cudaPointerAttributes at = {};
-    if (cudaPointerGetAttributes(&at, logits_dev) != cudaSuccess || at.type == cudaMemoryTypeUnregistered ||
-        at.type == cudaMemoryTypeHost || at.device != lm->device) {
-      cudaGetLastError();
-      return fail(VASR_ERR_INVALID, "the logits are not device memory on the LM's device (" +
-                                        std::to_string(lm->device) + ")");
-    }
-  }
-  DeviceGuard dev_guard(lm->device);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int W = beam_width;
-  const int64_t M = B * L, cap = 1 + L * W;
-  float2* stats = nullptr;
-  int32_t* trie = nullptr;
-  float *trie_lm = nullptr, *rows = nullptr;
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)5 * B * cap * sizeof(int32_t), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie_lm), (size_t)B * cap * sizeof(float), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&rows), (size_t)B * W * V * sizeof(float), s));
-  KL(launch_beam_rows(logits_dev, stats, nullptr, M, (int)V, 0, blank, s, nullptr));   // log-softmax stats only
-  KL(launch_beam_search_lm(logits_dev, stats, lm->view, lm_weight, B, L, (int)V, W, blank, trie, trie_lm, cap, rows,
-                           tokens_dev, lens_dev, scores_dev, s));
-  CK(cudaFreeAsync(stats, s));
-  CK(cudaFreeAsync(trie, s));
-  CK(cudaFreeAsync(trie_lm, s));
-  CK(cudaFreeAsync(rows, s));
-  return VASR_OK;
+  return beam_search(logits_dev, nullptr, nullptr, 0, B, L, V, beam_width, blank, lm, lm_weight, 0.0, tokens_dev,
+                     lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
 }
 
 int vasr_ctc_beam_search_word_lm(const float* logits_dev, int64_t B, int64_t L, int64_t V, int beam_width, int blank,
@@ -1426,49 +1481,16 @@ int vasr_ctc_beam_search_word_lm(const float* logits_dev, int64_t B, int64_t L, 
                                  int32_t* lens_dev, double* scores_dev, void* stream) {
   if (!lm) return fail(VASR_ERR_INVALID, "null LM");
   if (!lm->word) return fail(VASR_ERR_INVALID, "a token LM runs in vasr_ctc_beam_search_lm");
-  if (!tokens_dev && B * beam_width * L > 0) return fail(VASR_ERR_INVALID, "null argument");
-  if (!lens_dev || !scores_dev || (!logits_dev && B * L > 0)) return fail(VASR_ERR_INVALID, "null argument");
-  if (beam_width < 1 || beam_width > 32) return fail(VASR_ERR_INVALID, "beam_width must be in [1, 32]");
-  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
-  if (V != lm->vocab)
-    return fail(VASR_ERR_INVALID, "the LM is built for a vocabulary of " + std::to_string(lm->vocab) +
-                                      " tokens, the logits have " + std::to_string(V));
-  if (blank != lm->blank)
-    return fail(VASR_ERR_INVALID, "the LM is built with blank token " + std::to_string(lm->blank) +
-                                      ", the search uses " + std::to_string(blank));
-  if (!std::isfinite(lm_weight) || lm_weight < 0) return fail(VASR_ERR_INVALID, "lm_weight must be finite and >= 0");
-  if (!std::isfinite(word_score)) return fail(VASR_ERR_INVALID, "word_score must be finite");
-  if (B <= 0) return VASR_OK;
-  if (B * L > 0) {
-    cudaPointerAttributes at = {};
-    if (cudaPointerGetAttributes(&at, logits_dev) != cudaSuccess || at.type == cudaMemoryTypeUnregistered ||
-        at.type == cudaMemoryTypeHost || at.device != lm->device) {
-      cudaGetLastError();
-      return fail(VASR_ERR_INVALID, "the logits are not device memory on the LM's device (" +
-                                        std::to_string(lm->device) + ")");
-    }
-  }
-  DeviceGuard dev_guard(lm->device);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int W = beam_width;
-  // lexicon-free: each frame's W+2 best non-blank tokens (beam.cu: why W+2); constrained: log-softmax stats only
-  const int K = lm->lex.constrained ? 0 : (int)(V - 1 < W + 2 ? (V - 1 > 0 ? V - 1 : 1) : W + 2);
-  const int64_t M = B * L, cap = 1 + L * W;
-  float2* stats = nullptr;
-  int32_t *top = nullptr, *trie = nullptr;
-  float* trie_f = nullptr;
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&stats), (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&top), (size_t)(M * K > 0 ? M * K : 1) * sizeof(int32_t), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie), (size_t)9 * B * cap * sizeof(int32_t), s));
-  CK(cudaMallocAsync(reinterpret_cast<void**>(&trie_f), (size_t)B * cap * sizeof(float), s));
-  KL(launch_beam_rows(logits_dev, stats, top, M, (int)V, K, blank, s, nullptr));
-  KL(launch_beam_search_word_lm(logits_dev, stats, top, K, lm->view, lm->lex, lm_weight, word_score, B, L, (int)V, W,
-                                blank, trie, trie_f, cap, tokens_dev, lens_dev, scores_dev, s));
-  CK(cudaFreeAsync(stats, s));
-  CK(cudaFreeAsync(top, s));
-  CK(cudaFreeAsync(trie, s));
-  CK(cudaFreeAsync(trie_f, s));
-  return VASR_OK;
+  return beam_search(logits_dev, nullptr, nullptr, 0, B, L, V, beam_width, blank, lm, lm_weight, word_score,
+                     tokens_dev, lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
+}
+
+int vasr_ctc_beam_search_ragged(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L,
+                                int64_t V, int beam_width, int blank, const vasr_lm* lm, double lm_weight,
+                                double word_score, int32_t* tokens_dev, int32_t* lens_dev, double* scores_dev,
+                                void* stream) {
+  return beam_search(logits_dev, row_lens_host, nullptr, 0, B, L, V, beam_width, blank, lm, lm_weight, word_score,
+                     tokens_dev, lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
 }
 
 // Per-utterance dims of a ragged batch -> k.ragbuf, k.rag.  `lens` (host) are samples (from_samples) or mel
@@ -1587,6 +1609,85 @@ int vasr_transcribe_ragged_host(vasr_handle* h, const float* pcm_host, const int
   DeviceGuard dev_guard(h->device);
   return transcribe_impl(h, nullptr, pcm_host, B, S, nullptr, nullptr, tokens_host, lens_host, h->own_stream,
                          sample_lens_host);
+}
+
+// PCM -> n-best: transcribe_impl's sequence with the logits-writing CTC head (vasr_forward's, for the fp32 and the
+// FakeQuantize model alike) and the prefix beam search in place of the greedy decode.  A ragged batch's search
+// reads each utterance's token count from the uploaded dims (RAG_L).  Host variant: results come back through
+// device scratch and the call synchronises once at the end.
+static int transcribe_beam_impl(vasr_handle* h, const float* pcm_dev, const float* pcm_host,
+                                const int32_t* sample_lens, int64_t B, int64_t S, int beam_width, const vasr_lm* lm,
+                                double lm_weight, double word_score, int32_t* tokens, int32_t* lens, double* scores,
+                                cudaStream_t s) {
+  const bool host = pcm_host != nullptr;
+  if (lm && lm->device != h->device)
+    return fail(VASR_ERR_INVALID, "the LM is on device " + std::to_string(lm->device) + ", the model on " +
+                                      std::to_string(h->device));
+  const Dims q = make_dims(h, B, S, vasr_num_frames(S));
+  // every argument of the search is checked before any device work (sample_lens by upload_ragged below)
+  RET(beam_check(nullptr, B, q.L, q.V, beam_width, 0, lm, lm_weight, word_score, tokens, lens, scores));
+  if (B == 0) return VASR_OK;
+  CallOrder call_order(h, s);
+  Work k;
+  RET(ensure_workspace(h, q, true, true, &k, host));
+  if (sample_lens) RET(upload_ragged(h, q, k, sample_lens, true, s));
+  const int64_t W = beam_width;
+  int32_t *tok_dev = tokens, *len_dev = lens;
+  double* sc_dev = scores;
+  // host variant: device copies of the results, released (stream-ordered) on every return, errors included
+  struct Stage {
+    void* p[3] = {};
+    cudaStream_t s;
+    ~Stage() {
+      for (void* q : p)
+        if (q) cudaFreeAsync(q, s);
+    }
+  } stage{{}, s};
+  if (host) {
+    CK(cudaMallocAsync(&stage.p[0], (size_t)B * W * q.L * sizeof(int32_t), s));
+    CK(cudaMallocAsync(&stage.p[1], (size_t)B * W * sizeof(int32_t), s));
+    CK(cudaMallocAsync(&stage.p[2], (size_t)B * W * sizeof(double), s));
+    tok_dev = static_cast<int32_t*>(stage.p[0]);
+    len_dev = static_cast<int32_t*>(stage.p[1]);
+    sc_dev = static_cast<double*>(stage.p[2]);
+  }
+  timing_begin(h, s);
+  if (host) RET(run_mel_from_host(h, q, k, pcm_host, s));
+  else RET(run_mel(h, q, k, pcm_dev, 1, s));
+  KL(launch_mel_finish(k.raw, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  RET(run_model(h, q, k, k.logits, nullptr, nullptr, nullptr, s));
+  RET(beam_search(k.logits, nullptr, k.rag ? k.rag + RAG_L : nullptr, RAG_STRIDE, q.B, q.L, q.V, beam_width, 0, lm,
+                  lm_weight, word_score, tok_dev, len_dev, sc_dev, s));
+  timing_end(h, s);
+  if (host) {
+    CK(cudaMemcpyAsync(tokens, tok_dev, (size_t)B * W * q.L * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(lens, len_dev, (size_t)B * W * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(scores, sc_dev, (size_t)B * W * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+  }
+  return VASR_OK;
+}
+
+int vasr_transcribe_beam(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B, int64_t S,
+                         int beam_width, const vasr_lm* lm, double lm_weight, double word_score, int32_t* tokens_dev,
+                         int32_t* lens_dev, double* scores_dev, void* stream) {
+  RET(check_ready(h));
+  if (B < 0 || !pcm_dev) return fail(VASR_ERR_INVALID, "null argument");
+  if (S <= PAD) return fail(VASR_ERR_SHAPE, "reflect padding needs more than 200 samples (audio.py:100-101)");
+  DeviceGuard dev_guard(h->device);
+  return transcribe_beam_impl(h, pcm_dev, nullptr, sample_lens_host, B, S, beam_width, lm, lm_weight, word_score,
+                              tokens_dev, lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
+}
+
+int vasr_transcribe_beam_host(vasr_handle* h, const float* pcm_host, const int32_t* sample_lens_host, int64_t B,
+                              int64_t S, int beam_width, const vasr_lm* lm, double lm_weight, double word_score,
+                              int32_t* tokens_host, int32_t* lens_host, double* scores_host) {
+  RET(check_ready(h));
+  if (B <= 0 || !pcm_host) return fail(VASR_ERR_INVALID, "null argument");
+  if (S <= PAD) return fail(VASR_ERR_SHAPE, "reflect padding needs more than 200 samples (audio.py:100-101)");
+  DeviceGuard dev_guard(h->device);
+  return transcribe_beam_impl(h, nullptr, pcm_host, sample_lens_host, B, S, beam_width, lm, lm_weight, word_score,
+                              tokens_host, lens_host, scores_host, h->own_stream);
 }
 
 int vasr_forward_ragged(vasr_handle* h, const float* mel_dev, const int32_t* frame_lens_host, int64_t B, int64_t T,

@@ -153,14 +153,17 @@ cudaError_t launch_ctc_collapse(int32_t* pred, int32_t* tokens, int32_t* lens, i
 
 // ---------------------------------------------------------------- CTC prefix beam search
 // per (utterance, frame) row: stats = (max, log sum exp(x - max)); top_tok (M, K) = the K best non-blank
-// tokens by log-prob, ties to the lower id, -1 padded
+// tokens by log-prob, ties to the lower id, -1 padded.  M = B * L.  lens (optional, B entries at lens[b *
+// lens_stride], e.g. the RAG_L column of a ragged dims buffer): rows b * L + t with t >= lens[b] are skipped.
 cudaError_t launch_beam_rows(const float* logits, float2* stats, int32_t* top_tok, int64_t M, int V, int K,
-                             int blank, cudaStream_t s, int64_t* launches);
+                             int blank, int64_t L, const int32_t* lens, int lens_stride, cudaStream_t s,
+                             int64_t* launches);
 // trie: 3 x (B, trie_cap) int32 (parent | token | depth), trie_cap >= 1 + L * W.  out_tokens (B, W, L),
-// out_lens (B, W) (-1 = no such beam), out_scores (B, W) fp64, best first.
+// out_lens (B, W) (-1 = no such beam), out_scores (B, W) fp64, best first.  lens as in launch_beam_rows:
+// utterance b is searched over its first lens[b] rows (NULL: all L); its token rows are -1 past each beam's length.
 cudaError_t launch_beam_search(const float* logits, const float2* stats, const int32_t* top_tok, int K, int64_t B,
-                               int64_t L, int V, int W, int blank, int32_t* trie, int64_t trie_cap,
-                               int32_t* out_tokens, int32_t* out_lens, double* out_scores, cudaStream_t s,
-                               int64_t* launches);
+                               int64_t L, const int32_t* lens, int lens_stride, int V, int W, int blank,
+                               int32_t* trie, int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens,
+                               double* out_scores, cudaStream_t s, int64_t* launches);
 
 }  // namespace vasr

@@ -159,10 +159,11 @@ cudaError_t launch_lm_log_prob(const LmView& lm, const int32_t* prefixes, const 
                                const int32_t* tokens, float* out, cudaStream_t s);
 // The prefix beam search with the LM fused (beam.cu); stats from launch_beam_rows.  trie: 5 x (B, trie_cap) int32
 // (parent | token | depth | first child | next sibling), trie_lm (B, trie_cap) fp32, rows (B, W, V) fp32 scratch.
+// lens / lens_stride: the optional per-utterance frame counts of launch_beam_search.
 cudaError_t launch_beam_search_lm(const float* logits, const float2* stats, const LmView& lm, double lm_weight,
-                                  int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_lm,
-                                  int64_t trie_cap, float* rows, int32_t* out_tokens, int32_t* out_lens,
-                                  double* out_scores, cudaStream_t s);
+                                  int64_t B, int64_t L, const int32_t* lens, int lens_stride, int V, int W, int blank,
+                                  int32_t* trie, float* trie_lm, int64_t trie_cap, float* rows, int32_t* out_tokens,
+                                  int32_t* out_lens, double* out_scores, cudaStream_t s);
 
 struct LexHostTables {
   std::vector<std::string> words;              // word id -> string (the unigram words, <s> excluded, file order)
@@ -178,10 +179,11 @@ bool lm_parse_word_arpa(const char* path, const char* const* vocab, int V, int b
 cudaError_t lex_upload(const LexHostTables& x, bool constrained, void** block, LexView* view);
 // The prefix beam search with a word LM fused (beam.cu).  top_tok (B*L, K) from launch_beam_rows (lexicon-free mode
 // only, K = min(W + 2, V - 1)); trie: 9 x (B, trie_cap) int32, trie_f (B, trie_cap) fp32.
+// lens / lens_stride as in launch_beam_search; the end-of-utterance step follows each utterance's last frame.
 cudaError_t launch_beam_search_word_lm(const float* logits, const float2* stats, const int32_t* top_tok, int K,
                                        const LmView& lm, const LexView& lx, double lm_weight, double word_score,
-                                       int64_t B, int64_t L, int V, int W, int blank, int32_t* trie, float* trie_f,
-                                       int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens, double* out_scores,
-                                       cudaStream_t s);
+                                       int64_t B, int64_t L, const int32_t* lens, int lens_stride, int V, int W,
+                                       int blank, int32_t* trie, float* trie_f, int64_t trie_cap, int32_t* out_tokens,
+                                       int32_t* out_lens, double* out_scores, cudaStream_t s);
 
 }  // namespace vasr

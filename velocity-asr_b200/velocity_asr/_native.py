@@ -51,6 +51,12 @@ _SIGNATURES = {
     "vasr_lm_lexicon_size": (c_int64, [c_void_p]),
     "vasr_ctc_beam_search_word_lm": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_double,
                                              c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_ctc_beam_search_ragged": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p,
+                                            c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_transcribe_beam": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_double,
+                                     c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_transcribe_beam_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_double,
+                                          c_double, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "vasr_transcribe_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),

@@ -109,24 +109,10 @@ class DecodingResult:
     timestamps: Optional[List[Tuple[int, int]]] = None
 
 
-def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int = BLANK_TOKEN,
-                    lm_weight: float = 0.0, lm_scorer: Optional[Any] = None,
-                    word_score: float = 0.0) -> List[List[DecodingResult]]:
-    """decode.py:128-217 on the GPU: per utterance the `beam_width` best prefixes, best first, with the
-    reference's rule (log_softmax; blank / repeated token keep the prefix, any other token extends it; equal
-    prefixes keep the better score; fp64 score sums; ties in insertion order).
-
-    Shallow fusion: with an NGramLM as `lm_scorer` and lm_weight > 0, an offer that extends a prefix by `tok`
-    scores (score + log_prob[tok]) + lm_weight * lm(prefix, tok); blank and repeat offers are unchanged and the
-    returned scores are the fused ones.  The LM must be built for this vocabulary size and blank token and live on
-    the logits' device (host logits are staged to it).  A Python `lm_scorer` callback cannot run inside the device
-    loop and is refused rather than silently ignored.
-
-    With a WordNGramLM, words are spelled in the vocabulary and closed by its delimiter: closing a non-empty word
-    adds lm_weight * lm(history, word) + word_score, and the end of the utterance closes the last word and adds
-    lm_weight * lm(history, </s>) (include/vasr.h states the rule).  lm_weight must be finite and >= 0 and
-    word_score finite.  A lexicon-free word LM with lm_weight == 0 and word_score == 0 takes the plain search; in
-    lexicon-constrained mode beams that cannot end on a lexicon word are dropped, so fewer may come back."""
+def _search_lm(lm_scorer: Optional[Any], lm_weight: float, word_score: float):
+    """The LM rules shared by ctc_beam_search and VELOCITYASR.transcribe_beam: the LM to search with, or None when
+    the search runs LM-free (off means off).  A Python `lm_scorer` callback with lm_weight > 0 cannot run inside the
+    device loop and is refused rather than silently ignored."""
     word_lm = isinstance(lm_scorer, WordNGramLM)
     if word_lm:
         if not (math.isfinite(lm_weight) and lm_weight >= 0):
@@ -141,22 +127,65 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     if lm_scorer is not None and lm_weight > 0 and not use_lm:
         raise NotImplementedError("velocity_asr (B200 build): ctc_beam_search runs on the device and takes no "
                                   "Python lm_scorer (use velocity_asr.NGramLM)")
+    return lm_scorer if use_lm else None
+
+
+def _check_lm_fits(lm, V: int, blank_token: int) -> None:
+    lm._live()
+    if V != lm.vocab_size:
+        raise ValueError(f"the LM is built for a vocabulary of {lm.vocab_size} tokens, the logits have {V}")
+    if int(blank_token) != lm.blank_token:
+        raise ValueError(f"the LM is built with blank token {lm.blank_token}, the search uses {blank_token}")
+
+
+def _beam_results(tokens: torch.Tensor, lens: torch.Tensor, scores: torch.Tensor) -> List[List[DecodingResult]]:
+    """(B, W, L) tokens, (B, W) lens (-1: no such beam), (B, W) fp64 scores -> per utterance its beams, best first."""
+    tokens, lens, scores = tokens.cpu().numpy(), lens.cpu().tolist(), scores.cpu().tolist()
+    return [[DecodingResult(text="", tokens=tokens[b, r, :n].tolist(), score=scores[b][r])
+             for r, n in enumerate(lens[b]) if n >= 0] for b in range(len(lens))]
+
+
+def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int = BLANK_TOKEN,
+                    lm_weight: float = 0.0, lm_scorer: Optional[Any] = None,
+                    word_score: float = 0.0, lengths=None) -> List[List[DecodingResult]]:
+    """decode.py:128-217 on the GPU: per utterance the `beam_width` best prefixes, best first, with the
+    reference's rule (log_softmax; blank / repeated token keep the prefix, any other token extends it; equal
+    prefixes keep the better score; fp64 score sums; ties in insertion order).
+
+    Shallow fusion: with an NGramLM as `lm_scorer` and lm_weight > 0, an offer that extends a prefix by `tok`
+    scores (score + log_prob[tok]) + lm_weight * lm(prefix, tok); blank and repeat offers are unchanged and the
+    returned scores are the fused ones.  The LM must be built for this vocabulary size and blank token and live on
+    the logits' device (host logits are staged to it).  A Python `lm_scorer` callback cannot run inside the device
+    loop and is refused rather than silently ignored.
+
+    With a WordNGramLM, words are spelled in the vocabulary and closed by its delimiter: closing a non-empty word
+    adds lm_weight * lm(history, word) + word_score, and the end of the utterance closes the last word and adds
+    lm_weight * lm(history, </s>) (include/vasr.h states the rule).  lm_weight must be finite and >= 0 and
+    word_score finite.  A lexicon-free word LM with lm_weight == 0 and word_score == 0 takes the plain search; in
+    lexicon-constrained mode beams that cannot end on a lexicon word are dropped, so fewer may come back.
+
+    `lengths` (B frame counts, each in [0, L]; a list, tuple or tensor): a ragged batch, such as the logits of
+    forward(mel, lengths=...).  Utterance b is searched over its first lengths[b] frames only and gets bit for bit
+    what ctc_beam_search(logits[b:b+1, :lengths[b]]) gives; the padding rows are never read.  A wrong count or a
+    length outside [0, L] raises RuntimeError before any device work."""
+    lm = _search_lm(lm_scorer, lm_weight, word_score)
     if logits.dim() != 3:
         raise RuntimeError(f"expected (batch, seq_len, vocab) logits, got {tuple(logits.shape)}")
-    if use_lm:
-        lm_scorer._live()
-        if logits.shape[-1] != lm_scorer.vocab_size:
-            raise ValueError(f"the LM is built for a vocabulary of {lm_scorer.vocab_size} tokens, the logits have "
-                             f"{logits.shape[-1]}")
-        if int(blank_token) != lm_scorer.blank_token:
-            raise ValueError(f"the LM is built with blank token {lm_scorer.blank_token}, the search uses {blank_token}")
+    B, L, V = logits.shape
+    rows = None
+    if lengths is not None:
+        from .model import _lengths_tensor
+        rows = _lengths_tensor(lengths, B)
+        if B and (int(rows.min()) < 0 or int(rows.max()) > L):
+            raise RuntimeError(f"every length must be in [0, {L}], got {rows.tolist()}")
+    if lm is not None:
+        _check_lm_fits(lm, V, blank_token)
         if logits.device.type != "cuda":   # host logits: staged to the LM's device
-            logits = logits.to(lm_scorer.device)
-        elif logits.device != lm_scorer.device:
-            raise ValueError(f"the LM is on {lm_scorer.device}, the logits on {logits.device}")
+            logits = logits.to(lm.device)
+        elif logits.device != lm.device:
+            raise ValueError(f"the LM is on {lm.device}, the logits on {logits.device}")
     elif logits.device.type != "cuda":     # host logits: staged to the current CUDA device (no CPU decoder exists)
         logits = logits.to(_native.default_cuda_device())
-    B, L, V = logits.shape
     W = int(beam_width)
     if B == 0:
         return []
@@ -164,24 +193,12 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     tokens = torch.empty(B, W, max(L, 1), dtype=torch.int32, device=lg.device)
     lens = torch.empty(B, W, dtype=torch.int32, device=lg.device)
     scores = torch.empty(B, W, dtype=torch.float64, device=lg.device)
-    lib = _native.lib()
     with torch.cuda.device(lg.device):
-        stream = ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)
-        if use_lm and word_lm:
-            _native.check(lib.vasr_ctc_beam_search_word_lm(
-                _native.ptr(lg), B, L, V, W, int(blank_token), lm_scorer._handle, float(lm_weight), float(word_score),
-                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), stream))
-        elif use_lm:
-            _native.check(lib.vasr_ctc_beam_search_lm(
-                _native.ptr(lg), B, L, V, W, int(blank_token), lm_scorer._handle, float(lm_weight),
-                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), stream))
-        else:
-            _native.check(lib.vasr_ctc_beam_search(
-                _native.ptr(lg), B, L, V, W, int(blank_token), _native.ptr(tokens), _native.ptr(lens),
-                _native.ptr(scores), stream))
-    tokens, lens, scores = tokens.cpu().numpy(), lens.cpu().tolist(), scores.cpu().tolist()
-    return [[DecodingResult(text="", tokens=tokens[b, r, :n].tolist(), score=scores[b][r])
-             for r, n in enumerate(lens[b]) if n >= 0] for b in range(B)]
+        _native.check(_native.lib().vasr_ctc_beam_search_ragged(
+            _native.ptr(lg), _native.ptr(rows), B, L, V, W, int(blank_token), lm._handle if lm is not None else None,
+            float(lm_weight), float(word_score), _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores),
+            ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)))
+    return _beam_results(tokens, lens, scores)
 
 
 class CTCDecoder:
@@ -198,11 +215,13 @@ class CTCDecoder:
         return [self._tokens_to_text(s) for s in seqs]
 
     def decode_beam_search(self, logits: torch.Tensor, beam_width: int = 10, return_all_beams: bool = False,
-                           lm_scorer: Optional[Any] = None, lm_weight: float = 0.0, word_score: float = 0.0):
+                           lm_scorer: Optional[Any] = None, lm_weight: float = 0.0, word_score: float = 0.0,
+                           lengths=None):
         """decode.py:265-300: best-beam texts, or every beam with its text filled in.  `lm_scorer` / `lm_weight` /
-        `word_score` go to ctc_beam_search (shallow fusion with an NGramLM or a WordNGramLM)."""
+        `word_score` / `lengths` go to ctc_beam_search (shallow fusion with an NGramLM or a WordNGramLM; a ragged
+        batch)."""
         beams = ctc_beam_search(logits, beam_width=beam_width, blank_token=self.blank_token, lm_weight=lm_weight,
-                                lm_scorer=lm_scorer, word_score=word_score)
+                                lm_scorer=lm_scorer, word_score=word_score, lengths=lengths)
         if return_all_beams:
             for utt in beams:
                 for r in utt:

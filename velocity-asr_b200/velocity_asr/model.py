@@ -272,6 +272,56 @@ class VELOCITYASR(nn.Module):
         return _token_lists(tokens, lens)
 
     @torch.no_grad()
+    def transcribe_beam(self, audio: torch.Tensor, lengths=None, beam_width: int = 10, lm_scorer=None,
+                        lm_weight: float = 0.0, word_score: float = 0.0):
+        """Fused PCM -> n-best: 16 kHz PCM (S,) | (B, S) -> per utterance its `beam_width` best prefixes
+        (List[List[DecodingResult]], best first, text ""), in one native call: log-mel, forward, the CTC head writing
+        logits, and the device prefix beam search (ctc_beam_search, blank 0), with or without an NGramLM /
+        WordNGramLM under the same rules and errors.  The LM must live on the model's execution device.
+        `lengths` (B sample counts): a ragged batch as in transcribe().  Utterance b gets bit for bit
+        ctc_beam_search(forward(compute_mel_spectrogram(audio[b, :lengths[b]]).unsqueeze(0)), ...)[0].
+        A CUDA tensor is consumed in place; a CPU tensor (pin it) is copied in inside the call."""
+        from .decode import _beam_results, _check_lm_fits, _search_lm
+        lm = _search_lm(lm_scorer, lm_weight, word_score)
+        if audio.dim() == 1:
+            audio = audio.unsqueeze(0)
+        B, S = audio.shape
+        dev = self._exec_device(audio)
+        slen = None if lengths is None else _lengths_tensor(lengths, B)
+        if lm is not None:
+            _check_lm_fits(lm, self.config.vocab_size, 0)
+            if lm.device.index != (dev.index if dev.index is not None else torch.cuda.current_device()):
+                raise ValueError(f"the LM is on {lm.device}, the model runs on {dev}")
+        W = int(beam_width)
+        if not 1 <= W <= 32:       # before the result buffers are sized by it; the library's rule and exception type
+            raise ValueError(f"beam_width must be in [1, 32], got {W}")
+        eng = self._engine(dev)
+        L = self.get_output_length(1 + S // 160)
+        hlm = lm._handle if lm is not None else None
+        if audio.device.type == "cpu":
+            pcm = audio.to(torch.float32).contiguous()
+            cache = self.__dict__.setdefault("_pinned_beam_out", {})   # per shape, as transcribe() does
+            if (B, W, L) not in cache:
+                if len(cache) >= 8:
+                    cache.clear()
+                cache[(B, W, L)] = (torch.empty(B, W, L, dtype=torch.int32, pin_memory=True),
+                                    torch.empty(B, W, dtype=torch.int32, pin_memory=True),
+                                    torch.empty(B, W, dtype=torch.float64, pin_memory=True))
+            tokens, lens, scores = cache[(B, W, L)]
+            _native.check(eng.lib.vasr_transcribe_beam_host(
+                eng.handle, _native.ptr(pcm), _native.ptr(slen), B, S, W, hlm, float(lm_weight), float(word_score),
+                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores)))
+        else:
+            pcm = self._check_input(audio, "audio")
+            tokens = torch.empty(B, W, L, dtype=torch.int32, device=pcm.device)
+            lens = torch.empty(B, W, dtype=torch.int32, device=pcm.device)
+            scores = torch.empty(B, W, dtype=torch.float64, device=pcm.device)
+            _native.check(eng.lib.vasr_transcribe_beam(
+                eng.handle, _native.ptr(pcm), _native.ptr(slen), B, S, W, hlm, float(lm_weight), float(word_score),
+                _native.ptr(tokens), _native.ptr(lens), _native.ptr(scores), _stream_ptr(pcm.device)))
+        return _beam_results(tokens, lens, scores)
+
+    @torch.no_grad()
     def transcribe_batches(self, batches: Iterable[torch.Tensor], as_arrays: bool = False
                            ) -> Iterator[List[List[int]]]:
         """transcribe() over a stream of host batches, pipelined: while the kernels of batch i run,
