@@ -248,6 +248,54 @@ int vasr_transcribe_beam_host(vasr_handle* h, const float* pcm_host, const int32
                               int64_t S, int beam_width, const vasr_lm* lm, double lm_weight, double word_score,
                               int32_t* tokens_host, int32_t* lens_host, double* scores_host);
 
+/* ---- CTC forced alignment and transcript log-likelihood
+ * Inputs: logits (B, L, V), utterance b over its first row_lens[b] frames; a target y = targets[b, :target_lens[b]]
+ * of length U; blank.  Per-frame log-probs lp[t][v]: by default the beam search's fp32 table
+ * (x - max) - log sum exp(x - max), from the statistics of beam_rows_kernel; with log_probs != 0 the inputs already
+ * are log-probs and are read as they are.
+ * States are the usual CTC expansion blank, y0, blank, y1, ..., blank: 2U + 1 states with label(s).  From s-1 any
+ * state may be entered; from s-2 only when label(s) != blank and label(s) != label(s-2).  All sums are fp64 of fp32
+ * lp values, added in time order.
+ * Viterbi (vasr_ctc_align): delta[0][0] = lp[0][blank], delta[0][1] = lp[0][y0], every other state at frame 0 is
+ * -inf; for t >= 1 delta[t][s] = max(delta[t-1][s], delta[t-1][s-1], delta[t-1][s-2]) + lp[t][label(s)].  Inside the
+ * max the first candidate, in the order stay, s-1, s-2, that has the strictly greatest value wins.  The final state
+ * is 2U-1 (last token) or 2U (trailing blank); on a tie the last-token state wins.  Outputs: frame_labels (B, L) int32,
+ * the token id of the state the best path occupies at each frame, blank included; frame_log_probs (B, L) fp32, lp at
+ * that frame and label; scores (B) fp64, the path score.  Equal neighbouring targets are always separated by a blank,
+ * so frame labels identify target positions: token k spans [first frame in state 2k+1, last frame + 1), the units and
+ * the half-open convention of vasr_ctc_greedy_timestamps.
+ * Log-likelihood (vasr_ctc_log_likelihood): the same lattice with the max replaced by a log-add in fp64: with m the
+ * largest present term, m + log sum exp(x_i - m), and -inf when every term is -inf; the end is the log-add of the
+ * two final states.  The result equals -ctc_loss(reduction="none") of that utterance.
+ * Edge cases: U = 0 is the all-blank path (with row_lens[b] = 0 as well the score is 0).  A target that cannot fit
+ * (row_lens[b] < U + the number of equal neighbouring targets, row_lens[b] = 0 < U included) gets score -inf, and its
+ * frames label -1 and log-prob 0.  Frames at or past row_lens[b] are never read, so NaN padding cannot matter; they
+ * also get label -1 and log-prob 0.
+ * Contract: utterance b gets bit for bit what the same call gives on logits[b:b+1, :row_lens[b]] with targets[b:b+1].
+ * row_lens_host (B, or NULL: every utterance has L frames), targets_host (B, U_max) and target_lens_host (B) are HOST
+ * arrays, copied before the call returns.  Checks, all before any device call: VASR_ERR_INVALID for a null pointer,
+ * blank outside [0, V), or a target id outside [0, V) or equal to blank (only the first target_lens[b] entries of a
+ * row are read); VASR_ERR_SHAPE for row_lens[b] outside [0, L] or target_lens[b] outside [0, U_max].
+ * Device scratch, allocated stream-ordered per call, with U = the largest target_lens[b]: the Viterbi backpointers,
+ * B * L * ceil((2U + 1) / 16) * 4 bytes (2 bits per state and frame); B * L * 8 bytes of row statistics unless
+ * log_probs; and when the 2U + 1 fp64 scores of an utterance do not fit the shared memory of one CTA (U above about
+ * 12,000 on a B200) about B * (2U + 1) * 8 bytes more. */
+int vasr_ctc_align(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int blank,
+                   int log_probs, const int32_t* targets_host, const int32_t* target_lens_host, int64_t U_max,
+                   int32_t* frame_labels_dev, float* frame_log_probs_dev, double* scores_dev, void* stream);
+/* The same inputs; ll (B) fp64 is the only output. */
+int vasr_ctc_log_likelihood(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V,
+                            int blank, int log_probs, const int32_t* targets_host, const int32_t* target_lens_host,
+                            int64_t U_max, double* ll_dev, void* stream);
+/* PCM -> forced alignment in one call: the sequence of vasr_transcribe_beam (log-mel, model, the CTC head writing
+ * logits into the workspace, blank 0, a ragged batch by sample_lens_host) with vasr_ctc_align in place of the search.
+ * L = vasr_num_tokens(vasr_num_frames(S)); outputs as vasr_ctc_align.  Works for the fp32 and the FakeQuantize model.
+ * Contract: utterance b gets bit for bit what vasr_ctc_align gives on the logits vasr_forward produces for that
+ * utterance alone (its first sample_lens[b] samples, or all S). */
+int vasr_align(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B, int64_t S,
+               const int32_t* targets_host, const int32_t* target_lens_host, int64_t U_max, int32_t* frame_labels_dev,
+               float* frame_log_probs_dev, double* scores_dev, void* stream);
+
 /* ---- transcribe: load -> mel -> model -> greedy (scripts/transcribe.py:69-82), batched.
  * tokens (B, L) int32, lens (B); L = vasr_num_tokens(vasr_num_frames(S)). */
 int vasr_transcribe(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S,

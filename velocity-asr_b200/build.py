@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "velocity_asr", "libvasr.so")
-SOURCES = ["engine.cu", "gemm.cu", "gemm_tc.cu", "norm_conv.cu", "scan.cu", "mel.cu", "context.cu", "ctc.cu", "beam.cu", "lm.cu"]
+SOURCES = ["engine.cu", "gemm.cu", "gemm_tc.cu", "norm_conv.cu", "scan.cu", "mel.cu", "context.cu", "ctc.cu", "beam.cu", "lm.cu", "align.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-O3,-Wall", "--expt-relaxed-constexpr"]
 

@@ -1493,6 +1493,114 @@ int vasr_ctc_beam_search_ragged(const float* logits_dev, const int32_t* row_lens
                      tokens_dev, lens_dev, scores_dev, static_cast<cudaStream_t>(stream));
 }
 
+namespace {
+
+// Argument checks of every alignment entry point (no device call).  Only the first target_lens[b] ids of a row are
+// read.  row_lens_host (optional): B frame counts, each in [0, L].
+int align_check(const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int blank, const int32_t* targets_host,
+                const int32_t* target_lens_host, int64_t U_max) {
+  if (B < 0 || L < 0 || U_max < 0) return fail(VASR_ERR_SHAPE, "negative size");
+  if (B > 0 && (!target_lens_host || (!targets_host && U_max > 0))) return fail(VASR_ERR_INVALID, "null argument");
+  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  for (int64_t b = 0; b < B; ++b) {
+    const int64_t U = target_lens_host[b];
+    if (U < 0 || U > U_max)
+      return fail(VASR_ERR_SHAPE, "every target length must be in [0, U_max] (utterance " + std::to_string(b) +
+                                      " has " + std::to_string(U) + ")");
+    for (int64_t u = 0; u < U; ++u) {
+      const int32_t id = targets_host[b * U_max + u];
+      if (id < 0 || id >= V || id == blank)
+        return fail(VASR_ERR_INVALID, "target id " + std::to_string(id) + " of utterance " + std::to_string(b) +
+                                          " is outside the vocabulary or the blank");
+    }
+  }
+  if (row_lens_host)
+    for (int64_t b = 0; b < B; ++b)
+      if (row_lens_host[b] < 0 || row_lens_host[b] > L)
+        return fail(VASR_ERR_SHAPE, "ragged alignment: every utterance needs between 0 and L frames (utterance " +
+                                        std::to_string(b) + " has " + std::to_string(row_lens_host[b]) + ")");
+  return VASR_OK;
+}
+
+// The body of every alignment entry point after its checks: scratch, the row statistics and the alignment kernel.
+// ll == NULL: Viterbi into labels / lps / scores; else the log-likelihood into ll.  Frame counts as beam_search.
+int ctc_align_run(const float* logits_dev, const int32_t* row_lens_host, const int32_t* lens_dev, int lens_stride,
+                  int64_t B, int64_t L, int64_t V, int blank, int log_probs, const int32_t* targets_host,
+                  const int32_t* target_lens_host, int64_t U_max, int32_t* labels, float* lps, double* scores,
+                  double* ll, cudaStream_t s) {
+  if (B <= 0) return VASR_OK;
+  const bool viterbi = ll == nullptr;
+  int64_t U = 0;
+  for (int64_t b = 0; b < B; ++b) U = target_lens_host[b] > U ? target_lens_host[b] : U;
+  int threads = 0, E = 0;
+  ctc_align_layout(U, viterbi, &threads, &E);
+  int dev = 0, smem_max = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  const bool delta_smem = ctc_align_smem(threads, E, true) <= (size_t)smem_max;
+  const int64_t M = B * L, words = ctc_align_words(U);
+  // host arrays -> one pageable copy of our own ([target_lens | row_lens | targets]), so the caller may reuse its
+  // arrays, pinned or not, as soon as the call returns (cudaMemcpyAsync stages a pageable source before returning)
+  std::vector<int32_t> pack((size_t)(2 * B + B * U_max));
+  std::copy(target_lens_host, target_lens_host + B, pack.begin());
+  if (row_lens_host) std::copy(row_lens_host, row_lens_host + B, pack.begin() + B);
+  if (U_max > 0) std::copy(targets_host, targets_host + B * U_max, pack.begin() + 2 * B);
+  // scratch, released (stream-ordered) on every return, errors included
+  struct Scratch {
+    void* p[4] = {};
+    cudaStream_t s;
+    ~Scratch() {
+      for (void* q : p)
+        if (q) cudaFreeAsync(q, s);
+    }
+  } scratch{{}, s};
+  CK(cudaMallocAsync(&scratch.p[0], pack.size() * sizeof(int32_t), s));
+  int32_t* packed = static_cast<int32_t*>(scratch.p[0]);
+  CK(cudaMemcpyAsync(packed, pack.data(), pack.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  if (row_lens_host) {
+    lens_dev = packed + B;
+    lens_stride = 1;
+  }
+  if (!log_probs) CK(cudaMallocAsync(&scratch.p[1], (size_t)(M > 0 ? M : 1) * sizeof(float2), s));
+  if (!delta_smem) CK(cudaMallocAsync(&scratch.p[2], (size_t)B * E * threads * sizeof(double), s));
+  if (viterbi) CK(cudaMallocAsync(&scratch.p[3], (size_t)(M > 0 ? M : 1) * words * sizeof(uint32_t), s));
+  float2* stats = static_cast<float2*>(scratch.p[1]);
+  if (!log_probs) KL(launch_beam_rows(logits_dev, stats, nullptr, M, (int)V, 0, blank, L, lens_dev, lens_stride, s,
+                                      nullptr));
+  KL(launch_ctc_align(logits_dev, stats, B, L, (int)V, blank, lens_dev, lens_stride, packed + 2 * B, U_max, packed,
+                      threads, E, static_cast<double*>(scratch.p[2]), static_cast<uint32_t*>(scratch.p[3]), words,
+                      labels, lps, viterbi ? scores : ll, s));
+  return VASR_OK;
+}
+
+int ctc_align_entry(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int blank,
+                    int log_probs, const int32_t* targets_host, const int32_t* target_lens_host, int64_t U_max,
+                    int32_t* labels, float* lps, double* scores, double* ll, void* stream) {
+  if (!logits_dev && B * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  RET(align_check(row_lens_host, B, L, V, blank, targets_host, target_lens_host, U_max));
+  return ctc_align_run(logits_dev, row_lens_host, nullptr, 0, B, L, V, blank, log_probs, targets_host,
+                       target_lens_host, U_max, labels, lps, scores, ll, static_cast<cudaStream_t>(stream));
+}
+
+}  // namespace
+
+int vasr_ctc_align(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int blank,
+                   int log_probs, const int32_t* targets_host, const int32_t* target_lens_host, int64_t U_max,
+                   int32_t* frame_labels_dev, float* frame_log_probs_dev, double* scores_dev, void* stream) {
+  if (!scores_dev || ((!frame_labels_dev || !frame_log_probs_dev) && B * L > 0))
+    return fail(VASR_ERR_INVALID, "null argument");
+  return ctc_align_entry(logits_dev, row_lens_host, B, L, V, blank, log_probs, targets_host, target_lens_host, U_max,
+                         frame_labels_dev, frame_log_probs_dev, scores_dev, nullptr, stream);
+}
+
+int vasr_ctc_log_likelihood(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V,
+                            int blank, int log_probs, const int32_t* targets_host, const int32_t* target_lens_host,
+                            int64_t U_max, double* ll_dev, void* stream) {
+  if (!ll_dev) return fail(VASR_ERR_INVALID, "null argument");
+  return ctc_align_entry(logits_dev, row_lens_host, B, L, V, blank, log_probs, targets_host, target_lens_host, U_max,
+                         nullptr, nullptr, nullptr, ll_dev, stream);
+}
+
 // Per-utterance dims of a ragged batch -> k.ragbuf, k.rag.  `lens` (host) are samples (from_samples) or mel
 // frames; each utterance gets the dims make_dims would give it alone.
 static int upload_ragged(vasr_handle* h, const Dims& q, Work& k, const int32_t* lens, bool from_samples,
@@ -1688,6 +1796,35 @@ int vasr_transcribe_beam_host(vasr_handle* h, const float* pcm_host, const int32
   DeviceGuard dev_guard(h->device);
   return transcribe_beam_impl(h, nullptr, pcm_host, sample_lens_host, B, S, beam_width, lm, lm_weight, word_score,
                               tokens_host, lens_host, scores_host, h->own_stream);
+}
+
+// PCM -> forced alignment: transcribe_beam_impl's sequence (log-mel, model, the logits-writing CTC head, blank 0, a
+// ragged batch's token counts from RAG_L) with the Viterbi alignment in place of the search.
+int vasr_align(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B, int64_t S,
+               const int32_t* targets_host, const int32_t* target_lens_host, int64_t U_max, int32_t* frame_labels_dev,
+               float* frame_log_probs_dev, double* scores_dev, void* stream) {
+  RET(check_ready(h));
+  if (B < 0 || !pcm_dev || !frame_labels_dev || !frame_log_probs_dev || !scores_dev)
+    return fail(VASR_ERR_INVALID, "null argument");
+  if (S <= PAD) return fail(VASR_ERR_SHAPE, "reflect padding needs more than 200 samples (audio.py:100-101)");
+  const Dims q = make_dims(h, B, S, vasr_num_frames(S));
+  // every argument of the alignment is checked before any device work (sample_lens by upload_ragged below)
+  RET(align_check(nullptr, B, q.L, q.V, 0, targets_host, target_lens_host, U_max));
+  if (B == 0) return VASR_OK;
+  DeviceGuard dev_guard(h->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  CallOrder call_order(h, s);
+  Work k;
+  RET(ensure_workspace(h, q, true, true, &k, false));
+  if (sample_lens_host) RET(upload_ragged(h, q, k, sample_lens_host, true, s));
+  timing_begin(h, s);
+  RET(run_mel(h, q, k, pcm_dev, 1, s));
+  KL(launch_mel_finish(k.raw, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  RET(run_model(h, q, k, k.logits, nullptr, nullptr, nullptr, s));
+  RET(ctc_align_run(k.logits, nullptr, k.rag ? k.rag + RAG_L : nullptr, RAG_STRIDE, q.B, q.L, q.V, 0, 0, targets_host,
+                    target_lens_host, U_max, frame_labels_dev, frame_log_probs_dev, scores_dev, nullptr, s));
+  timing_end(h, s);
+  return VASR_OK;
 }
 
 int vasr_forward_ragged(vasr_handle* h, const float* mel_dev, const int32_t* frame_lens_host, int64_t B, int64_t T,

@@ -166,4 +166,20 @@ cudaError_t launch_beam_search(const float* logits, const float2* stats, const i
                                int32_t* trie, int64_t trie_cap, int32_t* out_tokens, int32_t* out_lens,
                                double* out_scores, cudaStream_t s, int64_t* launches);
 
+// ---------------------------------------------------------------- CTC forced alignment / log-likelihood
+// One CTA per utterance over the 2U+1 states of its target (align.cu).  ctc_align_layout gives the CTA size and the
+// states per thread for the longest target U (viterbi: E a multiple of 16, so a backpointer word has one writer);
+// ctc_align_smem the dynamic shared memory, with or without the scores (fp64, E * threads of them) in it.
+int64_t ctc_align_words(int64_t U);   // backpointer words per (utterance, frame): ceil((2U + 1) / 16)
+void ctc_align_layout(int64_t U, bool viterbi, int* threads, int* E);
+size_t ctc_align_smem(int threads, int E, bool delta_in_smem);
+// stats: launch_beam_rows' (max, log sum exp) per row, or NULL when the logits are log-probs.  lens as in
+// launch_beam_rows.  targets (B, U_max) with target_lens (B), device.  delta_g: NULL (scores in shared memory) or
+// (B, E * threads) doubles.  bp != NULL: Viterbi, with bp (B, L, words) scratch, out_labels / out_lp (B, L) and the
+// path score in out_score (B); bp == NULL: the log-likelihood in out_score.
+cudaError_t launch_ctc_align(const float* logits, const float2* stats, int64_t B, int64_t L, int V, int blank,
+                             const int32_t* lens, int lens_stride, const int32_t* targets, int64_t U_max,
+                             const int32_t* target_lens, int threads, int E, double* delta_g, uint32_t* bp,
+                             int64_t words, int32_t* out_labels, float* out_lp, double* out_score, cudaStream_t s);
+
 }  // namespace vasr

@@ -13,6 +13,7 @@ from .config import VelocityASRConfig, config_from_yaml, SCAN_MODES
 from .model import VELOCITYASR
 from .audio import compute_mel_spectrogram, SAMPLE_RATE, N_FFT, HOP_LENGTH, N_MELS
 from .decode import (ctc_greedy_decode, ctc_greedy_decode_with_timestamps, ctc_beam_search, DecodingResult, CTCDecoder,
+                  ctc_forced_align, ctc_log_likelihood, AlignmentResult,
                   create_default_vocabulary, frames_to_seconds, words_with_timestamps,
                   BLANK_TOKEN)
 from .lm import NGramLM, WordNGramLM
@@ -31,6 +32,7 @@ __all__ = [
     "__version__", "VELOCITYASR", "VelocityASRConfig", "config_from_yaml", "from_pretrained",
     "compute_mel_spectrogram", "SAMPLE_RATE", "N_FFT", "HOP_LENGTH", "N_MELS",
     "ctc_greedy_decode", "ctc_greedy_decode_with_timestamps", "ctc_beam_search", "DecodingResult", "CTCDecoder", "create_default_vocabulary", "BLANK_TOKEN",
+    "ctc_forced_align", "ctc_log_likelihood", "AlignmentResult",
     "NGramLM", "WordNGramLM",
     "frames_to_seconds", "words_with_timestamps",
     "selective_scan", "selective_scan_fn", "linear", "split_tf32", "MAMBA_AVAILABLE", "SCAN_MODES",

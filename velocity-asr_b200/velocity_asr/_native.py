@@ -57,6 +57,12 @@ _SIGNATURES = {
                                      c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe_beam_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_double,
                                           c_double, c_void_p, c_void_p, c_void_p]),
+    "vasr_ctc_align": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p,
+                               c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_ctc_log_likelihood": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p,
+                                        c_void_p, c_int64, c_void_p, c_void_p]),
+    "vasr_align": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                           c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "vasr_transcribe_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "vasr_transcribe_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),

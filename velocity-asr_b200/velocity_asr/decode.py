@@ -201,6 +201,126 @@ def ctc_beam_search(logits: torch.Tensor, beam_width: int = 10, blank_token: int
     return _beam_results(tokens, lens, scores)
 
 
+@dataclass
+class AlignmentResult:
+    """One utterance's CTC forced alignment (include/vasr.h, vasr_ctc_align, states the rule).
+    tokens: the target.  timestamps: per token its [start, end) frame range on the best path, or None when the
+    target cannot fit.  frame_labels (frames,) int32 / frame_log_probs (frames,) float32 host tensors over the
+    utterance's own frames: the label of the state the best path occupies at each frame (blank included) and the
+    log-prob there; -1 / 0 everywhere when there is no path.  score: the best path's log-prob, fp64 (-inf: no path)."""
+
+    tokens: List[int]
+    timestamps: Optional[List[Tuple[int, int]]]
+    frame_labels: torch.Tensor
+    frame_log_probs: torch.Tensor
+    score: float
+
+
+def _align_targets(targets, B: int, V: int, blank_token: int):
+    """Token-id lists -> (host int32 (B, max(U_max, 1)) targets, host int32 (B,) lengths, U_max).  Raises before any
+    device work: RuntimeError for a count that is not B, ValueError for a blank outside the vocabulary or an id
+    outside it or equal to the blank."""
+    import numpy as np
+    if len(targets) != B:
+        raise RuntimeError(f"expected {B} targets, got {len(targets)}")
+    if not 0 <= int(blank_token) < V:
+        raise ValueError(f"blank token {blank_token} is outside the vocabulary of {V}")
+    rows = [np.asarray(t, dtype=np.int64).reshape(-1) for t in targets]
+    U_max = max((r.size for r in rows), default=0)
+    tgt = np.zeros((B, max(U_max, 1)), np.int32)
+    for b, r in enumerate(rows):
+        if r.size and (r.min() < 0 or r.max() >= V or (r == blank_token).any()):
+            raise ValueError(f"target {b} has an id outside [0, {V}) or equal to the blank {blank_token}")
+        tgt[b, :r.size] = r
+    return torch.from_numpy(tgt), torch.tensor([r.size for r in rows], dtype=torch.int32), U_max
+
+
+def _alignment_results(tgt: torch.Tensor, tlens: torch.Tensor, labels: torch.Tensor, lps: torch.Tensor,
+                       scores: torch.Tensor, frames: List[int], blank_token: int) -> List[AlignmentResult]:
+    """The targets and lengths of _align_targets, (B, L) labels / log-probs and (B,) scores of vasr_ctc_align -> one
+    AlignmentResult per utterance."""
+    labels, lps, scores = labels.cpu(), lps.cpu(), scores.cpu().tolist()
+    tgt, tlens = tgt.numpy(), tlens.tolist()
+    # equal neighbouring targets are separated by a blank on every path, so a run of one label is one token; frames
+    # without a path or past an utterance's end are -1.  Runs are found for the whole batch at once.
+    x = labels.numpy()[:, :max(frames, default=0)]
+    tok = (x != blank_token) & (x >= 0)
+    start = tok.copy()
+    start[:, 1:] &= x[:, 1:] != x[:, :-1]
+    end = tok.copy()
+    end[:, :-1] &= x[:, :-1] != x[:, 1:]
+    starts = start.nonzero()[1].tolist()
+    ends = (end.nonzero()[1] + 1).tolist()
+    out, k = [], 0
+    for b, n in enumerate(frames):                       # a path has one run per token; no path has none
+        m = tlens[b] if scores[b] != -math.inf else 0
+        spans = list(zip(starts[k:k + m], ends[k:k + m])) if scores[b] != -math.inf else None
+        k += m
+        out.append(AlignmentResult(tokens=tgt[b, :tlens[b]].tolist(), timestamps=spans, frame_labels=labels[b, :n],
+                                   frame_log_probs=lps[b, :n], score=scores[b]))
+    return out
+
+
+def _align_inputs(logits: torch.Tensor, targets, lengths, blank_token: int):
+    """Checks and staging shared by ctc_forced_align and ctc_log_likelihood (all checks before device work)."""
+    if logits.dim() != 3:
+        raise RuntimeError(f"expected (batch, seq_len, vocab) logits, got {tuple(logits.shape)}")
+    B, L, V = logits.shape
+    tgt, tlens, U_max = _align_targets(targets, B, V, blank_token)
+    rows = None
+    if lengths is not None:
+        from .model import _lengths_tensor
+        rows = _lengths_tensor(lengths, B)
+        if B and (int(rows.min()) < 0 or int(rows.max()) > L):
+            raise RuntimeError(f"every length must be in [0, {L}], got {rows.tolist()}")
+    if logits.device.type != "cuda":       # host logits: staged to the current CUDA device (no CPU path exists)
+        logits = logits.to(_native.default_cuda_device())
+    frames = [L] * B if rows is None else rows.tolist()
+    return logits.to(torch.float32).contiguous(), rows, tgt, tlens, U_max, frames
+
+
+def ctc_forced_align(logits: torch.Tensor, targets: List[List[int]], lengths=None, blank_token: int = BLANK_TOKEN,
+                     log_probs: bool = False) -> List[AlignmentResult]:
+    """CTC forced alignment on the GPU: per utterance the best path of its target (a list of token ids) through its
+    logits (B, L, V), with each token's [start, end) frame range (the units of ctc_greedy_decode_with_timestamps).
+    Per-frame log-probs are log_softmax(logits) in fp32, as the beam search computes them, or the input itself with
+    log_probs=True; path scores are fp64.  Ties go to the earlier of stay / advance / skip and, at the end, to the
+    last-token state (include/vasr.h states the rule).  `lengths` (B frame counts in [0, L]): utterance b is aligned
+    over its first lengths[b] frames only, bit for bit as if alone.  Host logits are staged to the current CUDA
+    device.  A bad id raises ValueError, a bad length RuntimeError, both before any device work."""
+    lg, rows, tgt, tlens, U_max, frames = _align_inputs(logits, targets, lengths, blank_token)
+    B, L, V = lg.shape
+    if B == 0:
+        return []
+    labels = torch.empty(B, max(L, 1), dtype=torch.int32, device=lg.device)
+    lps = torch.empty(B, max(L, 1), dtype=torch.float32, device=lg.device)
+    scores = torch.empty(B, dtype=torch.float64, device=lg.device)
+    with torch.cuda.device(lg.device):
+        _native.check(_native.lib().vasr_ctc_align(
+            _native.ptr(lg), _native.ptr(rows), B, L, V, int(blank_token), int(bool(log_probs)), _native.ptr(tgt),
+            _native.ptr(tlens), U_max, _native.ptr(labels), _native.ptr(lps), _native.ptr(scores),
+            ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)))
+    return _alignment_results(tgt, tlens, labels, lps, scores, frames, int(blank_token))
+
+
+def ctc_log_likelihood(logits: torch.Tensor, targets: List[List[int]], lengths=None, blank_token: int = BLANK_TOKEN,
+                       log_probs: bool = False) -> torch.Tensor:
+    """log P(target | logits) under CTC, summed over every alignment, per utterance: (B,) float64, equal to
+    -torch.nn.functional.ctc_loss(..., reduction="none") (-inf when the target cannot fit).  Arguments, checks and
+    staging as ctc_forced_align; the result is on the logits' device."""
+    home = logits.device
+    lg, rows, tgt, tlens, U_max, _ = _align_inputs(logits, targets, lengths, blank_token)
+    B, L, V = lg.shape
+    ll = torch.empty(B, dtype=torch.float64, device=lg.device)
+    if B > 0:
+        with torch.cuda.device(lg.device):
+            _native.check(_native.lib().vasr_ctc_log_likelihood(
+                _native.ptr(lg), _native.ptr(rows), B, L, V, int(blank_token), int(bool(log_probs)),
+                _native.ptr(tgt), _native.ptr(tlens), U_max, _native.ptr(ll),
+                ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)))
+    return ll if home.type == "cuda" else ll.to(home)
+
+
 class CTCDecoder:
     """decode.py:220-328: vocabulary lookup around the greedy and beam-search decoders."""
 
@@ -228,6 +348,15 @@ class CTCDecoder:
                     r.text = self._tokens_to_text(r.tokens)
             return beams
         return [self._tokens_to_text(utt[0].tokens) if utt else "" for utt in beams]
+
+    def align(self, logits: torch.Tensor, texts: List[str], lengths=None) -> List[List[dict]]:
+        """Word timings of known transcripts: each text goes through text_to_tokens, is force-aligned to its logits
+        (ctc_forced_align) and assembled into words by words_with_timestamps ([{"word", "start", "end"}] in
+        seconds).  A transcript that cannot fit its frames gives []."""
+        res = ctc_forced_align(logits, [self.text_to_tokens(t) for t in texts], lengths=lengths,
+                               blank_token=self.blank_token)
+        return [words_with_timestamps(r.tokens, r.timestamps, self.vocabulary) if r.timestamps is not None else []
+                for r in res]
 
     def _tokens_to_text(self, tokens: List[int]) -> str:
         """decode.py:302-317: join, then turn the subword marker into spaces."""

@@ -322,6 +322,32 @@ class VELOCITYASR(nn.Module):
         return _beam_results(tokens, lens, scores)
 
     @torch.no_grad()
+    def align(self, audio: torch.Tensor, targets: List[List[int]], lengths=None):
+        """Fused PCM -> forced alignment: 16 kHz PCM (S,) | (B, S) and one target (token ids) per utterance -> per
+        utterance an AlignmentResult (ctc_forced_align's, blank 0), in one native call: log-mel, forward, the CTC head
+        writing logits, and the device Viterbi alignment.  `lengths` (B sample counts): a ragged batch as in
+        transcribe().  Utterance b gets bit for bit ctc_forced_align(forward(compute_mel_spectrogram(
+        audio[b, :lengths[b]]).unsqueeze(0)), targets[b:b+1])[0].  Host PCM is staged to the execution device."""
+        from .decode import _align_targets, _alignment_results
+        if audio.dim() == 1:
+            audio = audio.unsqueeze(0)
+        B, S = audio.shape
+        tgt, tlens, U_max = _align_targets(targets, B, self.config.vocab_size, 0)
+        slen = None if lengths is None else _lengths_tensor(lengths, B)
+        dev = self._exec_device(audio)
+        eng = self._engine(dev)
+        pcm = self._check_input(audio, "audio")
+        L = self.get_output_length(1 + S // 160)
+        labels = torch.empty(B, L, dtype=torch.int32, device=pcm.device)
+        lps = torch.empty(B, L, dtype=torch.float32, device=pcm.device)
+        scores = torch.empty(B, dtype=torch.float64, device=pcm.device)
+        _native.check(eng.lib.vasr_align(eng.handle, _native.ptr(pcm), _native.ptr(slen), B, S, _native.ptr(tgt),
+                                         _native.ptr(tlens), U_max, _native.ptr(labels), _native.ptr(lps),
+                                         _native.ptr(scores), _stream_ptr(pcm.device)))
+        frames = [L] * B if slen is None else [self.get_output_length(1 + n // 160) for n in slen.tolist()]
+        return _alignment_results(tgt, tlens, labels, lps, scores, frames, 0)
+
+    @torch.no_grad()
     def transcribe_batches(self, batches: Iterable[torch.Tensor], as_arrays: bool = False
                            ) -> Iterator[List[List[int]]]:
         """transcribe() over a stream of host batches, pipelined: while the kernels of batch i run,
