@@ -78,7 +78,9 @@ int64_t vasr_num_frames(int64_t samples);   /* 1 + samples / 160                
 int64_t vasr_num_tokens(int64_t frames);    /* (frames + 1) / 2                  */
 
 /* ---- compute_mel_spectrogram (velocity_asr/audio.py:65-143)
- * pcm (B, S) -> mel (B, T, n_mels), T = vasr_num_frames(S).  S must be > 200 (reflect pad). */
+ * pcm (B, S) -> mel (B, T, n_mels), T = vasr_num_frames(S).  S must be > 200 (reflect pad).  n_mels is the
+ * handle's mel_bins, any value in [1, 128]; the model's projections need 3 * mel_bins to be a multiple of 16,
+ * which vasr_commit_weights checks. */
 int vasr_log_mel(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S, int normalize,
                  float* mel_dev, void* stream);
 

@@ -201,11 +201,15 @@ def test_scan_golden(va, golden):
         assert torch.equal(ym, ys)
 
 
-@pytest.mark.parametrize("n,structured", [(64, True), (64, False), (32, True), (32, False), (16, True)])
+@pytest.mark.parametrize("n,structured,di", [
+    pytest.param(n, s, di, id=f"{n}-{s}" + (f"-di{di}" if di != 128 else ""))
+    for n, s, di in [(64, True, 128), (64, False, 128), (32, True, 128), (32, False, 128), (16, True, 128),
+                     (16, False, 128),                  # the unstructured-A kernels of N = 16
+                     (16, False, 64), (32, True, 192)]])  # 1-warp (N = 16) and 2-warp (N = 32) CTAs of the recurrence
 @pytest.mark.parametrize("mode", ["sequential", "parallel"])
-def test_scan_oracle(va, n, structured, mode):
+def test_scan_oracle(va, n, structured, di, mode):
     L = 203 if mode == "sequential" else 71            # not a multiple of the 32-step chunk / of 8
-    x, dt, A, Bm, Cm, D = FU.scan_inputs(2, L, 128, n, 100 + n, structured)
+    x, dt, A, Bm, Cm, D = FU.scan_inputs(2, L, di, n, 100 + n, structured)
     rs = np.random.RandomState(3)
     z = rs.standard_normal(x.shape).astype(np.float32)
     t = lambda a: torch.from_numpy(a).cuda()
@@ -215,6 +219,21 @@ def test_scan_oracle(va, n, structured, mode):
     assert rel(y, ref) < 1e-4
     y0 = va.selective_scan(t(x), t(dt), t(A), t(Bm), t(Cm), None, scan_mode=mode)   # no skip, no gate
     assert rel(y0, O.selective_scan(d(x), d(dt), d(A), d(Bm), d(Cm), None, mode)) < 1e-4
+    if n == 64 and structured and mode == "sequential":
+        # y rows 8-byte but not 16-byte aligned (ldy = Di + 2): the row-packed kernel declines them, and the
+        # structured recurrence kernel takes them (scan_seq_kernel<4, 4, 2, true>, which no other call reaches)
+        import ctypes
+        from velocity_asr import _native
+        B, Lx, Di = x.shape
+        xs, dts, As, Bs, Cs, Ds, zs = (t(a) for a in (x, dt, A, Bm, Cm, D, z))
+        ys = torch.full((B * Lx + 1, Di + 2), float("nan"), device="cuda")
+        _native.check(_native.lib().vasr_selective_scan(
+            _native.ptr(xs), Di, _native.ptr(dts), Di, _native.ptr(As), _native.ptr(Bs), n, _native.ptr(Cs), n,
+            _native.ptr(Ds), _native.ptr(zs), Di, _native.ptr(ys), Di + 2, B, Lx, Di, n, 0,
+            ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+        got = ys.cpu().numpy()
+        assert rel(got[:B * Lx, :Di].reshape(B, Lx, Di), ref) < 1e-4
+        assert np.isnan(got[:, Di:]).all() and np.isnan(got[B * Lx:]).all()
 
 
 def test_scan_scaled_state_extremes(va):

@@ -901,8 +901,8 @@ int vasr_create(const vasr_config* cfg, int device, vasr_handle** out) {
   if (c.scan_mode < 0 || c.scan_mode > 2) return fail(VASR_ERR_INVALID, "Unknown scan_mode");
   if (c.d_model <= 0 || c.d_model > 192 || (c.d_model % 16) != 0)
     return fail(VASR_ERR_UNSUPPORTED, "d_model must be a multiple of 16, at most 192");
-  if ((c.mel_bins * 3) % 16 != 0 || c.mel_bins * 8 > 1024)
-    return fail(VASR_ERR_UNSUPPORTED, "mel_bins must make 3*mel_bins a multiple of 16 (and be <= 128)");
+  // the front end takes any width up to 128; the temporal-binding projection's constraint is checked at commit
+  if (c.mel_bins < 1 || c.mel_bins > 128) return fail(VASR_ERR_UNSUPPORTED, "mel_bins must be in [1, 128]");
   auto n_ok = [](int n) { return n == 16 || n == 32 || n == 64; };
   if (!n_ok(c.ssm_state_dim) || !n_ok(c.global_ssm_state_dim))
     return fail(VASR_ERR_UNSUPPORTED, "ssm state_dim must be 16, 32 or 64");
@@ -991,6 +991,8 @@ int vasr_commit_weights(vasr_handle* h) {
   h->w_ctc_ln = h->b_ctc_ln = h->s_ctc = h->w_f3p = h->b_f3p = nullptr;
   const vasr_config& c = h->cfg;
   const int d = c.d_model, nm = c.mel_bins, att = c.attention_dim;
+  if ((nm * 3) % 16 != 0)
+    return fail(VASR_ERR_UNSUPPORTED, "mel_bins must make 3*mel_bins a multiple of 16 (the temporal-binding projection)");
   // temporal binding: conv.weight (d, mel, 3) -> (d, 3*mel) with k index = tap*mel + channel
   std::vector<float> cwv;
   RET(get_w(h, "temporal_binding.conv.weight", (int64_t)d * nm * 3, d, &cwv));
@@ -1118,7 +1120,7 @@ int vasr_log_mel(vasr_handle* h, const float* pcm_dev, int64_t B, int64_t S, int
   Work k;
   RET(ensure_workspace(h, q, true, false, &k));
   RET(run_mel(h, q, k, pcm_dev, normalize, s));
-  KL(launch_mel_finish(k.raw, nullptr, nullptr, mel_dev, q.B, q.T, q.n_mels, q.T, 0, s, &h->launches, nullptr,
+  KL(launch_mel_finish(k.raw, mel_dev, q.B, q.T, q.n_mels, q.T, 0, s, &h->launches, nullptr,
                        normalize ? k.part : nullptr));
   return VASR_OK;
 }
@@ -1134,7 +1136,7 @@ int vasr_forward(vasr_handle* h, const float* mel_dev, int64_t B, int64_t T, flo
   Work k;
   RET(ensure_workspace(h, q, false, false, &k));
   timing_begin(h, s);
-  KL(launch_mel_finish(mel_dev, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches));
+  KL(launch_mel_finish(mel_dev, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches));
   RET(run_model(h, q, k, logits_dev, feat_tb_dev, feat_local_dev, feat_fused_dev, s));
   timing_end(h, s);
   return VASR_OK;
@@ -1660,7 +1662,7 @@ static int transcribe_impl(vasr_handle* h, const float* pcm_dev, const float* pc
   timing_begin(h, s);
   if (host) RET(run_mel_from_host(h, q, k, pcm_host, s));
   else RET(run_mel(h, q, k, pcm_dev, 1, s));
-  KL(launch_mel_finish(k.raw, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  KL(launch_mel_finish(k.raw, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
   RET(run_model(h, q, k, from_parts ? nullptr : k.logits, nullptr, nullptr, nullptr, s));
   if (from_parts) {
     KL(launch_ctc_collapse(k.pred, tokens_dev, lens_dev, q.B, q.L, 0, 1, s, &h->launches, k.rag, k.amax_val, k.amax_idx,
@@ -1762,7 +1764,7 @@ static int transcribe_beam_impl(vasr_handle* h, const float* pcm_dev, const floa
   timing_begin(h, s);
   if (host) RET(run_mel_from_host(h, q, k, pcm_host, s));
   else RET(run_mel(h, q, k, pcm_dev, 1, s));
-  KL(launch_mel_finish(k.raw, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  KL(launch_mel_finish(k.raw, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
   RET(run_model(h, q, k, k.logits, nullptr, nullptr, nullptr, s));
   RET(beam_search(k.logits, nullptr, k.rag ? k.rag + RAG_L : nullptr, RAG_STRIDE, q.B, q.L, q.V, beam_width, 0, lm,
                   lm_weight, word_score, tok_dev, len_dev, sc_dev, s));
@@ -1819,7 +1821,7 @@ int vasr_align(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_
   if (sample_lens_host) RET(upload_ragged(h, q, k, sample_lens_host, true, s));
   timing_begin(h, s);
   RET(run_mel(h, q, k, pcm_dev, 1, s));
-  KL(launch_mel_finish(k.raw, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  KL(launch_mel_finish(k.raw, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
   RET(run_model(h, q, k, k.logits, nullptr, nullptr, nullptr, s));
   RET(ctc_align_run(k.logits, nullptr, k.rag ? k.rag + RAG_L : nullptr, RAG_STRIDE, q.B, q.L, q.V, 0, 0, targets_host,
                     target_lens_host, U_max, frame_labels_dev, frame_log_probs_dev, scores_dev, nullptr, s));
@@ -1839,7 +1841,7 @@ int vasr_forward_ragged(vasr_handle* h, const float* mel_dev, const int32_t* fra
   RET(ensure_workspace(h, q, false, false, &k));
   RET(upload_ragged(h, q, k, frame_lens_host, false, s));
   timing_begin(h, s);
-  KL(launch_mel_finish(mel_dev, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag));
+  KL(launch_mel_finish(mel_dev, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag));
   RET(run_model(h, q, k, logits_dev, nullptr, nullptr, nullptr, s));
   timing_end(h, s);
   return VASR_OK;
@@ -1875,7 +1877,7 @@ int vasr_calibrate(vasr_handle* h, const float* mel_dev, int64_t B, int64_t T, v
   const Dims q = make_dims(h, B, 0, T);
   Work k;
   RET(ensure_workspace(h, q, false, true, &k));
-  KL(launch_mel_finish(mel_dev, nullptr, nullptr, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches));
+  KL(launch_mel_finish(mel_dev, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches));
   h->calibrating = 1;
   const int r = run_model(h, q, k, k.logits, nullptr, nullptr, nullptr, s);
   h->calibrating = 0;
@@ -1934,7 +1936,7 @@ int vasr_quant_site(vasr_handle* h, const char* module, const float* x_dev, int6
     const Dims dm = make_dims(h, B, 0, R);
     Work k;
     RET(ensure_workspace(h, dm, false, false, &k));
-    KL(launch_mel_finish(x_dev, nullptr, nullptr, k.melpad, dm.B, dm.T, dm.n_mels, dm.Tp, 1, s, &h->launches));
+    KL(launch_mel_finish(x_dev, k.melpad, dm.B, dm.T, dm.n_mels, dm.Tp, 1, s, &h->launches));
     g.A = k.melpad; g.lda = 2 * dm.n_mels; g.rows_per_batch = dm.L; g.batch_stride = dm.Tp * dm.n_mels;
     g.W = h->tb_w; g.bias = h->tb_b; g.M = dm.M; g.K = 3 * dm.n_mels;
   } else {
@@ -2085,6 +2087,77 @@ int vasr_debug_gemm(vasr_debug_gemm_args* a) {
     const int f[8] = {v->family, v->tn, v->act, v->pe, v->resid, v->quant, v->wres, v->epi};
     memcpy(a->variant, f, sizeof(f));
   }
+  return VASR_OK;
+}
+
+/* debug hook (not in vasr.h): one call of a streaming kernel's launcher from kernels.cuh, for testing it on its own
+ * (tests/test_stream_kernels.py).  `kernel` names the launcher; each takes the fields its comment lists, as device
+ * pointers, and ignores the others:
+ *   layer_norm     x, ldx, y, ldy, gamma, beta, M, C
+ *   ln_dwconv      x, y (= u), gamma, beta, w, bias, B, L, C, k, run_len (0: the launcher's rule; the run length
+ *                  used comes back in run_len_used)
+ *   adaptive_pool  x, ldx, y, B, L, K, C, rag, f_in, f_out
+ *   attention      x (= q), ldx, kv, y (= o), ldy, B, L, K (= keys), heads, hd, rag
+ *   gate_mix       x (= f3), y, M, C
+ *   argmax         x (= logits), pred, M, V
+ *   ctc_collapse   pred, tokens, lens, B, L, blank, collapse, rag, and with amax_val: amax_idx, slots
+ *   ctc_runs       pred, tokens, starts, ends, lens, B, L, blank
+ *   minmax         x, ldx, M, c0, nc, mm, then set_qparams into q_scale / q_zp
+ * The call synchronises the stream; a launcher that declines its arguments gives VASR_ERR_UNSUPPORTED. */
+struct vasr_debug_kernel_args {
+  const char* kernel;
+  const float* x; int64_t ldx;
+  const float* kv;
+  float* y; int64_t ldy;
+  const float* gamma; const float* beta; const float* w; const float* bias;
+  int32_t* pred; int32_t* tokens; int32_t* lens; int32_t* starts; int32_t* ends;
+  const float* amax_val; const int32_t* amax_idx; int32_t slots;
+  float* mm; float* q_scale; float* q_zp; int32_t c0, nc;
+  const int32_t* rag; int32_t f_in, f_out;
+  int64_t B, L, M, K;
+  int32_t C, k, heads, hd, V, blank, collapse, run_len;
+  void* stream;
+  int32_t run_len_used;
+};
+
+int vasr_debug_kernel(vasr_debug_kernel_args* a) {
+  if (!a || !a->kernel) return fail(VASR_ERR_INVALID, "null argument");
+  const std::string n(a->kernel);
+  cudaStream_t s = static_cast<cudaStream_t>(a->stream);
+  cudaError_t e;
+  if (n == "layer_norm") {
+    e = launch_layer_norm(a->x, a->ldx, a->y, a->ldy, a->gamma, a->beta, a->M, a->C, s, nullptr);
+  } else if (n == "ln_dwconv") {
+    int used = 0;
+    e = launch_ln_dwconv(a->x, a->y, a->gamma, a->beta, a->w, a->bias, a->B, a->L, a->C, a->k, s, nullptr, a->run_len,
+                         &used);
+    a->run_len_used = used;
+  } else if (n == "adaptive_pool") {
+    e = launch_adaptive_pool(a->x, a->ldx, a->y, a->B, a->L, a->K, a->C, s, nullptr, a->rag, a->f_in, a->f_out);
+  } else if (n == "attention") {
+    e = launch_attention(a->x, a->ldx, a->kv, a->y, a->ldy, a->B, a->L, a->K, a->heads, a->hd, s, nullptr, a->rag);
+  } else if (n == "gate_mix") {
+    e = launch_gate_mix(a->x, a->y, a->M, a->C, s, nullptr);
+  } else if (n == "argmax") {
+    e = launch_argmax(a->x, a->pred, a->M, a->V, s, nullptr);
+  } else if (n == "ctc_collapse") {
+    e = launch_ctc_collapse(a->pred, a->tokens, a->lens, a->B, a->L, a->blank, a->collapse, s, nullptr, a->rag,
+                            a->amax_val, a->amax_idx, a->slots);
+  } else if (n == "ctc_runs") {
+    e = launch_ctc_runs(a->pred, a->tokens, a->starts, a->ends, a->lens, a->B, a->L, a->blank, s, nullptr);
+  } else if (n == "minmax") {
+    e = launch_minmax(a->x, a->ldx, a->M, a->c0, a->nc, a->mm, s, nullptr);
+    if (e == cudaSuccess) e = launch_set_qparams(a->mm, a->q_scale, a->q_zp, a->c0, a->nc, s, nullptr);
+  } else {
+    return fail(VASR_ERR_INVALID, "unknown kernel: " + n);
+  }
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(e == cudaErrorInvalidValue ? VASR_ERR_UNSUPPORTED : VASR_ERR_CUDA,
+                "launch_" + n + ": " + cudaGetErrorString(e));
+  }
+  const cudaError_t se = cudaStreamSynchronize(s);     // a fault of the kernel surfaces here
+  if (se != cudaSuccess) return fail(VASR_ERR_CUDA, "vasr_debug_kernel " + n + ": " + cudaGetErrorString(se));
   return VASR_OK;
 }
 

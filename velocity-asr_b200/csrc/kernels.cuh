@@ -76,10 +76,11 @@ cudaError_t launch_set_qparams(const float* mm, float* q_scale, float* q_zp, int
 cudaError_t launch_layer_norm(const float* x, int64_t ldx, float* y, int64_t ldy, const float* gamma,
                               const float* beta, int64_t M, int C, cudaStream_t s, int64_t* launches);
 // u = causal depthwise conv_k( LayerNorm(x) ) + bias on (B, L, C); zero left padding is
-// applied to the LayerNorm output (ssm.py:408-414).  w: (C, k) row-major.
+// applied to the LayerNorm output (ssm.py:408-414).  w: (C, k) row-major.  A warp takes run_len consecutive
+// tokens (0: the launcher's rule, which fills whole waves of the GPU); the run length used goes to *run_len_used.
 cudaError_t launch_ln_dwconv(const float* x, float* u, const float* gamma, const float* beta,
                              const float* w, const float* bias, int64_t B, int64_t L, int C, int k,
-                             cudaStream_t s, int64_t* launches);
+                             cudaStream_t s, int64_t* launches, int run_len = 0, int* run_len_used = nullptr);
 
 // ---------------------------------------------------------------- selective scan --------
 struct ScanArgs {
@@ -118,9 +119,9 @@ cudaError_t launch_mel_fft(const float* pcm, float* raw, double* part, int64_t B
                            const float* tw, cudaStream_t s, int64_t* launches, const int32_t* rag = nullptr);
 // out[b, t + front, j] = (raw[b,t,j] - mean[b,j]) * rstd[b,j]; out has frames_per_utt rows per utterance, rows
 // outside [front, front + T) are zeroed.  The statistics — per (b, j) the mean and 1 / (unbiased std + 1e-10) over
-// the T frames — come from `part` (the partials of launch_mel_fft, merged inside the kernel) when given, else from
-// mean / rstd; with neither the kernel is a plain copy.
-cudaError_t launch_mel_finish(const float* raw, const float* mean, const float* rstd, float* out, int64_t B,
+// the T frames — come from `part` (the partials of launch_mel_fft, merged inside the kernel); without it the kernel
+// is a plain copy.
+cudaError_t launch_mel_finish(const float* raw, float* out, int64_t B,
                               int64_t T, int n_mels, int64_t frames_per_utt, int front, cudaStream_t s,
                               int64_t* launches, const int32_t* rag = nullptr, const double* part = nullptr);
 

@@ -204,8 +204,6 @@ __global__ void __launch_bounds__(MEL_WARPS * 32) mel_fft_kernel(
 // was a separate one-CTA-per-utterance kernel running Chan's update block by block, two fp64 divisions inside a
 // dependent chain of 47 steps — 28 us on the critical path for 5,120 numbers.
 __global__ void __launch_bounds__(256) mel_finish_kernel(const float* __restrict__ raw,
-                                                         const float* __restrict__ mean,
-                                                         const float* __restrict__ rstd,
                                                          const double* __restrict__ part, int nblk,
                                                          float* __restrict__ out, int64_t T, int n_mels, int64_t fpu,
                                                          int front, const int32_t* __restrict__ rag, int per_cta) {
@@ -214,8 +212,8 @@ __global__ void __launch_bounds__(256) mel_finish_kernel(const float* __restrict
   pdl_wait();
   const int64_t b = blockIdx.y;
   const int64_t Tb = rag ? rag[b * RAG_STRIDE + RAG_T] : T;   // the partials keep the row stride nblk of the longest
-  const bool norm = part != nullptr || mean != nullptr;
-  if (part) {
+  const bool norm = part != nullptr;
+  if (norm) {
     // threads (j, g): mel bin j, every G-th block starting at g — the loads of a pass are in flight together, the
     // G partial sums of a bin are added in the order of g (the same bits in every CTA of the utterance)
     __shared__ double s_acc[256];
@@ -255,12 +253,6 @@ __global__ void __launch_bounds__(256) mel_finish_kernel(const float* __restrict
       const double sd = sqrt(m2t / (double)(Tb - 1));
       s_mean[j] = (float)mu;
       s_rstd[j] = (float)(1.0 / (sd + 1e-10));
-    }
-    __syncthreads();
-  } else if (mean) {
-    if (threadIdx.x < n_mels) {
-      s_mean[threadIdx.x] = mean[b * n_mels + threadIdx.x];
-      s_rstd[threadIdx.x] = rstd[b * n_mels + threadIdx.x];
     }
     __syncthreads();
   }
@@ -322,7 +314,7 @@ cudaError_t launch_mel_fft(const float* pcm, float* raw, double* part, int64_t B
   return e;
 }
 
-cudaError_t launch_mel_finish(const float* raw, const float* mean, const float* rstd, float* out, int64_t B,
+cudaError_t launch_mel_finish(const float* raw, float* out, int64_t B,
                               int64_t T, int n_mels, int64_t frames_per_utt, int front, cudaStream_t s,
                               int64_t* launches, const int32_t* rag, const double* part) {
   if (B <= 0) return cudaSuccess;
@@ -333,7 +325,7 @@ cudaError_t launch_mel_finish(const float* raw, const float* mean, const float* 
   int64_t per_cta = total / 128 > 8192 ? total / 128 : 8192;
   per_cta = (per_cta + 1023) / 1024 * 1024;
   dim3 grid((unsigned)((total + per_cta - 1) / per_cta), (unsigned)B);
-  const cudaError_t e = launch_k(mel_finish_kernel, grid, dim3(256), 0, s, raw, mean, rstd, part, (int)mel_fft_blocks(T), out,
+  const cudaError_t e = launch_k(mel_finish_kernel, grid, dim3(256), 0, s, raw, part, (int)mel_fft_blocks(T), out,
                                  T, n_mels, frames_per_utt, front, rag, (int)per_cta);
   if (launches) ++*launches;
   return e;

@@ -168,27 +168,31 @@ cudaError_t launch_layer_norm(const float* x, int64_t ldx, float* y, int64_t ldy
 
 cudaError_t launch_ln_dwconv(const float* x, float* u, const float* gamma, const float* beta, const float* w,
                              const float* bias, int64_t B, int64_t L, int C, int k, cudaStream_t s,
-                             int64_t* launches) {
+                             int64_t* launches, int run_len, int* run_len_used) {
   if (B <= 0 || L <= 0) return cudaSuccess;
-  if (C > 32 * DW_PER || k < 1 || k > MAXK || B > 65535) return cudaErrorInvalidValue;
+  if (C > 32 * DW_PER || k < 1 || k > MAXK || B > 65535 || run_len < 0) return cudaErrorInvalidValue;
   // Run length: a warp re-normalises the k - 1 rows before its run, so its cost is run + k - 1 rows, and the grid
   // runs in waves of (resident CTAs per SM) x SMs.  At config 2 runs of 16 tokens gave 768 CTAs for 592 resident
   // ones — a second wave of 176 — where runs of 21 give one wave of 576 (24 rows per warp instead of 2 x 19).
-  static int slots = 0;
-  if (slots == 0) {
-    int dev = 0, sms = 148, occ = 4;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ln_dwconv_kernel<4>, 128, 0) != cudaSuccess || occ < 1) occ = 4;
-    slots = occ * sms;
+  // A given run_len > 0 replaces the rule (the result does not depend on it: tests place run boundaries with it).
+  if (run_len == 0) {
+    static int slots = 0;
+    if (slots == 0) {
+      int dev = 0, sms = 148, occ = 4;
+      cudaGetDevice(&dev);
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ln_dwconv_kernel<4>, 128, 0) != cudaSuccess || occ < 1) occ = 4;
+      slots = occ * sms;
+    }
+    run_len = 16;
+    int64_t best = -1;
+    for (int r = 4; r <= 64; ++r) {
+      const int64_t ctas = B * (((L + r - 1) / r + 3) / 4);
+      const int64_t cost = ((ctas + slots - 1) / slots) * (r + k - 1);
+      if (best < 0 || cost < best) { best = cost; run_len = r; }
+    }
   }
-  int run_len = 16;
-  int64_t best = -1;
-  for (int r = 4; r <= 64; ++r) {
-    const int64_t ctas = B * (((L + r - 1) / r + 3) / 4);
-    const int64_t cost = ((ctas + slots - 1) / slots) * (r + k - 1);
-    if (best < 0 || cost < best) { best = cost; run_len = r; }
-  }
+  if (run_len_used) *run_len_used = run_len;
   const int64_t runs = (L + run_len - 1) / run_len;
   dim3 grid((unsigned)((runs + 3) / 4), (unsigned)B);
   cudaError_t e_launch = cudaSuccess;
