@@ -127,6 +127,42 @@ int vasr_ctc_greedy_timestamps(const float* logits_dev, int64_t B, int64_t L, in
                                int32_t* tokens_dev, int32_t* starts_dev, int32_t* ends_dev, int32_t* lens_dev,
                                void* stream);
 
+/* ---- the greedy path with timestamps and scores
+ * Utterance b has the frames t < len_b (row_lens[b], or L).  Per frame: a_t = argmax of x_t, ties to the lowest index
+ * (the argmax of vasr_transcribe, so the tokens are its tokens bit for bit), and the fp32 value
+ * lp_t = x_t[a_t] - log sum_v exp(x_t[v]).  Tokens, starts and ends are those of vasr_ctc_greedy_timestamps over the
+ * utterance's own frames: one token per run of equal non-blank a_t, [start, end) frames.  Blank frames belong to no
+ * token.  token_log_probs[k] = sum of lp_t over token k's run, fp64, in time order; log_probs[b] = sum of lp_t over all
+ * t < len_b, fp64, in time order: the log-prob of the greedy path, blank frames included.  len_b = 0 gives no tokens
+ * and log-prob 0.
+ * From logits (vasr_ctc_greedy_confidence), lp_t = (x_t[a_t] - max) - log sum exp(x_t - max) is the beam search's and
+ * vasr_ctc_align's fp32 table, so log_probs[b] equals vasr_ctc_align's score for the greedy tokens whenever the best
+ * path of that target is unique.  The fused calls on the fp32 model take lp_t = -log Z_t from the CTC head's epilogue,
+ * Z_t = sum over its 128-column halves p of (sum over p's columns of exp(x - max_p)) * exp(max_p - max), in fp32:
+ * within float rounding of the same value.
+ * Outputs: tokens / starts / ends (B, L) int32, -1 past lens[b]; token_log_probs (B, L) fp64, 0 past lens[b];
+ * lens (B) int32; log_probs (B) fp64.  Frames at or past len_b are never read (NaN padding does not matter).
+ * Contract: utterance b gets bit for bit what the same call gives for logits[b:b+1, :row_lens[b]] alone.
+ * row_lens_host: B frame counts, a HOST array copied before the call returns, or NULL.  Checks, all before any device
+ * call: VASR_ERR_INVALID for a null pointer or blank outside [0, V); VASR_ERR_SHAPE for a negative size or row_lens[b]
+ * outside [0, L].  Scratch, allocated stream-ordered per call: B * L * 16 bytes. */
+int vasr_ctc_greedy_confidence(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V,
+                               int blank, int32_t* tokens_dev, int32_t* starts_dev, int32_t* ends_dev,
+                               double* token_log_probs_dev, int32_t* lens_dev, double* log_probs_dev, void* stream);
+/* PCM -> the greedy path with timestamps and scores in one call: vasr_transcribe's sequence (a ragged batch by
+ * sample_lens_host, as vasr_transcribe_ragged), blank 0, L = vasr_num_tokens(vasr_num_frames(S)), outputs as
+ * vasr_ctc_greedy_confidence.  The fp32 model's CTC head writes no logits: its epilogue leaves the per-frame argmax
+ * partials and softmax normalisers.  The FakeQuantize model's head writes logits into the workspace and the
+ * vasr_ctc_greedy_confidence route follows.  Contract: utterance b gets bit for bit what the same call gives for
+ * that utterance alone; its tokens and lens equal vasr_transcribe[_ragged]'s.  The _host variant takes host PCM,
+ * returns host results and synchronises once at the end. */
+int vasr_transcribe_timestamps(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B,
+                               int64_t S, int32_t* tokens_dev, int32_t* starts_dev, int32_t* ends_dev,
+                               double* token_log_probs_dev, int32_t* lens_dev, double* log_probs_dev, void* stream);
+int vasr_transcribe_timestamps_host(vasr_handle* h, const float* pcm_host, const int32_t* sample_lens_host, int64_t B,
+                                    int64_t S, int32_t* tokens_host, int32_t* starts_host, int32_t* ends_host,
+                                    double* token_log_probs_host, int32_t* lens_host, double* log_probs_host);
+
 /* ---- ragged batches (the reference's collator pads with zeros and never masks, data.py:145-203, so an
  * utterance's transcript depends on its batch mates; these entry points take the true lengths instead)
  * pcm (B, S) holds utterance b in its first sample_lens[b] samples (200 < len <= S; the rest is ignored).

@@ -200,10 +200,16 @@ struct Work {
   int32_t *tok_stage, *len_stage;
   int32_t* ragbuf;       // B x RAG_STRIDE per-utterance dims of a ragged batch (kernels.cuh)
   const int32_t* rag;    // = ragbuf for a ragged call, NULL otherwise
+  // the greedy path with scores (vasr_transcribe_timestamps): the head's softmax normalisers next to amax_* (fp32
+  // model), or the row statistics of the logits (FakeQuantize model); per-frame fp32 log-probs
+  float* amax_sum;
+  float2* stats;
+  float* lp;
 };
 
 // Carves the arena; with measure_only it just computes the size.
-size_t carve(vasr_handle* h, const Dims& q, bool need_mel, bool need_logits, Work* w, bool need_stage = false) {
+size_t carve(vasr_handle* h, const Dims& q, bool need_mel, bool need_logits, Work* w, bool need_stage = false,
+             bool need_conf = false) {
   Arena a = h->ws;
   a.reset();
   Work t{};
@@ -244,13 +250,18 @@ size_t carve(vasr_handle* h, const Dims& q, bool need_mel, bool need_logits, Wor
     t.tok_stage = a.take<int32_t>(q.M);
     t.len_stage = a.take<int32_t>(q.B);
   }
+  if (need_conf) {
+    if (need_logits) t.stats = reinterpret_cast<float2*>(a.take<float>(q.M * 2));
+    else t.amax_sum = a.take<float>(q.M * argmax_slots(q.V));
+    t.lp = a.take<float>(q.M);
+  }
   if (w) *w = t;
   return a.used + 256;
 }
 
 int ensure_workspace(vasr_handle* h, const Dims& q, bool need_mel, bool need_logits, Work* w,
-                     bool need_stage = false) {
-  const size_t need = carve(h, q, need_mel, need_logits, nullptr, need_stage);
+                     bool need_stage = false, bool need_conf = false) {
+  const size_t need = carve(h, q, need_mel, need_logits, nullptr, need_stage, need_conf);
   if (need > h->ws.bytes) {
     CK(cudaDeviceSynchronize());
     if (h->ws.base) CK(cudaFree(h->ws.base));
@@ -261,7 +272,7 @@ int ensure_workspace(vasr_handle* h, const Dims& q, bool need_mel, bool need_log
     h->ws.base = static_cast<char*>(p);
     h->ws.bytes = need;
   }
-  carve(h, q, need_mel, need_logits, w, need_stage);
+  carve(h, q, need_mel, need_logits, w, need_stage, need_conf);
   return VASR_OK;
 }
 
@@ -714,13 +725,14 @@ int run_global_context(vasr_handle* h, const Dims& q, const Work& k, cudaStream_
 }
 
 // logits == NULL (fp32 model only): greedy decode, the head leaves per-frame argmax partials in k.amax_* instead
+// (and the softmax normalisers in k.amax_sum when the workspace has them)
 int run_ctc_head(vasr_handle* h, const Dims& q, const Work& k, const float* x, float* logits, cudaStream_t s) {
   if (h->w_ctc_ln) {         // fp32 model: the head's LayerNorm folded into its projection
     GemmArgs g;
     g.A = x; g.lda = q.d; g.W = h->w_ctc_ln; g.bias = h->b_ctc_ln; g.C = logits; g.ldc = q.V;
     g.M = q.M; g.N = q.V; g.K = q.d;
     g.ln_s = h->s_ctc; g.ln_stats = k.lnstat;
-    if (!logits) { g.amax_val = k.amax_val; g.amax_idx = k.amax_idx; }
+    if (!logits) { g.amax_val = k.amax_val; g.amax_idx = k.amax_idx; g.amax_sum = k.amax_sum; }
     return gemm(h, g, s);
   }
   if (!logits) return fail(VASR_ERR_STATE, "the FakeQuantize model decodes from its logits");
@@ -1240,6 +1252,67 @@ int vasr_ctc_greedy_timestamps(const float* logits_dev, int64_t B, int64_t L, in
   KL(launch_argmax(logits_dev, pred, B * L, (int)V, s, nullptr));
   KL(launch_ctc_runs(pred, tokens_dev, starts_dev, ends_dev, lens_dev, B, L, blank, s, nullptr));
   CK(cudaFreeAsync(pred, s));
+  return VASR_OK;
+}
+
+namespace {
+
+// Argument checks of the greedy-path-with-scores entry points (no device call), with vasr_ctc_align's error codes.
+int confidence_check(const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V, int blank, const void* tokens,
+                     const void* starts, const void* ends, const void* token_log_probs, const void* lens,
+                     const void* log_probs) {
+  if (B < 0 || L < 0) return fail(VASR_ERR_SHAPE, "negative size");
+  if (B > 0 && (!lens || !log_probs || (L > 0 && (!tokens || !starts || !ends || !token_log_probs))))
+    return fail(VASR_ERR_INVALID, "null argument");
+  if (V < 1 || blank < 0 || blank >= V) return fail(VASR_ERR_INVALID, "blank token outside the vocabulary");
+  if (row_lens_host)
+    for (int64_t b = 0; b < B; ++b)
+      if (row_lens_host[b] < 0 || row_lens_host[b] > L)
+        return fail(VASR_ERR_SHAPE, "ragged decode: every utterance needs between 0 and L frames (utterance " +
+                                        std::to_string(b) + " has " + std::to_string(row_lens_host[b]) + ")");
+  return VASR_OK;
+}
+
+// Scratch of the entry points below, released (stream-ordered) on every return, errors included.
+struct StreamScratch {
+  void* p[8] = {};
+  cudaStream_t s;
+  explicit StreamScratch(cudaStream_t st) : s(st) {}
+  ~StreamScratch() {
+    for (void* q : p)
+      if (q) cudaFreeAsync(q, s);
+  }
+};
+
+}  // namespace
+
+int vasr_ctc_greedy_confidence(const float* logits_dev, const int32_t* row_lens_host, int64_t B, int64_t L, int64_t V,
+                               int blank, int32_t* tokens_dev, int32_t* starts_dev, int32_t* ends_dev,
+                               double* token_log_probs_dev, int32_t* lens_dev, double* log_probs_dev, void* stream) {
+  if (!logits_dev && B * L > 0) return fail(VASR_ERR_INVALID, "null argument");
+  RET(confidence_check(row_lens_host, B, L, V, blank, tokens_dev, starts_dev, ends_dev, token_log_probs_dev, lens_dev,
+                       log_probs_dev));
+  if (B == 0) return VASR_OK;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int64_t M = B * L, M1 = M > 0 ? M : 1;
+  StreamScratch scratch(s);
+  const int32_t* rows = nullptr;
+  if (row_lens_host) {    // our own pageable copy: the caller may reuse its array as soon as the call returns
+    std::vector<int32_t> copy(row_lens_host, row_lens_host + B);
+    CK(cudaMallocAsync(&scratch.p[0], (size_t)B * sizeof(int32_t), s));
+    CK(cudaMemcpyAsync(scratch.p[0], copy.data(), (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    rows = static_cast<const int32_t*>(scratch.p[0]);
+  }
+  CK(cudaMallocAsync(&scratch.p[1], (size_t)M1 * sizeof(int32_t), s));
+  CK(cudaMallocAsync(&scratch.p[2], (size_t)M1 * sizeof(float2), s));
+  CK(cudaMallocAsync(&scratch.p[3], (size_t)M1 * sizeof(float), s));
+  int32_t* pred = static_cast<int32_t*>(scratch.p[1]);
+  float2* stats = static_cast<float2*>(scratch.p[2]);
+  KL(launch_argmax(logits_dev, pred, M, (int)V, s, nullptr));
+  KL(launch_beam_rows(logits_dev, stats, nullptr, M, (int)V, 0, blank, L, rows, 1, s, nullptr));
+  KL(launch_ctc_confidence(pred, static_cast<float*>(scratch.p[3]), logits_dev, stats, (int)V, nullptr, nullptr,
+                           nullptr, 0, tokens_dev, starts_dev, ends_dev, token_log_probs_dev, lens_dev, log_probs_dev,
+                           B, L, blank, rows, 1, s, nullptr));
   return VASR_OK;
 }
 
@@ -1829,6 +1902,89 @@ int vasr_align(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_
   return VASR_OK;
 }
 
+// PCM -> the greedy path with timestamps and scores: transcribe_impl's sequence, ragged or not.  The fp32 model's
+// CTC head runs its argmax epilogue with the softmax normalisers (EPI_ASUM) and writes no logits; the FakeQuantize
+// model's head writes logits, followed by argmax_kernel and beam_rows_kernel's statistics.  Host variant: results
+// come back through device scratch and the call synchronises once at the end.
+static int transcribe_timestamps_impl(vasr_handle* h, const float* pcm_dev, const float* pcm_host,
+                                      const int32_t* sample_lens, int64_t B, int64_t S, int32_t* tokens,
+                                      int32_t* starts, int32_t* ends, double* token_lps, int32_t* lens,
+                                      double* log_probs, cudaStream_t s) {
+  const bool host = pcm_host != nullptr;
+  const Dims q = make_dims(h, B, S, vasr_num_frames(S));
+  RET(confidence_check(nullptr, B, q.L, q.V, 0, tokens, starts, ends, token_lps, lens, log_probs));
+  if (B == 0) return VASR_OK;
+  CallOrder call_order(h, s);
+  Work k;
+  const bool from_parts = h->w_ctc_ln != nullptr;
+  RET(ensure_workspace(h, q, true, !from_parts, &k, host, true));
+  if (sample_lens) RET(upload_ragged(h, q, k, sample_lens, true, s));
+  int32_t *tok_d = tokens, *st_d = starts, *en_d = ends, *len_d = lens;
+  double *tlp_d = token_lps, *lp_d = log_probs;
+  StreamScratch stage(s);
+  if (host) {
+    CK(cudaMallocAsync(&stage.p[0], (size_t)3 * q.M * sizeof(int32_t), s));
+    CK(cudaMallocAsync(&stage.p[1], (size_t)q.M * sizeof(double), s));
+    CK(cudaMallocAsync(&stage.p[2], (size_t)B * sizeof(int32_t), s));
+    CK(cudaMallocAsync(&stage.p[3], (size_t)B * sizeof(double), s));
+    tok_d = static_cast<int32_t*>(stage.p[0]);
+    st_d = tok_d + q.M;
+    en_d = st_d + q.M;
+    tlp_d = static_cast<double*>(stage.p[1]);
+    len_d = static_cast<int32_t*>(stage.p[2]);
+    lp_d = static_cast<double*>(stage.p[3]);
+  }
+  const int32_t* rows = k.rag ? k.rag + RAG_L : nullptr;
+  timing_begin(h, s);
+  if (host) RET(run_mel_from_host(h, q, k, pcm_host, s));
+  else RET(run_mel(h, q, k, pcm_dev, 1, s));
+  KL(launch_mel_finish(k.raw, k.melpad, q.B, q.T, q.n_mels, q.Tp, 1, s, &h->launches, k.rag, k.part));
+  RET(run_model(h, q, k, from_parts ? nullptr : k.logits, nullptr, nullptr, nullptr, s));
+  if (from_parts) {
+    KL(launch_ctc_confidence(k.pred, k.lp, nullptr, nullptr, q.V, k.amax_val, k.amax_idx, k.amax_sum,
+                             argmax_slots(q.V), tok_d, st_d, en_d, tlp_d, len_d, lp_d, q.B, q.L, 0, rows, RAG_STRIDE,
+                             s, &h->launches));
+  } else {
+    KL(launch_argmax(k.logits, k.pred, q.M, q.V, s, &h->launches));
+    KL(launch_beam_rows(k.logits, k.stats, nullptr, q.M, q.V, 0, 0, q.L, rows, RAG_STRIDE, s, &h->launches));
+    KL(launch_ctc_confidence(k.pred, k.lp, k.logits, k.stats, q.V, nullptr, nullptr, nullptr, 0, tok_d, st_d, en_d,
+                             tlp_d, len_d, lp_d, q.B, q.L, 0, rows, RAG_STRIDE, s, &h->launches));
+  }
+  timing_end(h, s);
+  if (host) {
+    CK(cudaMemcpyAsync(tokens, tok_d, (size_t)q.M * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(starts, st_d, (size_t)q.M * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(ends, en_d, (size_t)q.M * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(token_lps, tlp_d, (size_t)q.M * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(lens, len_d, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(log_probs, lp_d, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+  }
+  return VASR_OK;
+}
+
+int vasr_transcribe_timestamps(vasr_handle* h, const float* pcm_dev, const int32_t* sample_lens_host, int64_t B,
+                               int64_t S, int32_t* tokens_dev, int32_t* starts_dev, int32_t* ends_dev,
+                               double* token_log_probs_dev, int32_t* lens_dev, double* log_probs_dev, void* stream) {
+  RET(check_ready(h));
+  if (B < 0 || (!pcm_dev && B > 0)) return fail(VASR_ERR_INVALID, "null argument");
+  if (S <= PAD) return fail(VASR_ERR_SHAPE, "reflect padding needs more than 200 samples (audio.py:100-101)");
+  DeviceGuard dev_guard(h->device);
+  return transcribe_timestamps_impl(h, pcm_dev, nullptr, sample_lens_host, B, S, tokens_dev, starts_dev, ends_dev,
+                                    token_log_probs_dev, lens_dev, log_probs_dev, static_cast<cudaStream_t>(stream));
+}
+
+int vasr_transcribe_timestamps_host(vasr_handle* h, const float* pcm_host, const int32_t* sample_lens_host, int64_t B,
+                                    int64_t S, int32_t* tokens_host, int32_t* starts_host, int32_t* ends_host,
+                                    double* token_log_probs_host, int32_t* lens_host, double* log_probs_host) {
+  RET(check_ready(h));
+  if (B <= 0 || !pcm_host) return fail(VASR_ERR_INVALID, "null argument");
+  if (S <= PAD) return fail(VASR_ERR_SHAPE, "reflect padding needs more than 200 samples (audio.py:100-101)");
+  DeviceGuard dev_guard(h->device);
+  return transcribe_timestamps_impl(h, nullptr, pcm_host, sample_lens_host, B, S, tokens_host, starts_host, ends_host,
+                                    token_log_probs_host, lens_host, log_probs_host, h->own_stream);
+}
+
 int vasr_forward_ragged(vasr_handle* h, const float* mel_dev, const int32_t* frame_lens_host, int64_t B, int64_t T,
                         float* logits_dev, void* stream) {
   RET(check_ready(h));
@@ -2012,7 +2168,7 @@ struct vasr_debug_gemm_args {
   int32_t variant[8];
 };
 
-int vasr_debug_gemm(vasr_debug_gemm_args* a) {
+static int debug_gemm(vasr_debug_gemm_args* a, float* amax_sum) {
   if (!a || !a->A || !a->W || (!a->C && !a->amax_val) || (a->ln_gamma && !a->ln_beta))
     return fail(VASR_ERR_INVALID, "null argument");
   const int64_t M = a->M, N = a->N, K = a->K;
@@ -2065,7 +2221,7 @@ int vasr_debug_gemm(vasr_debug_gemm_args* a) {
   g.act = a->act; g.act_from = a->act_from;
   g.resid = a->resid; g.ldr = a->ldr;
   if (lna) { g.ln_s = buf + o_s; g.ln_stats = buf + o_st; g.ln_eps = a->ln_eps; }
-  g.amax_val = a->amax_val; g.amax_idx = a->amax_idx;
+  g.amax_val = a->amax_val; g.amax_idx = a->amax_idx; g.amax_sum = amax_sum;
   g.gate = a->gate;
   g.pe_time = a->pe_time; g.pe_freq = a->pe_freq; g.pe_half = (int)a->pe_half; g.pe_rows = a->pe_rows;
   int sms = a->num_sms;
@@ -2087,6 +2243,48 @@ int vasr_debug_gemm(vasr_debug_gemm_args* a) {
     const int f[8] = {v->family, v->tn, v->act, v->pe, v->resid, v->quant, v->wres, v->epi};
     memcpy(a->variant, f, sizeof(f));
   }
+  return VASR_OK;
+}
+
+int vasr_debug_gemm(vasr_debug_gemm_args* a) { return debug_gemm(a, nullptr); }
+
+/* debug hook (not in vasr.h): vasr_debug_gemm with GemmArgs::amax_sum = amax_sum (device, slots x M): the argmax
+ * epilogue with the softmax normalisers (tests/test_greedy_confidence.py). */
+int vasr_debug_gemm_asum(vasr_debug_gemm_args* a, float* amax_sum) {
+  if (!amax_sum) return fail(VASR_ERR_INVALID, "null argument");
+  return debug_gemm(a, amax_sum);
+}
+
+/* debug hook (not in vasr.h): one launch_ctc_confidence call with every argument exposed, device pointers
+ * (tests/test_greedy_confidence.py).  amax_val != NULL: from the slot partials (amax_val / amax_idx / amax_sum,
+ * `slots`; pred is written); else from pred, logits (B*L, V) and stats ((max, log sum) per row).  lens_in (B entries
+ * at stride lens_stride) or NULL.  The call synchronises the stream. */
+struct vasr_debug_confidence_args {
+  const float* logits; const float* stats; int64_t V;
+  const float* amax_val; const int32_t* amax_idx; const float* amax_sum; int64_t slots;
+  int32_t* pred; float* lp;
+  int32_t* tokens; int32_t* starts; int32_t* ends; double* token_log_probs; int32_t* lens; double* log_probs;
+  const int32_t* lens_in; int64_t lens_stride;
+  int64_t B, L, blank;
+  void* stream;
+};
+
+int vasr_debug_confidence(vasr_debug_confidence_args* a) {
+  if (!a || !a->pred || !a->lp || !a->tokens || !a->starts || !a->ends || !a->token_log_probs || !a->lens ||
+      !a->log_probs)
+    return fail(VASR_ERR_INVALID, "null argument");
+  cudaStream_t s = static_cast<cudaStream_t>(a->stream);
+  const cudaError_t e = launch_ctc_confidence(
+      a->pred, a->lp, a->logits, reinterpret_cast<const float2*>(a->stats), (int)a->V, a->amax_val, a->amax_idx,
+      a->amax_sum, (int)a->slots, a->tokens, a->starts, a->ends, a->token_log_probs, a->lens, a->log_probs, a->B, a->L,
+      (int)a->blank, a->lens_in, (int)a->lens_stride, s, nullptr);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(e == cudaErrorInvalidValue ? VASR_ERR_UNSUPPORTED : VASR_ERR_CUDA,
+                std::string("launch_ctc_confidence: ") + cudaGetErrorString(e));
+  }
+  const cudaError_t se = cudaStreamSynchronize(s);
+  if (se != cudaSuccess) return fail(VASR_ERR_CUDA, std::string("vasr_debug_confidence: ") + cudaGetErrorString(se));
   return VASR_OK;
 }
 

@@ -234,9 +234,11 @@ struct TcArgs {
   // slot p = 2 * n_tile + half at amax_val / amax_idx[p * M + row]
   float* amax_val;
   int32_t* amax_idx;
+  // EPI_ASUM (with EPI_AMAX): also the slot's softmax normaliser sum exp(x - max) at amax_sum[p * M + row]
+  float* amax_sum;
 };
 // epilogue variants (template bit mask)
-constexpr int EPI_LNA = 1, EPI_AMAX = 2, EPI_GATE = 4;
+constexpr int EPI_LNA = 1, EPI_AMAX = 2, EPI_GATE = 4, EPI_ASUM = 8;
 // tile -> (m tile, n tile).  A persistent CTA takes tiles blockIdx.x, + gridDim.x, ...; with an n-tile
 // count that divides the grid every tile of a CTA would have the same n index, and the CTAs that own
 // the narrow last n-tile would do half the work of the others.  The n index is therefore rotated by
@@ -334,6 +336,7 @@ __device__ __forceinline__ void epilogue_loop(const TcArgs& g, uint8_t* stg, int
       // the folded LayerNorm) per column and leaves (max, first index of the max) of what it saw; the collapse
       // kernel takes the best of a row's partials in column order (ties -> lowest index, as torch.argmax).
       static_assert(!PE && !RESID && !QUANT && ACT == ACT_NONE, "argmax epilogue: plain projection only");
+      constexpr bool ASUM = (EPI & EPI_ASUM) != 0;
       const uint32_t r = mi0 + lane;
       const int64_t grow = (int64_t)batch * rpb + r;
       const int64_t slot = ((int64_t)nt * 2 + chalf) * g.M + grow;
@@ -342,7 +345,11 @@ __device__ __forceinline__ void epilogue_loop(const TcArgs& g, uint8_t* stg, int
       if (c_begin >= c_end) {
         tc_fence_before();
         arrive_empty(acc);
-        if (r < rpb) { g.amax_val[slot] = -INFINITY; g.amax_idx[slot] = -1; }
+        if (r < rpb) {
+          g.amax_val[slot] = -INFINITY;
+          g.amax_idx[slot] = -1;
+          if (ASUM) g.amax_sum[slot] = 0.f;
+        }
         continue;
       }
       uint32_t v0[32], v1[32];
@@ -385,7 +392,32 @@ __device__ __forceinline__ void epilogue_loop(const TcArgs& g, uint8_t* stg, int
           if (x1 > best) { best = x1; bi = (int)n + 1; }
           if (x2 > best) { best = x2; bi = (int)n + 2; }
           if (x3 > best) { best = x3; bi = (int)n + 3; }
+          if constexpr (ASUM) {    // the accumulators are dead once read: they keep x for the second pass
+            uint32_t* v = j == 0 ? v0 : v1;
+            v[4 * k4] = __float_as_uint(x0); v[4 * k4 + 1] = __float_as_uint(x1);
+            v[4 * k4 + 2] = __float_as_uint(x2); v[4 * k4 + 3] = __float_as_uint(x3);
+          }
         }
+      }
+      if constexpr (ASUM) {
+        // second pass over the same registers, now that the slot's max is known: sum exp(x - max) over the slot's
+        // columns below N, one accumulator per column of a group of four
+        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          if (c_begin + j >= c_end) break;
+          const uint32_t nb = ncol0 + (c_begin + j) * 32;
+          const uint32_t* v = j == 0 ? v0 : v1;
+#pragma unroll
+          for (int k4 = 0; k4 < 8; ++k4) {
+            if (nb + 4 * k4 >= (uint32_t)g.N) break;
+            s0 += expf(__uint_as_float(v[4 * k4]) - best);
+            s1 += expf(__uint_as_float(v[4 * k4 + 1]) - best);
+            s2 += expf(__uint_as_float(v[4 * k4 + 2]) - best);
+            s3 += expf(__uint_as_float(v[4 * k4 + 3]) - best);
+          }
+        }
+        if (r < rpb) g.amax_sum[slot] = (s0 + s1) + (s2 + s3);
       }
       if (r < rpb) { g.amax_val[slot] = best; g.amax_idx[slot] = bi; }
       continue;
@@ -1411,7 +1443,8 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   // out_proj / ffn2 -18 %, fusion -17 %.  Instantiated for the plain (+ residual), softplus and GELU epilogues.
   // VASR_TC_T192=2 restricts it to the N that would otherwise end in a 64-column tile.
   // epilogue variants: folded LayerNorm (ln_s), argmax partials instead of the output (amax_val), gated fusion
-  const bool lna = g.ln_s != nullptr, amax = g.amax_val != nullptr, gate = g.gate != 0;
+  const bool lna = g.ln_s != nullptr, amax = g.amax_val != nullptr, gate = g.gate != 0, asum = g.amax_sum != nullptr;
+  if (asum && !amax) return cudaErrorNotSupported;
   if (lna && (!pair || !g.ln_stats || g.K % TBK != 0 || g.K / TBK <= 4 || g.pe_time || g.resid || g.q_scale ||
               !(reinterpret_cast<uintptr_t>(g.ln_s) % 16 == 0) || !(g.act == ACT_NONE || (g.act == ACT_GELU && !amax))))
     return cudaErrorNotSupported;      // K / 32 > A slots: a row's entry is not rewritten before its tile's epilogue read it
@@ -1450,7 +1483,7 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   a.resid = g.resid; a.ldr = g.ldr;
   a.pe_time = g.pe_time; a.pe_freq = g.pe_freq; a.pe_half = g.pe_half;
   a.ln_s = g.ln_s; a.ln_stats = reinterpret_cast<float2*>(g.ln_stats); a.ln_eps = g.ln_eps;
-  a.amax_val = g.amax_val; a.amax_idx = g.amax_idx;
+  a.amax_val = g.amax_val; a.amax_idx = g.amax_idx; a.amax_sum = g.amax_sum;
   a.trace = g_trace;
   static const int rot_env = debug_env_int("VASR_TC_ROT", 1);
   a.rotate_n = rot_env;
@@ -1512,7 +1545,13 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
     return cudaSuccess;
   }
   if (lna || amax) {      // plain projection with a folded LayerNorm and / or the argmax epilogue (CTC head, q, k | v)
-    if (a.wres) {
+    if (asum && a.wres) {   // the argmax epilogue with the softmax normaliser
+      if (lna) VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_LNA | EPI_AMAX | EPI_ASUM);
+      else VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_AMAX | EPI_ASUM);
+    } else if (asum) {
+      if (lna) VASR_GO2(ACT_NONE, false, false, false, false, 128, EPI_LNA | EPI_AMAX | EPI_ASUM);
+      else VASR_GO2(ACT_NONE, false, false, false, false, 128, EPI_AMAX | EPI_ASUM);
+    } else if (a.wres) {
       if (lna && amax) VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_LNA | EPI_AMAX);
       else if (lna) VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_LNA);
       else VASR_GO2(ACT_NONE, false, false, false, true, 128, EPI_AMAX);

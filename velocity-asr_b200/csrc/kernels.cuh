@@ -39,6 +39,9 @@ struct GemmArgs {
   // the slot covers, at amax_val / amax_idx[p * M + m]; launch_ctc_collapse takes them (argmax_slots(N) slots)
   float* amax_val = nullptr;
   int32_t* amax_idx = nullptr;
+  // with amax_val: also sum over the slot's columns of exp(x - the slot's max) at amax_sum[p * M + m] (0 for a slot
+  // past N), the softmax normaliser launch_ctc_confidence merges.  NULL: the launch is exactly the one without it.
+  float* amax_sum = nullptr;
   // GatedFusion: W rows permuted by gate_perm_row (N = 3 C): C[m, c] = s l + (1 - s) t, s = sigmoid(gate), C is (M, C)
   int gate = 0;
   const float* pe_time = nullptr;  // (>= pe_rows, pe_half)
@@ -151,6 +154,16 @@ cudaError_t launch_ctc_collapse(int32_t* pred, int32_t* tokens, int32_t* lens, i
                                 int blank, int collapse, cudaStream_t s, int64_t* launches,
                                 const int32_t* rag = nullptr, const float* amax_val = nullptr,
                                 const int32_t* amax_idx = nullptr, int slots = 0);
+// The greedy path with per-token and per-utterance log-probs (include/vasr.h, vasr_ctc_greedy_confidence), one CTA
+// per utterance over its first lens_in[b * lens_stride] frames (NULL: L).  Frame predictions and fp32 log-probs
+// come from the CTC head's slot partials (amax_val / amax_idx / amax_sum, `slots` of them; pred is written) or,
+// with amax_val NULL, from pred (argmax) with the logits and launch_beam_rows' statistics.  pred / lp (B, L) are
+// scratch.  tokens / starts / ends / token_log_probs (B, L), -1 / 0 past lens[b]; log_probs (B) fp64.
+cudaError_t launch_ctc_confidence(int32_t* pred, float* lp, const float* logits, const float2* stats, int V,
+                                  const float* amax_val, const int32_t* amax_idx, const float* amax_sum, int slots,
+                                  int32_t* tokens, int32_t* starts, int32_t* ends, double* token_log_probs,
+                                  int32_t* lens, double* log_probs, int64_t B, int64_t L, int blank,
+                                  const int32_t* lens_in, int lens_stride, cudaStream_t s, int64_t* launches);
 
 // ---------------------------------------------------------------- CTC prefix beam search
 // per (utterance, frame) row: stats = (max, log sum exp(x - max)); top_tok (M, K) = the K best non-blank

@@ -12,7 +12,8 @@ __version__ = "2.0.0+b200"
 from .config import VelocityASRConfig, config_from_yaml, SCAN_MODES
 from .model import VELOCITYASR
 from .audio import compute_mel_spectrogram, SAMPLE_RATE, N_FFT, HOP_LENGTH, N_MELS
-from .decode import (ctc_greedy_decode, ctc_greedy_decode_with_timestamps, ctc_beam_search, DecodingResult, CTCDecoder,
+from .decode import (ctc_greedy_decode, ctc_greedy_decode_with_timestamps, ctc_beam_search,
+                  ctc_greedy_decode_with_confidence, GreedyResult, DecodingResult, CTCDecoder,
                   ctc_forced_align, ctc_log_likelihood, AlignmentResult,
                   create_default_vocabulary, frames_to_seconds, words_with_timestamps,
                   BLANK_TOKEN)
@@ -33,6 +34,7 @@ __all__ = [
     "compute_mel_spectrogram", "SAMPLE_RATE", "N_FFT", "HOP_LENGTH", "N_MELS",
     "ctc_greedy_decode", "ctc_greedy_decode_with_timestamps", "ctc_beam_search", "DecodingResult", "CTCDecoder", "create_default_vocabulary", "BLANK_TOKEN",
     "ctc_forced_align", "ctc_log_likelihood", "AlignmentResult",
+    "ctc_greedy_decode_with_confidence", "GreedyResult",
     "NGramLM", "WordNGramLM",
     "frames_to_seconds", "words_with_timestamps",
     "selective_scan", "selective_scan_fn", "linear", "split_tf32", "MAMBA_AVAILABLE", "SCAN_MODES",

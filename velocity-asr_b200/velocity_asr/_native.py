@@ -38,6 +38,12 @@ _SIGNATURES = {
     "vasr_ctc_greedy": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "vasr_ctc_greedy_timestamps": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p,
                                            c_void_p, c_void_p]),
+    "vasr_ctc_greedy_confidence": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_transcribe_timestamps": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vasr_transcribe_timestamps_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
+                                                c_void_p, c_void_p, c_void_p, c_void_p]),
     "vasr_ctc_beam_search": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                      c_void_p]),
     "vasr_lm_create_arpa": (c_int, [c_char_p, c_void_p, c_int64, c_int, c_int, POINTER(c_void_p)]),

@@ -66,34 +66,101 @@ def ctc_greedy_decode_with_timestamps(logits: torch.Tensor, blank_token: int = B
             for b, n in enumerate(lens)]
 
 
+@dataclass
+class GreedyResult:
+    """One utterance's greedy path with scores (include/vasr.h, vasr_ctc_greedy_confidence, states the rule).
+    tokens: the greedy transcript.  timestamps: per token its [start, end) frame range (the run of equal non-blank
+    argmax frames it was collapsed from).  token_log_probs: per token the sum of its frames' log-softmax values at the
+    argmax (fp64).  log_prob: that sum over every frame of the utterance, blank frames included: the log-prob of the
+    greedy path (fp64)."""
+
+    tokens: List[int]
+    timestamps: List[Tuple[int, int]]
+    token_log_probs: List[float]
+    log_prob: float
+
+
+def _greedy_results(buf, tlp, lens, lp) -> List[GreedyResult]:
+    """(3, B, L) tokens / starts / ends, (B, L) token log-probs, (B,) lens and (B,) log-probs -> GreedyResult list."""
+    buf, tlp, lens, lp = buf.cpu().numpy(), tlp.cpu().numpy(), lens.cpu().tolist(), lp.cpu().tolist()
+    return [GreedyResult(tokens=buf[0, b, :n].tolist(), timestamps=list(zip(buf[1, b, :n].tolist(), buf[2, b, :n].tolist())),
+                         token_log_probs=tlp[b, :n].tolist(), log_prob=lp[b]) for b, n in enumerate(lens)]
+
+
+def ctc_greedy_decode_with_confidence(logits: torch.Tensor, lengths=None, blank_token: int = BLANK_TOKEN
+                                      ) -> List[GreedyResult]:
+    """ctc_greedy_decode_with_timestamps plus scores: per utterance a GreedyResult with the same tokens and
+    timestamps, each token's log-prob (the sum over its frames of log_softmax(logits)[argmax], the fp32 table of the
+    beam search, added in fp64) and the greedy path's log-prob.  `lengths` (B frame counts in [0, L]): utterance b is
+    decoded over its first lengths[b] frames only, bit for bit as if alone.  Host logits are staged to the current
+    CUDA device.  A bad length raises RuntimeError, a blank outside the vocabulary ValueError, before device work."""
+    if logits.dim() != 3:
+        raise RuntimeError(f"expected (batch, seq_len, vocab) logits, got {tuple(logits.shape)}")
+    B, L, V = logits.shape
+    rows = None
+    if lengths is not None:
+        from .model import _lengths_tensor
+        rows = _lengths_tensor(lengths, B)
+        if B and (int(rows.min()) < 0 or int(rows.max()) > L):
+            raise RuntimeError(f"every length must be in [0, {L}], got {rows.tolist()}")
+    if not 0 <= int(blank_token) < V:
+        raise ValueError(f"blank token {blank_token} is outside the vocabulary of {V}")
+    if logits.device.type != "cuda":       # host logits: staged to the current CUDA device (no CPU decoder exists)
+        logits = logits.to(_native.default_cuda_device())
+    if B == 0:
+        return []
+    lg = logits.to(torch.float32).contiguous()
+    buf = torch.empty(3, B, max(L, 1), dtype=torch.int32, device=lg.device)
+    tlp = torch.empty(B, max(L, 1), dtype=torch.float64, device=lg.device)
+    lens = torch.empty(B, dtype=torch.int32, device=lg.device)
+    lp = torch.empty(B, dtype=torch.float64, device=lg.device)
+    with torch.cuda.device(lg.device):
+        _native.check(_native.lib().vasr_ctc_greedy_confidence(
+            _native.ptr(lg), _native.ptr(rows), B, L, V, int(blank_token), _native.ptr(buf[0]), _native.ptr(buf[1]),
+            _native.ptr(buf[2]), _native.ptr(tlp), _native.ptr(lens), _native.ptr(lp),
+            ctypes.c_void_p(torch.cuda.current_stream(lg.device).cuda_stream)))
+    return _greedy_results(buf, tlp, lens, lp)
+
+
 def frames_to_seconds(frame_idx: int, hop_length: int = 160, sample_rate: int = 16000) -> float:
     """Token index -> seconds (scripts/transcribe.py:42-45): one token spans two mel frames (stride-2 conv)."""
     return (frame_idx * 2 * hop_length) / sample_rate
 
 
-def words_with_timestamps(tokens: List[int], timestamps: List[Tuple[int, int]], vocabulary: List[str]
-                          ) -> List[dict]:
+def words_with_timestamps(tokens: List[int], timestamps: List[Tuple[int, int]], vocabulary: List[str],
+                          token_log_probs: Optional[List[float]] = None) -> List[dict]:
     """Word assembly of scripts/transcribe.py:80-126 on one utterance's output of
     ctc_greedy_decode_with_timestamps: characters accumulate into a word until a space / subword marker; a
     word starts at its first character's start frame and ends at the END frame of the separator that closed
-    it (the last word: at the end frame of the last token).  Returns [{"word", "start", "end"}] in seconds."""
+    it (the last word: at the end frame of the last token).  Returns [{"word", "start", "end"}] in seconds.
+    With token_log_probs (a GreedyResult's), each word also gets "confidence" = exp(sum of its characters' token
+    log-probs / sum of their frame counts): the geometric mean of its characters' frame probabilities, separators
+    excluded."""
     words, chars, start = [], [], None
+    lp_sum, n_frames = 0.0, 0
 
     def close(end_frame):
         text = "".join(chars).replace("▁", "")
         if text:
-            words.append({"word": text, "start": frames_to_seconds(start), "end": frames_to_seconds(end_frame)})
+            w = {"word": text, "start": frames_to_seconds(start), "end": frames_to_seconds(end_frame)}
+            if token_log_probs is not None:
+                w["confidence"] = math.exp(lp_sum / n_frames)
+            words.append(w)
 
-    for tok, (f0, f1) in zip(tokens, timestamps):
+    for i, (tok, (f0, f1)) in enumerate(zip(tokens, timestamps)):
         ch = vocabulary[tok] if 0 <= tok < len(vocabulary) else "<unk>"
         if ch in (" ", "▁"):
             if chars:
                 close(f1)
                 chars, start = [], None
+                lp_sum, n_frames = 0.0, 0
         else:
             if start is None:
                 start = f0
             chars.append(ch)
+            if token_log_probs is not None:
+                lp_sum += token_log_probs[i]
+                n_frames += f1 - f0
     if chars and timestamps:
         close(timestamps[-1][1])
     return words

@@ -322,6 +322,47 @@ class VELOCITYASR(nn.Module):
         return _beam_results(tokens, lens, scores)
 
     @torch.no_grad()
+    def transcribe_with_timestamps(self, audio: torch.Tensor, lengths=None):
+        """Fused PCM -> greedy transcript with token timestamps and scores: 16 kHz PCM (S,) | (B, S) -> per utterance
+        a GreedyResult (ctc_greedy_decode_with_confidence's, blank 0), in one native call that writes no logits for
+        the fp32 model: the CTC head's epilogue leaves each frame's argmax partials and softmax normalisers.  The
+        tokens are transcribe()'s, the timestamps those of ctc_greedy_decode_with_timestamps on forward()'s logits.
+        `lengths` (B sample counts): a ragged batch as in transcribe(); utterance b gets bit for bit what it gets
+        alone.  A CUDA tensor is consumed in place; a CPU tensor (pin it) is copied in inside the call."""
+        from .decode import _greedy_results
+        if audio.dim() == 1:
+            audio = audio.unsqueeze(0)
+        B, S = audio.shape
+        dev = self._exec_device(audio)
+        eng = self._engine(dev)
+        L = self.get_output_length(1 + S // 160)
+        slen = None if lengths is None else _lengths_tensor(lengths, B)
+        if audio.device.type == "cpu":
+            pcm = audio.to(torch.float32).contiguous()
+            cache = self.__dict__.setdefault("_pinned_ts_out", {})   # per shape, as transcribe() does
+            if (B, L) not in cache:
+                if len(cache) >= 8:
+                    cache.clear()
+                cache[(B, L)] = (torch.empty(3, B, L, dtype=torch.int32, pin_memory=True),
+                                 torch.empty(B, L, dtype=torch.float64, pin_memory=True),
+                                 torch.empty(B, dtype=torch.int32, pin_memory=True),
+                                 torch.empty(B, dtype=torch.float64, pin_memory=True))
+            buf, tlp, lens, lp = cache[(B, L)]
+            _native.check(eng.lib.vasr_transcribe_timestamps_host(
+                eng.handle, _native.ptr(pcm), _native.ptr(slen), B, S, _native.ptr(buf[0]), _native.ptr(buf[1]),
+                _native.ptr(buf[2]), _native.ptr(tlp), _native.ptr(lens), _native.ptr(lp)))
+        else:
+            pcm = self._check_input(audio, "audio")
+            buf = torch.empty(3, B, L, dtype=torch.int32, device=pcm.device)
+            tlp = torch.empty(B, L, dtype=torch.float64, device=pcm.device)
+            lens = torch.empty(B, dtype=torch.int32, device=pcm.device)
+            lp = torch.empty(B, dtype=torch.float64, device=pcm.device)
+            _native.check(eng.lib.vasr_transcribe_timestamps(
+                eng.handle, _native.ptr(pcm), _native.ptr(slen), B, S, _native.ptr(buf[0]), _native.ptr(buf[1]),
+                _native.ptr(buf[2]), _native.ptr(tlp), _native.ptr(lens), _native.ptr(lp), _stream_ptr(pcm.device)))
+        return _greedy_results(buf, tlp, lens, lp)
+
+    @torch.no_grad()
     def align(self, audio: torch.Tensor, targets: List[List[int]], lengths=None):
         """Fused PCM -> forced alignment: 16 kHz PCM (S,) | (B, S) and one target (token ids) per utterance -> per
         utterance an AlignmentResult (ctc_forced_align's, blank 0), in one native call: log-mel, forward, the CTC head
