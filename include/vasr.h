@@ -373,10 +373,11 @@ int vasr_quant_site(vasr_handle* h, const char* module, const float* x_dev, int6
 int vasr_linear(const float* x_dev, int64_t ldx, const float* w_dev, const float* bias_dev,
                 float* out_dev, int64_t ldo, int64_t M, int64_t K, int64_t N, int act, void* stream);
 
-/* Same contract through the tensor-core kernel (tcgen05 + TMEM + TMA, 3xTF32 split): the
- * kernel every token-sized projection of the model runs on.  K % 4 == 0, N % 4 == 0.
- * The kernel reads the weight as two TF32 matrices [hi | lo] (2*N*K floats) made by
- * vasr_split_tf32; pass w_split_dev = NULL to have the call split w_dev on the fly. */
+/* Same contract through the tensor-core kernel (tcgen05 + TMEM + TMA; fp32 operands split into a TF32 hi part
+ * and bf16 corrections): the kernel every token-sized projection of the model runs on.  K % 4 == 0, N % 4 == 0.
+ * The kernel reads the weight as 2*N*K 32-bit words made by vasr_split_tf32: the (N, K) matrix hi = rna_tf32(w),
+ * then an (N, K) matrix of bf16 pairs, bf16(hi) in the low and bf16(w - hi) in the high 16 bits of each word (both
+ * round-to-nearest-even); pass w_split_dev = NULL to have the call split w_dev on the fly. */
 int vasr_split_tf32(const float* w_dev, float* split_dev, int64_t numel, void* stream);
 /* resid_dev (M, N) with row stride ldr, or NULL: added after the activation (the residual adds of
  * ssm.py:418-425 are fused this way). */

@@ -98,7 +98,7 @@ struct vasr_handle {
   int64_t rag_pin_cap = 0;
   int rag_next = 0;
   float* q_mm = nullptr;     // (2) min / max scratch
-  // TF32 hi/lo split of each weight matrix the tensor-core kernel has used, keyed by the fp32 copy
+  // hi / bf16-pair split of each weight matrix the tensor-core kernel has used, keyed by the fp32 copy
   std::unordered_map<const float*, float*> w_split;
 
   std::vector<BlockW> local, global;
@@ -544,7 +544,7 @@ void free_weights(vasr_handle* h) {
 // one projection.  Every projection of the model runs on the tensor-core kernel whatever its row
 // count, so a row's result does not depend on how many utterances share the batch (the sharding
 // rule of DESIGN.md section 5); the CUDA-core kernel serves the DFT rows and unaligned views.
-// [W_hi | W_lo] for the tensor-core kernel: made on the device the first time a weight matrix is used
+// [W_hi | (W_hi, W_lo) bf16 pairs] for the tensor-core kernel: made on the device the first time a weight matrix is used
 // (warm-up), then reused until the weights are re-committed.
 int split_of(vasr_handle* h, const float* W, int64_t numel, cudaStream_t s, const float** out) {
   auto it = h->w_split.find(W);

@@ -1,27 +1,32 @@
 // gemm_tc.cu — tensor-core projection kernel for sm_100a: C = epi(A · Wᵀ) with fp32-grade accuracy.
 //
-// tcgen05.mma (kind::tf32) issued by one thread; the weight operand is staged in shared memory
+// tcgen05.mma (kind::tf32 and kind::f16) issued by one thread; the weight operand is staged in shared memory
 // by TMA (128-byte swizzle), the activation operand is fed from TENSOR MEMORY, accumulators live
 // in TMEM and are read back with tcgen05.ld for a fused, coalesced epilogue.
 //
 // Accuracy.  One TF32 pass carries ~1e-3 relative error, which flips ~0.3 % of the CTC argmaxes
-// (SURVEY.md section 7.3c).  Each fp32 operand is therefore split into hi + lo, both TF32 values
-// (hi = rna_tf32(x), lo = rna_tf32(x - hi); round-to-nearest keeps the residual error unbiased, which
-// matters for the 400-term DFT rows), and every k-step issues three MMAs,
-// A_lo·W_hi + A_hi·W_lo + A_hi·W_hi, accumulated in fp32 in TMEM (error ~2^-22 per product).
+// (SURVEY.md section 7.3c).  Each fp32 operand is therefore split into hi = rna_tf32(x) and lo = x - hi
+// (round-to-nearest keeps the residual error unbiased, which matters for the 400-term DFT rows).  The main
+// product A_hi·W_hi is one TF32 MMA; the two correction terms, about 2^-12 of it, need no TF32 and share one bf16
+// MMA: the "lo" word of an element holds a PAIR of bf16 values, (bf16(A_lo), bf16(A_hi)) for the activations and
+// (bf16(W_hi), bf16(W_lo)) for the weights, in its low and high half.  Read as a K-major bf16 operand twice as deep,
+// elements 2j and 2j+1 multiply A_lo·W_hi and A_hi·W_lo, so per 8-deep slice a kind::f16 MMA (K = 16, same 32 bytes,
+// same TMEM columns, same descriptor advance) adds both corrections and a kind::tf32 MMA the main product,
+// accumulated in fp32 in TMEM (error ~2^-20 per product; 2^-22 with three TF32 MMAs, at 12 instead of 8 MMAs per
+// k-block; DESIGN.md).
 //
 // Where the split happens (round-1 ncu: the first version split both tiles in shared memory and was
 // bound by shared-memory bandwidth — TMA write + converter read/write + 3x MMA operand reads):
 //   * weights are split ONCE (launch_split_tf32, cached per weight matrix by the engine) and TMA
 //     brings W_hi and W_lo tiles straight from L2;
 //   * the activation tile arrives as raw fp32; four converter warps read it once (one row per
-//     thread = one TMEM lane), split it in registers and tcgen05.st the hi and lo halves into TMEM,
+//     thread = one TMEM lane), split it in registers and tcgen05.st the hi and bf16-pair halves into TMEM,
 //     from where the MMA reads its A operand.  Shared memory then carries only the TMA writes, one
 //     read of A and the MMA reads of W.
 //
 // Structure (persistent, one CTA per SM, 14 warps):
 //   warp 0      TMA producer      : A (128 x 32 fp32), W_hi and W_lo (128 x 32) per stage, 4 stages
-//   warp 1      MMA issuer        : 12 tcgen05.mma per stage; tcgen05.commit frees the stage
+//   warp 1      MMA issuer        : 8 tcgen05.mma per stage (4 bf16-pair + 4 TF32); tcgen05.commit frees the stage
 //   warps 2-5   converters        : smem A row -> hi/lo -> TMEM (64 columns per stage)
 //   warps 6-13  epilogue          : TMEM -> registers -> per-warp smem transpose -> bias / act /
 //                                   pos-enc / residual on 128-byte row segments -> coalesced stores
@@ -57,10 +62,11 @@ static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB of dynamic shared memory
 constexpr int B_FULL = 0, B_CONV = STAGES, B_EMPTY = 2 * STAGES, B_TFULL = 3 * STAGES, B_TEMPTY = 3 * STAGES + 2;
 constexpr int N_BARS = 3 * STAGES + 4;
 
-// instruction descriptor (cute::UMMA::InstrDescriptor): c=F32 [4,6), a=TF32 [7,10), b=TF32 [10,13),
-// K-major A and B, n_dim = N>>3 at [17,23), m_dim = M>>4 at [24,29)
-__device__ __forceinline__ uint32_t make_idesc(uint32_t n) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((n >> 3) << 17) | ((uint32_t)(TBM >> 4) << 24);
+// instruction descriptor (cute::UMMA::InstrDescriptor): c_format [4,6) = F32, a_format [7,10) and b_format [10,13)
+// = FMT_TF32 (kind::tf32) or FMT_BF16 (kind::f16), K-major A and B, n_dim = N>>3 at [17,23), m_dim = M>>4 at [24,29)
+constexpr uint32_t FMT_BF16 = 1, FMT_TF32 = 2;
+__device__ __forceinline__ uint32_t make_idesc(uint32_t fmt, uint32_t m, uint32_t n) {
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -132,6 +138,17 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, u
       ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] · B[smem]ᵀ : 128 x N x 16, bf16 inputs, fp32 accumulate.  16 bf16 are 32 bytes, as 8 tf32 are:
+// the same TMEM columns and the same descriptor advance as one umma_tf32_ts
+__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
@@ -188,6 +205,18 @@ __device__ __forceinline__ uint32_t rna_tf32(float x) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
   return r;
+}
+// (bf16(hi) << 16) | bf16(lo), both round-to-nearest-even: bf16 element 2j + 1 and element 2j of a K-major operand
+__device__ __forceinline__ uint32_t pack_bf16x2(float hi, float lo) {
+  uint32_t r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+// An activation x as the converters leave it in TMEM: the TF32 word rna_tf32(x) and the bf16 pair
+// (bf16(x - hi), bf16(hi)) in elements (2j, 2j + 1); split_tf32_kernel leaves W as rna_tf32(w) and (bf16(hi), bf16(w - hi))
+__device__ __forceinline__ void split_act(float x, uint32_t& hi, uint32_t& lo) {
+  hi = rna_tf32(x);
+  lo = pack_bf16x2(__uint_as_float(hi), x - __uint_as_float(hi));
 }
 
 template <int ACT>
@@ -861,7 +890,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       // columns of this tile that exist, rounded up to the MMA's N granularity (16)
       int64_t nrem = g.N - (int64_t)nt * TBN;
       const uint32_t n_mma = nrem >= TBN ? (uint32_t)TBN : (uint32_t)((nrem + 15) & ~15LL);
-      const uint32_t idesc = make_idesc(n_mma);
+      const uint32_t idesc = make_idesc(FMT_TF32, TBM, n_mma), idesc_bf = make_idesc(FMT_BF16, TBM, n_mma);
       const uint32_t acc = (uint32_t)(it & 1);
       mbar_wait(BAR(B_TEMPTY + acc), (uint32_t)((it >> 1) & 1) ^ 1);
       tc_fence_after();
@@ -877,9 +906,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (elect_one()) {
 #pragma unroll
           for (int k4 = 0; k4 < TBK / 8; ++k4) {
-            const uint64_t adv = (uint64_t)(k4 * 2);   // 8 tf32 = 32 bytes = 2 x 16-byte units
-            umma_tf32_ts(tmem_d, a_lo + 8 * k4, db_hi + adv, idesc, (kb | k4) != 0);
-            umma_tf32_ts(tmem_d, a_hi + 8 * k4, db_lo + adv, idesc, 1);
+            const uint64_t adv = (uint64_t)(k4 * 2);   // 8 tf32 = 16 bf16 = 32 bytes = 2 x 16-byte units
+            umma_bf16_ts(tmem_d, a_lo + 8 * k4, db_lo + adv, idesc_bf, (kb | k4) != 0);   // A_lo·W_hi + A_hi·W_lo
             umma_tf32_ts(tmem_d, a_hi + 8 * k4, db_hi + adv, idesc, 1);
           }
           umma_commit(BAR(B_EMPTY + stage));
@@ -910,10 +938,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
           const float4 v = *reinterpret_cast<const float4*>(arow + ((c ^ (row & 7)) << 4));
-          hi[4 * c + 0] = rna_tf32(v.x); lo[4 * c + 0] = rna_tf32(v.x - __uint_as_float(hi[4 * c + 0]));
-          hi[4 * c + 1] = rna_tf32(v.y); lo[4 * c + 1] = rna_tf32(v.y - __uint_as_float(hi[4 * c + 1]));
-          hi[4 * c + 2] = rna_tf32(v.z); lo[4 * c + 2] = rna_tf32(v.z - __uint_as_float(hi[4 * c + 2]));
-          hi[4 * c + 3] = rna_tf32(v.w); lo[4 * c + 3] = rna_tf32(v.w - __uint_as_float(hi[4 * c + 3]));
+          split_act(v.x, hi[4 * c + 0], lo[4 * c + 0]);
+          split_act(v.y, hi[4 * c + 1], lo[4 * c + 1]);
+          split_act(v.z, hi[4 * c + 2], lo[4 * c + 2]);
+          split_act(v.w, hi[4 * c + 3], lo[4 * c + 3]);
         }
         // the TMEM slot of this stage was last read by MMAs whose commit released `empty[stage]`,
         // which the producer waited on before the TMA that completed `full[stage]`
@@ -1039,6 +1067,15 @@ __device__ __forceinline__ void umma_tf32_ts_pair(uint32_t tmem_d, uint32_t tmem
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::2.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_bf16_ts_pair(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc,
+                                                  uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
       ::"r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -1174,7 +1211,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA only) =====================
     // Measured (tools/gemm_trace.py, K = 192, N-tile 128): the k-blocks of a tile complete 1300 / 600 / 1050 /
-    // 790 / 800 / 790 clocks apart with the epilogue switched off (ideal 768 each: 12 MMAs x 64), i.e. ~800
+    // 790 / 800 / 790 clocks apart with the epilogue switched off (ideal 768 each: 12 TF32 MMAs x 64 then), i.e. ~800
     // clocks are lost at the start of every tile, and the epilogue's staging + store phase costs the third and
     // fourth k-block another ~1200.  Ruled out as the cause of the tile-start loss: an accumulator-switch
     // penalty of the tensor pipe (tools/probes/mma_probe.cu: none), the epilogue's tcgen05.ld traffic
@@ -1192,7 +1229,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         const int64_t nrem = g.N - (int64_t)nt * TBN;
         const uint32_t n_mma = nrem >= TBN ? (uint32_t)TBN : (uint32_t)((nrem + 15) & ~15LL);
         // M = 256 across the pair
-        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((n_mma >> 3) << 17) | ((256u >> 4) << 24);
+        const uint32_t idesc = make_idesc(FMT_TF32, 2 * TBM, n_mma), idesc_bf = make_idesc(FMT_BF16, 2 * TBM, n_mma);
         const uint32_t acc = it & 1u;
         mbar_wait_cluster(BAR(PB_TEMPTY + acc), ((it >> 1) & 1u) ^ 1u);
         tc_fence_after();
@@ -1212,8 +1249,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 #pragma unroll
             for (int k4 = 0; k4 < TBK / 8; ++k4) {
               const uint64_t adv = (uint64_t)(k4 * 2);
-              umma_tf32_ts_pair(tmem_d, a_lo + 8 * k4, db_hi + adv, idesc, (kb | k4) != 0);
-              umma_tf32_ts_pair(tmem_d, a_hi + 8 * k4, db_lo + adv, idesc, 1);
+              umma_bf16_ts_pair(tmem_d, a_lo + 8 * k4, db_lo + adv, idesc_bf, (kb | k4) != 0);
               umma_tf32_ts_pair(tmem_d, a_hi + 8 * k4, db_hi + adv, idesc, 1);
             }
             umma_commit_pair(BAR(PB_EMPTY + stage));
@@ -1270,10 +1306,10 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             unpack2(a, v.x, v.y);
             unpack2(b, v.z, v.w);
           }
-          hi[4 * c + 0] = rna_tf32(v.x); lo[4 * c + 0] = rna_tf32(v.x - __uint_as_float(hi[4 * c + 0]));
-          hi[4 * c + 1] = rna_tf32(v.y); lo[4 * c + 1] = rna_tf32(v.y - __uint_as_float(hi[4 * c + 1]));
-          hi[4 * c + 2] = rna_tf32(v.z); lo[4 * c + 2] = rna_tf32(v.z - __uint_as_float(hi[4 * c + 2]));
-          hi[4 * c + 3] = rna_tf32(v.w); lo[4 * c + 3] = rna_tf32(v.w - __uint_as_float(hi[4 * c + 3]));
+          split_act(v.x, hi[4 * c + 0], lo[4 * c + 0]);
+          split_act(v.y, hi[4 * c + 1], lo[4 * c + 1]);
+          split_act(v.z, hi[4 * c + 2], lo[4 * c + 2]);
+          split_act(v.w, hi[4 * c + 3], lo[4 * c + 3]);
         }
         if constexpr ((EPI & EPI_LNA) != 0) {
           if (kb == nkb - 1) {
@@ -1345,7 +1381,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   }
 }
 
-// w (n) -> hl[0..n) = rna_tf32(w), hl[n..2n) = rna_tf32(w - hi)
+// w (n) -> hl[0..n) = rna_tf32(w); word n + i of hl = (bf16(w - hi) << 16) | bf16(hi).  The pair keeps the 4-byte
+// element of the TF32 half, so both halves share one K-major tensor map layout (row stride 4 K bytes)
 __global__ void __launch_bounds__(256) split_tf32_kernel(const float* __restrict__ w, float* __restrict__ hl,
                                                          int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
@@ -1353,7 +1390,7 @@ __global__ void __launch_bounds__(256) split_tf32_kernel(const float* __restrict
   const float x = w[i];
   const float h = __uint_as_float(rna_tf32(x));
   hl[i] = h;
-  hl[n + i] = __uint_as_float(rna_tf32(x - h));
+  reinterpret_cast<uint32_t*>(hl)[n + i] = pack_bf16x2(x - h, h);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -1419,7 +1456,7 @@ cudaError_t launch_split_tf32(const float* w, float* hl, int64_t n, cudaStream_t
 }
 
 // Returns cudaErrorNotSupported when the tensor maps cannot be encoded (the caller then uses the
-// CUDA-core kernel); any other error is a real launch failure.  g.W_split = [W_hi | W_lo].
+// CUDA-core kernel); any other error is a real launch failure.  g.W_split = [W_hi | (W_hi, W_lo) bf16 pairs].
 cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64_t* launches) {
   if (g.M <= 0 || g.N <= 0) return cudaSuccess;
   if (!g.W_split || !gemm_tc_supported(g)) return cudaErrorNotSupported;
@@ -1437,9 +1474,10 @@ cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64
   // 192-column tiles (PairCfg<192>).  VASR_TC_T192=0 turns them off.
   static const int t192_env = debug_env_int("VASR_TC_T192", 1);
   // Rule: 192-column tiles whenever N tiles into them without a tile narrower than 128 columns (192, 384, 512 =
-  // 192 + 192 + 128, 576, 768, ...): a 128-column tile is exactly as fast as the control path (768 clocks of MMAs
-  // per k-block against ~770), a 192-column one has 50 % more tensor work per k-block and per A tile loaded and
-  // converted.  Measured against the 128-column tiling (W resident where it applied): in_proj -9 %, x / dt -6 %,
+  // 192 + 192 + 128, 576, 768, ...): a 128-column tile is no faster than the control path (512 clocks of MMAs per
+  // k-block, 768 with three TF32 MMAs per slice, against ~770), a 192-column one has 50 % more tensor work per k-block
+  // and per A tile loaded and converted.  Measured against the 128-column tiling with three TF32 MMAs per slice (W
+  // resident where it applied): in_proj -9 %, x / dt -6 %,
   // out_proj / ffn2 -18 %, fusion -17 %.  Instantiated for the plain (+ residual), softplus and GELU epilogues.
   // VASR_TC_T192=2 restricts it to the N that would otherwise end in a 64-column tile.
   // epilogue variants: folded LayerNorm (ln_s), argmax partials instead of the output (amax_val), gated fusion

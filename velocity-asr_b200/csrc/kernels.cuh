@@ -19,7 +19,7 @@ struct GemmArgs {
   int64_t rows_per_batch = 0;  // 0 -> plain matrix
   int64_t batch_stride = 0;
   const float* W = nullptr;
-  const float* W_split = nullptr;  // [rna_tf32(W) | rna_tf32(W - hi)], 2*N*K floats (launch_split_tf32); tensor-core path only
+  const float* W_split = nullptr;  // [rna_tf32(W) | bf16 pairs (hi, W - hi)], 2*N*K words (launch_split_tf32); tensor-core path only
   const float* bias = nullptr;
   const float* q_scale = nullptr;  // (N) device; with q_zp: output FakeQuantize per column (scale <= 0: none)
   const float* q_zp = nullptr;
@@ -52,7 +52,7 @@ struct GemmArgs {
 // CUDA-core fp32 kernel behind vasr_linear (a general-purpose op for views the tensor-core kernel cannot take,
 // e.g. K % 4 != 0); the model's launch sequence never uses it.
 cudaError_t launch_gemm(const GemmArgs& g, cudaStream_t s, int64_t* launches);
-// tcgen05 / TMEM / TMA path with 3xTF32 split accumulation (gemm_tc.cu); needs g.W_split.  Returns
+// tcgen05 / TMEM / TMA path with split accumulation, TF32 hi·hi + bf16 corrections (gemm_tc.cu); needs g.W_split.  Returns
 // cudaErrorNotSupported when a tensor map cannot be encoded for this view.
 cudaError_t launch_gemm_tc(const GemmArgs& g, int num_sms, cudaStream_t s, int64_t* launches);
 // The template instantiation a launch_gemm_tc call launched (family 1 = gemm_tc_kernel, 2 = gemm_tc2_kernel; tn, act,
@@ -61,7 +61,7 @@ struct TcVariant {
   int family, tn, act, pe, resid, quant, wres, epi;
 };
 extern thread_local const TcVariant* tc_last_variant;
-// hl[0..n) = rna_tf32(w), hl[n..2n) = rna_tf32(w - hl[0..n)): the weight operand of launch_gemm_tc.
+// hl[0..n) = rna_tf32(w), word n + i of hl = (bf16(w - hi) << 16) | bf16(hi): the weight operand of launch_gemm_tc.
 cudaError_t launch_split_tf32(const float* w, float* hl, int64_t n, cudaStream_t s);
 extern long long* g_trace;   // debug: device buffer (5 x 128 clock64 slots) CTA 0 of the projection kernel writes
 

@@ -66,8 +66,9 @@ _ACT = {None: 0, "none": 0, "gelu": 1, "softplus": 2, "sigmoid": 3}
 
 
 def split_tf32(weight: torch.Tensor) -> torch.Tensor:
-    """(N, K) fp32 weight -> (2, N, K): [rna_tf32(w), rna_tf32(w - hi)], the operand format of the
-    tensor-core projection kernel.  Done once per weight matrix."""
+    """(N, K) fp32 weight -> (2, N, K) 32-bit words, the operand format of the tensor-core projection kernel:
+    [0] = rna_tf32(w) (float32), [1] = a pair of bf16 per word, bf16(hi) in the low and bf16(w - hi) in the high
+    16 bits (view as int32 / uint32 to read them).  Done once per weight matrix."""
     if weight.device.type != "cuda":
         raise RuntimeError("split_tf32 runs on CUDA only (no CPU fallback)")
     weight = _f32c(weight)
@@ -83,7 +84,7 @@ def linear(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor] =
            weight_split: Optional[torch.Tensor] = None, residual: Optional[torch.Tensor] = None,
            out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """F.linear (+ optional activation) on (..., K) rows.  tensor_cores=False: CUDA-core fp32 kernel
-    (K % 16 == 0); True: tcgen05 3xTF32 kernel (K % 4 == 0, N % 4 == 0) — the one the model's
+    (K % 16 == 0); True: tcgen05 kernel, TF32 hi·hi + one bf16 MMA for both corrections (K % 4 == 0, N % 4 == 0) — the one the model's
     token-sized projections run on; weight_split = split_tf32(weight) skips the per-call split; residual
     (same shape as the result, tensor_cores only) is added after the activation; out = preallocated result."""
     if x.device.type != "cuda":
