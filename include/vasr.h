@@ -108,7 +108,8 @@ int vasr_ctc_head(vasr_handle* h, const float* x_dev, int64_t B, int64_t L, floa
  * (ssm.py:134-337).  x, dt: (B, L, Di) with row strides ldx, lddt; Bm, Cm: (B, L, N) with row
  * strides ldb, ldc; A: (N), D: (Di) or NULL (no skip term); z: (B, L, Di) stride ldz or NULL
  * (when given, y is multiplied by silu(z), ssm.py:129); y: (B, L, Di) stride ldy.
- * N in {16, 32, 64}.  All device pointers.  No handle: the operator is stateless. */
+ * N in {16, 32, 64} (else VASR_ERR_UNSUPPORTED); Di a positive multiple of 64 (else VASR_ERR_SHAPE).  All device
+ * pointers.  No handle: the operator is stateless. */
 int vasr_selective_scan(const float* x, int64_t ldx, const float* dt, int64_t lddt, const float* A,
                         const float* Bm, int64_t ldb, const float* Cm, int64_t ldc, const float* D,
                         const float* z, int64_t ldz, float* y, int64_t ldy, int64_t B, int64_t L,

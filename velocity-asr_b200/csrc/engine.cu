@@ -1201,6 +1201,13 @@ int vasr_ctc_head(vasr_handle* h, const float* x_dev, int64_t B, int64_t L, floa
   return VASR_OK;
 }
 
+// A[n] = -(n + 1) to a relative 2e-6: the scan's structured-A kernels take it (powers of exp(-dt), scan.cu)
+static int scan_structured_a(const float* ah, int64_t N) {
+  for (int64_t n = 0; n < N; ++n)
+    if (fabsf(ah[n] + (float)(n + 1)) > 2e-6f * (float)(n + 1)) return 0;
+  return 1;
+}
+
 int vasr_selective_scan(const float* x, int64_t ldx, const float* dt, int64_t lddt, const float* A, const float* Bm,
                         int64_t ldb, const float* Cm, int64_t ldc, const float* D, const float* z, int64_t ldz,
                         float* y, int64_t ldy, int64_t B, int64_t L, int64_t Di, int64_t N, int scan_mode,
@@ -1208,11 +1215,10 @@ int vasr_selective_scan(const float* x, int64_t ldx, const float* dt, int64_t ld
   if (!x || !dt || !A || !Bm || !Cm || !y) return fail(VASR_ERR_INVALID, "null argument");
   if (scan_mode < 0 || scan_mode > 2) return fail(VASR_ERR_INVALID, "Unknown scan_mode");
   if (N != 16 && N != 32 && N != 64) return fail(VASR_ERR_UNSUPPORTED, "state_dim must be 16, 32 or 64");
+  if (Di <= 0 || Di % 64 != 0) return fail(VASR_ERR_SHAPE, "d_inner must be a positive multiple of 64");
   float ah[64];
   CK(cudaMemcpy(ah, A, (size_t)N * sizeof(float), cudaMemcpyDeviceToHost));
-  int structured = 1;
-  for (int n = 0; n < N; ++n)
-    if (fabsf(ah[n] + (float)(n + 1)) > 2e-6f * (float)(n + 1)) structured = 0;
+  const int structured = scan_structured_a(ah, N);
   ScanArgs a;
   a.x = x; a.ldx = ldx; a.dt = dt; a.lddt = lddt; a.z = z; a.ldz = ldz;
   a.Bm = Bm; a.ldb = ldb; a.Cm = Cm; a.ldc = ldc; a.A = A; a.D = D; a.y = y; a.ldy = ldy;
@@ -2247,6 +2253,64 @@ static int debug_gemm(vasr_debug_gemm_args* a, float* amax_sum) {
 }
 
 int vasr_debug_gemm(vasr_debug_gemm_args* a) { return debug_gemm(a, nullptr); }
+
+/* debug hook (not in vasr.h): one launch_selective_scan call with every ScanArgs field exposed and the kernel chosen
+ * by hand, for testing the scan one instantiation at a time (tests/test_scan_variants.py).  Device arrays; Di, N and
+ * the strides are not checked beyond what the launcher checks (it declines what its kernels cannot take).
+ * structured: -1 = detect as vasr_selective_scan does, 0 = the generic kernels whatever A is, 1 = the structured ones
+ * (refused unless A is structured).  num_sms: the SM count the launch rule plans for (0 = the device's; more than the
+ * device has is refused), the only way the time split's slot count is set, so that every split is one the rule makes
+ * on some GPU.  rp / split: ScanOverride (kernels.cuh), except that split may only be 0 (rule) or -1 (never).  On
+ * return `variant` holds the launched instantiation (ScanVariant field order, family 0 = declined), and the call has
+ * synchronised the stream.  A declined launch returns VASR_ERR_UNSUPPORTED. */
+struct vasr_debug_scan_args {
+  const float* x; int64_t ldx; const float* dt; int64_t lddt; const float* z; int64_t ldz;
+  const float* Bm; int64_t ldb; const float* Cm; int64_t ldc; const float* A; const float* D;
+  float* y; int64_t ldy;
+  int64_t B, L; int32_t Di, N, parallel_quirk, structured, num_sms, rp, split;
+  void* stream;
+  int32_t variant[6];
+};
+
+int vasr_debug_scan(vasr_debug_scan_args* d) {
+  if (!d || !d->x || !d->dt || !d->A || !d->Bm || !d->Cm || !d->y) return fail(VASR_ERR_INVALID, "null argument");
+  if (d->N != 16 && d->N != 32 && d->N != 64) return fail(VASR_ERR_UNSUPPORTED, "state_dim must be 16, 32 or 64");
+  if (d->structured < -1 || d->structured > 1 || d->rp < -1 || d->rp > 2 || d->split < -1 || d->split > 0)
+    return fail(VASR_ERR_INVALID, "bad override");
+  memset(d->variant, 0, sizeof(d->variant));
+  cudaStream_t s = static_cast<cudaStream_t>(d->stream);
+  int dev = 0, dev_sms = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, dev));
+  if (d->num_sms < 0 || d->num_sms > dev_sms) return fail(VASR_ERR_INVALID, "num_sms above the device's SM count");
+  float ah[64];
+  CK(cudaMemcpy(ah, d->A, (size_t)d->N * sizeof(float), cudaMemcpyDeviceToHost));
+  const int detected = scan_structured_a(ah, d->N);
+  if (d->structured == 1 && !detected) return fail(VASR_ERR_INVALID, "A is not structured");
+  ScanArgs a;
+  a.x = d->x; a.ldx = d->ldx; a.dt = d->dt; a.lddt = d->lddt; a.z = d->z; a.ldz = d->ldz;
+  a.Bm = d->Bm; a.ldb = d->ldb; a.Cm = d->Cm; a.ldc = d->ldc; a.A = d->A; a.D = d->D; a.y = d->y; a.ldy = d->ldy;
+  a.B = d->B; a.L = d->L; a.Di = d->Di; a.N = d->N;
+  a.parallel_quirk = d->parallel_quirk != 0;
+  a.structured_a = d->structured < 0 ? detected : d->structured;
+  a.num_sms = d->num_sms > 0 ? d->num_sms : dev_sms;
+  ScanOverride ov;
+  ov.rp = d->rp;
+  ov.split = d->split;
+  scan_last_variant = nullptr;
+  const cudaError_t e = launch_selective_scan(a, s, nullptr, &ov);
+  const ScanVariant* v = scan_last_variant;
+  if (e == cudaErrorInvalidValue && !v) (void)cudaGetLastError();
+  const cudaError_t se = cudaStreamSynchronize(s);     // a fault of the kernel surfaces here
+  if (e == cudaErrorInvalidValue && !v) return fail(VASR_ERR_UNSUPPORTED, "launch_selective_scan declines this call");
+  if (e != cudaSuccess) return fail(VASR_ERR_CUDA, std::string("launch_selective_scan: ") + cudaGetErrorString(e));
+  if (se != cudaSuccess) return fail(VASR_ERR_CUDA, std::string("vasr_debug_scan: ") + cudaGetErrorString(se));
+  if (v) {
+    const int f[6] = {v->family, v->lpr, v->warps, v->rpl, v->structured, v->slots};
+    memcpy(d->variant, f, sizeof(f));
+  }
+  return VASR_OK;
+}
 
 /* debug hook (not in vasr.h): vasr_debug_gemm with GemmArgs::amax_sum = amax_sum (device, slots x M): the argmax
  * epilogue with the softmax normalisers (tests/test_greedy_confidence.py). */

@@ -101,7 +101,24 @@ struct ScanArgs {
   int structured_a = 0;       // A[n] == -(n+1): powers of exp(-dt) instead of one exp per state
   int num_sms = 0;            // 0 -> 148
 };
-cudaError_t launch_selective_scan(const ScanArgs& a, cudaStream_t s, int64_t* launches);
+// Host-side choice of the kernel for one call (NULL: the defaults, which are the rule below unless the debug build's
+// VASR_SCAN_OLD / VASR_SCAN_RP / VASR_SCAN_SPLIT say otherwise).  rp: 0 = the rule, 1 / 2 = scan_rp_kernel with that
+// many row pairs per lane, -1 = never (scan_seq_kernel on a shape scan_rp_kernel would take); a shape the problem does
+// not fit is declined (cudaErrorInvalidValue) when `ov` asks for it, ignored when the environment does.  split: 0 =
+// the rule, -1 = never, n > 0 = n slots (VASR_SCAN_SPLIT=n; capped by the resident CTAs, as the rule is).
+struct ScanOverride {
+  int rp = 0;
+  int split = 0;
+};
+cudaError_t launch_selective_scan(const ScanArgs& a, cudaStream_t s, int64_t* launches,
+                                  const ScanOverride* ov = nullptr);
+// The instantiation a launch_selective_scan call launched.  family 1 = scan_quirk_kernel<lpr, structured>, 2 =
+// scan_seq_kernel<lpr, warps, rpl, structured>, 3 = scan_rp_kernel<RP = lpr, warps, OCC = rpl> (structured A only);
+// slots = the time split's slot count, 0 when unsplit.  Each launch site sets it; the scan tests read it.
+struct ScanVariant {
+  int family, lpr, warps, rpl, structured, slots;
+};
+extern thread_local const ScanVariant* scan_last_variant;
 
 // ---------------------------------------------------------------- ragged batches ---------
 // A batch whose utterances have different lengths is stored padded to the longest; `rag` (device,

@@ -151,7 +151,9 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_quirk_kernel(ScanArgs a) {
   // Narrow mode (structured A): the states decay in order, state n at the rate (n + 1).  Once exp(A[n] S) is an
   // exact zero for every n >= NN in every row of the CTA, and the next power of two has passed (so that their
   // hP is zero, not just frozen), only the NN slowest states are left: the CTA continues with two states per lane
-  // instead of eight.  With dt ~ 0.7 that is after the first 16 tokens.
+  // instead of eight.  With dt ~ 0.7 that is after the first 16 tokens.  What it drops is exact zeros, but its powers
+  // (r^(2j+1) directly) and the order of its state sum differ from the wide mode's: unlike phases 2 and 3, the switch
+  // can move the last bit of a row's state sum (DESIGN.md).
   int64_t t_narrow = L;
   bool narrow_known = !STRUCT || N <= NN;
 
@@ -1382,8 +1384,11 @@ bool rp_takes(const ScanArgs& a) {
   return true;
 }
 
+// where each launch site records what it launched (scan_last_variant)
+thread_local ScanVariant scan_variant_rec;
+
 template <int RP, int OCC>
-cudaError_t launch_rp_cfg(const ScanArgs& a, int sms, cudaStream_t s) {
+cudaError_t launch_rp_cfg(const ScanArgs& a, int sms, int split_ov, cudaStream_t s) {
   using C = RpCfg<RP, OCC>;
   auto kernel = scan_rp_kernel<RP, RP_WARPS, OCC>;
   // A split launch asks for at least SPLIT_SMEM bytes of shared memory, more than a third of an SM's: never more
@@ -1416,10 +1421,9 @@ cudaError_t launch_rp_cfg(const ScanArgs& a, int sms, cudaStream_t s) {
   int64_t slots = (int64_t)(occ < 2 ? occ : 2) * sms;
   if (slots > RP_MAX_SLOTS) slots = RP_MAX_SLOTS;
   if (slots > total) slots = total;
-  static const int split_env = debug_env_int("VASR_SCAN_SPLIT", -1);     // -1: rule below; 0: never; n > 0: n slots
-  if (split_env > 0 && split_env <= (int64_t)occ * sms && split_env <= RP_MAX_SLOTS) slots = split_env;
+  if (split_ov > 0 && split_ov <= (int64_t)occ * sms && split_ov <= RP_MAX_SLOTS) slots = split_ov;
   bool split = occ > 0 && n_chains > slots && slots >= 1 && n_chains % slots != 0;
-  if (split_env == 0) split = false;
+  if (split_ov < 0) split = false;
   if (split) {
     RpScratch* sc = nullptr;
     e = rp_scratch(s, &sc);
@@ -1432,19 +1436,18 @@ cudaError_t launch_rp_cfg(const ScanArgs& a, int sms, cudaStream_t s) {
     grid = (unsigned)slots;
     smem = SPLIT_SMEM;
   }
+  scan_variant_rec = {3, RP, RP_WARPS, OCC, 1, sa.n_slots};
+  scan_last_variant = &scan_variant_rec;
   return launch_k(kernel, dim3(grid), dim3(C::THREADS), smem, s, a, sa);
 }
 
-cudaError_t launch_rp(const ScanArgs& a, cudaStream_t s) {
+cudaError_t launch_rp(const ScanArgs& a, const ScanOverride& ov, cudaStream_t s) {
   const int sms = a.num_sms > 0 ? a.num_sms : 148;
-  static const int rp_env = debug_env_int("VASR_SCAN_RP", 0);            // 1 / 2: force the CTA shape
   // 128-row CTAs once they fill two slots per SM (batch 128: 0.42 ms against 0.47 for 64-row CTAs and 0.50 for
   // scan_seq_kernel); below that the 64-row shape keeps more chains in flight (batch 64: 0.252 against 0.308)
-  const bool wide = rp_env ? rp_env == 2 : a.B * (a.Di / RpCfg<2>::ROWS) >= 2 * sms;
-  if (a.Di % RpCfg<2>::ROWS == 0 && wide) {
-    return launch_rp_cfg<2, 2>(a, sms, s);
-  }
-  return launch_rp_cfg<1, 3>(a, sms, s);
+  const bool wide = a.Di % RpCfg<2>::ROWS == 0 && (ov.rp ? ov.rp == 2 : a.B * (a.Di / RpCfg<2>::ROWS) >= 2 * sms);
+  if (wide) return launch_rp_cfg<2, 2>(a, sms, ov.split, s);
+  return launch_rp_cfg<1, 3>(a, sms, ov.split, s);
 }
 
 template <int LPR, int WARPS, int RPL>
@@ -1454,19 +1457,25 @@ cudaError_t launch_seq(const ScanArgs& a, cudaStream_t s) {
   constexpr size_t SMEM = (size_t)3 * TCH * (2 * N + 3 * ROWS) * sizeof(float);
   dim3 grid((unsigned)(a.Di / ROWS), (unsigned)a.B);
   cudaError_t e = cudaSuccess;
-  auto go = [&](auto kernel) {
+  auto go = [&](auto kernel, bool st) {
     if (SMEM > 48 * 1024) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM);
-    if (e == cudaSuccess) e = launch_k(kernel, grid, dim3(WARPS * 32), SMEM, s, a);
+    if (e != cudaSuccess) return;
+    scan_variant_rec = {2, LPR, WARPS, RPL, st ? 1 : 0, 0};
+    scan_last_variant = &scan_variant_rec;
+    e = launch_k(kernel, grid, dim3(WARPS * 32), SMEM, s, a);
   };
-  if (a.structured_a) go(scan_seq_kernel<LPR, WARPS, RPL, true>);
-  else go(scan_seq_kernel<LPR, WARPS, RPL, false>);
+  if (a.structured_a) go(scan_seq_kernel<LPR, WARPS, RPL, true>, true);
+  else go(scan_seq_kernel<LPR, WARPS, RPL, false>, false);
   return e;
 }
 
-// CTA shape of scan_seq_kernel: two rows per lane, 64 or 128 rows per CTA (Di is a multiple of 64: include/vasr.h).
+// CTA shape of scan_seq_kernel: two rows per lane, four warps of them if that is at most 128 rows and divides Di, else
+// a 64-row CTA (Di is a multiple of 64: include/vasr.h).  Only those two shapes are compiled.
 template <int LPR>
 cudaError_t launch_recurrence(const ScanArgs& a, cudaStream_t s) {
-  constexpr int G = 32 / LPR;
+  constexpr int RW = 2 * 32 / LPR;                      // rows per warp
+  constexpr int W_WIDE = 128 / RW < 4 ? 128 / RW : 4;   // warps of the wider CTA
+  constexpr int W_64 = 64 / RW;                         // warps of a 64-row CTA
   // cp.async moves 16-byte pieces: every row start must be 16-byte aligned
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   if ((a.ldx & 3) || (a.lddt & 3) || (a.ldy & 1) || !al16(a.x) || !al16(a.dt) || (a.z && ((a.ldz & 3) || !al16(a.z))) ||
@@ -1474,9 +1483,10 @@ cudaError_t launch_recurrence(const ScanArgs& a, cudaStream_t s) {
     return cudaErrorInvalidValue;
   // four warps = one warp of the CTA per SM sub-partition: the warps of a CTA then advance at the same rate and the
   // per-chunk barrier costs nothing (measured 0.320 ms vs 0.356 ms with three)
-  if (4 * G * 2 <= 128 && a.Di % (4 * G * 2) == 0) return launch_seq<LPR, 4, 2>(a, s);
-  if (2 * G * 2 <= 128 && a.Di % (2 * G * 2) == 0) return launch_seq<LPR, 2, 2>(a, s);
-  if (a.Di % (G * 2) == 0) return launch_seq<LPR, 1, 2>(a, s);
+  if (a.Di % (W_WIDE * RW) == 0) return launch_seq<LPR, W_WIDE, 2>(a, s);
+  if constexpr (W_64 != W_WIDE) {
+    if (a.Di % 64 == 0) return launch_seq<LPR, W_64, 2>(a, s);
+  }
   return cudaErrorInvalidValue;
 }
 
@@ -1486,22 +1496,40 @@ cudaError_t launch_lpr(const ScanArgs& a, cudaStream_t s) {
   constexpr int ROWS = SCAN_THREADS / LPR8;
   if (a.Di % ROWS != 0) return cudaErrorInvalidValue;
   dim3 grid((unsigned)(a.Di / ROWS), (unsigned)a.B);
+  scan_variant_rec = {1, LPR8, 0, 0, a.structured_a ? 1 : 0, 0};
+  scan_last_variant = &scan_variant_rec;
   if (a.structured_a) return launch_k(scan_quirk_kernel<LPR8, true>, grid, dim3(SCAN_THREADS), 0, s, a);
   return launch_k(scan_quirk_kernel<LPR8, false>, grid, dim3(SCAN_THREADS), 0, s, a);
 }
 
+// VASR_SCAN_OLD=1: scan_seq_kernel for every shape; VASR_SCAN_RP=1 / 2: that CTA shape of scan_rp_kernel;
+// VASR_SCAN_SPLIT=0: never split, n > 0: n slots.  (Read in the debug build only, common.cuh.)
+ScanOverride env_override() {
+  ScanOverride o;
+  o.rp = debug_env_int("VASR_SCAN_OLD", 0) ? -1 : debug_env_int("VASR_SCAN_RP", 0);
+  const int sp = debug_env_int("VASR_SCAN_SPLIT", -1);
+  o.split = sp == 0 ? -1 : (sp > 0 ? sp : 0);
+  return o;
+}
+
 }  // namespace
 
-cudaError_t launch_selective_scan(const ScanArgs& a, cudaStream_t s, int64_t* launches) {
+thread_local const ScanVariant* scan_last_variant = nullptr;
+
+cudaError_t launch_selective_scan(const ScanArgs& a, cudaStream_t s, int64_t* launches, const ScanOverride* ov) {
   if (a.B <= 0 || a.L <= 0) return cudaSuccess;
   if (a.B > 65535 || a.L >= (1LL << (NLEV - 2))) return cudaErrorInvalidValue;
   if ((a.ldb & 3) || (a.ldc & 3) || (reinterpret_cast<uintptr_t>(a.Bm) & 15) ||
       (reinterpret_cast<uintptr_t>(a.Cm) & 15))
     return cudaErrorInvalidValue;
+  static const ScanOverride env_ov = env_override();
+  const ScanOverride& o = ov ? *ov : env_ov;
   cudaError_t e;
-  static const int old_env = debug_env_int("VASR_SCAN_OLD", 0);          // 1: scan_seq_kernel for every shape
-  if (rp_takes(a) && !old_env) {
-    e = launch_rp(a, s);
+  const bool rp = rp_takes(a);
+  if (ov && ov->rp > 0 && (!rp || (ov->rp == 2 && a.Di % RpCfg<2>::ROWS != 0)))   // a forced shape that does not fit
+    return cudaErrorInvalidValue;
+  if (rp && o.rp >= 0) {
+    e = launch_rp(a, o, s);
     if (launches && e == cudaSuccess) ++*launches;
     return e;
   }

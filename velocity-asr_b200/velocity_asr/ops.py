@@ -35,6 +35,8 @@ def selective_scan(x: torch.Tensor, dt: torch.Tensor, A: torch.Tensor, B: torch.
         # presumes a growing cumsum: dt is a softplus output wherever the reference calls its scan (ssm.py:118)
         raise ValueError("selective_scan(scan_mode='parallel') needs dt >= 0 (dt is a softplus output, ssm.py:118)")
     Bsz, L, Di = x.shape
+    if Di <= 0 or Di % 64 != 0:
+        raise ValueError(f"selective_scan needs Di to be a positive multiple of 64, got {Di}")
     N = A.numel()
     y = torch.empty_like(x)
     if Bsz == 0 or L == 0:
